@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W     # the reference's CPU path (oracle port)
+    python bench.py --steps K --dump-outputs DIR              # + the last timed window's outputs as DIR/*.npy
 
 One "step" = one simulation timestep forward AND its backward, over every agent of the synthetic
 England-scale world (config.workload).  K steps are run as BPTT windows (forward w steps, backward
@@ -202,6 +203,34 @@ def workload_name(n_agents, policies=False):
             + (", social distancing + school/pub/cinema/gym closure + quarantine(stage 4) from day 15" if policies else ""))
 
 
+DUMP_AGENTS = 1 << 20      # agents in the sample of the per-agent state that --dump-outputs writes
+
+
+def window_outputs(out, window, data, per_agent):
+    """What a caller of the timed path receives from its last window, as host arrays: the result series and
+    d loss / d log_beta (a leading axis over the samples when a rank evaluates several) and, ``per_agent``, the
+    agents' final infection state in the order the world was loaded in, for a fixed seeded sample of agents."""
+    from grad_june.world import original_order
+
+    out = out.detach().cpu().numpy().astype(np.float32)
+    t = window + 1                   # the seeding step + `window` timesteps
+    arrays = {"cases_per_timestep": out[..., :t], "deaths_per_timestep": out[..., t:2 * t],
+              "grad_log_beta": out[..., 2 * t:]}
+    if per_agent:
+        inf = original_order(data, data["agent"].is_infected.detach())
+        idx = np.sort(np.random.default_rng(0).choice(inf.numel(), size=min(DUMP_AGENTS, inf.numel()), replace=False))
+        arrays["is_infected_sample"] = inf[torch.from_numpy(idx).to(inf.device)].cpu().numpy().astype(np.float32)
+        arrays["is_infected_sample_agent"] = idx.astype(np.float64)
+    return arrays
+
+
+def write_outputs(dirname, arrays):
+    d = Path(dirname)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.ascontiguousarray(a))
+
+
 # ------------------------------------------------------------------------------------------
 # parity inside the benchmark: one teacher-forced step at the benchmark's size against the oracle on the same GPU
 # ------------------------------------------------------------------------------------------
@@ -286,8 +315,10 @@ def measure(args, ctx, scaling, graph, full=True):
     per_step = 40.0 * N            # bytes retained per agent per step until backward (pre-state 24 + tape 8 + sums ~3)
     resident = 120.0 * N           # world CSR + static arrays + transient workspaces + initial state backup
     max_window = int(max(1, (free * 0.85 - resident) // per_step))
-    window = min(args.steps, args.window or min(max_window, 60), max_window)
-    if world_size > 1:             # the ranks of a partitioned world step together
+    # the timed region is exactly K = --steps timesteps in windows of one length: the longest that divides K
+    cap = min(args.steps, args.window or 60, max_window)
+    window = max(w for w in range(1, cap + 1) if args.steps % w == 0)
+    if world_size > 1:             # the ranks of a partitioned world step together (a divisor of K on every rank)
         wt = torch.tensor([window], device=dev)
         dist.all_reduce(wt, op=dist.ReduceOp.MIN)
         window = int(wt.item())
@@ -366,7 +397,7 @@ def measure(args, ctx, scaling, graph, full=True):
         return torch.cat([results["cases_per_timestep"], results["deaths_per_timestep"], grads])
 
     resident_log_beta = host_log_beta.to(dev)
-    n_windows = max(1, -(-args.steps // window))
+    n_windows = args.steps // window
     steps_done = n_windows * window
     eager_window = one_window
 
@@ -487,6 +518,9 @@ def measure(args, ctx, scaling, graph, full=True):
         torch.cuda.nvtx.range_pop()
         barrier()
         ms = e0.elapsed_time(e1)
+        outputs = None
+        if args.dump_outputs and rank == 0 and full:     # before the windows below overwrite the last one's state
+            outputs = window_outputs(out, window, data, per_agent=n_samples == 1 and world_size == 1)
         # ---- repeats: the same window R more times, each timed on its own (spread of the measurement) --------
         rep_ms = []
         for _ in range(args.repeats if full else 0):
@@ -554,7 +588,7 @@ def measure(args, ctx, scaling, graph, full=True):
         res = dict(value=total_units / (ms * 1e-3), ms=ms, steps_done=steps_done, window=window, N=N, n_total=n_total,
                    world=world, prof=prof, clk=clk, rank_ms=rank_ms, e2e_s=e2e_s, h2d=h2d, d2h=d2h, rep_ms=rep_ms,
                    parallelism=parallelism, parity=parity, graph=graph, scaling=scaling, total_units=total_units,
-                   batch=B)
+                   batch=B, outputs=outputs)
     if graphed is not None:
         ctx["captured_nccl"] = ctx.get("captured_nccl", False) or geo
         graphed.graph.reset()
@@ -564,7 +598,9 @@ def measure(args, ctx, scaling, graph, full=True):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=120)
+    ap.add_argument("--steps", type=int, default=120,
+                    help="timesteps K of the timed region, run as K / w BPTT windows of w timesteps: the longest w "
+                         "that divides K and that --window and the GPU's memory allow")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--agents", type=int, default=56_000_000,
@@ -596,7 +632,8 @@ def main():
     ap.add_argument("--policies", action="store_true",
                     help="BASELINE config 4: social distancing, school/leisure closures and quarantine from day 15")
     ap.add_argument("--window", type=int, default=0,
-                    help="BPTT window (0 = 60 timesteps as in BASELINE.json, fewer if memory does not allow)")
+                    help="longest BPTT window (0 = 60 timesteps as in BASELINE.json, fewer if memory does not allow); "
+                         "the window also divides --steps")
     ap.add_argument("--repeats", type=int, default=5, help="further windows timed one by one (median / spread)")
     ap.add_argument("--no-verify", dest="verify", action="store_false",
                     help="skip the teacher-forced parity step against the oracle (N = 1)")
@@ -607,7 +644,15 @@ def main():
     ap.add_argument("--cpu-agents", type=int, default=1_000_000, help="agents of the CPU-baseline sample")
     ap.add_argument("--cpu-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what their last window computed as DIR/<name>.npy: the result "
+                         "series, d loss / d log_beta and (one sample, one GPU) the final infection state of a fixed "
+                         f"seeded sample of {DUMP_AGENTS} agents; the inputs are the same for the same arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
 
     rank = int(os.environ.get("RANK", 0))
     world_size = int(os.environ.get("WORLD_SIZE", 1))
@@ -646,6 +691,8 @@ def main():
         weak = measure(args, ctx, "weak", graph, full=False)
 
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, m["outputs"])
         peak, peak_kind = measured_peak_gbs()
         world, prof, N, value = m["world"], m["prof"], m["N"], m["value"]
         steps_done = m["steps_done"]
