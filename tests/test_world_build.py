@@ -45,7 +45,7 @@ def _compare(native, ref, types):
     cells_total = 0
     for ti, t in enumerate(types):
         if ref.type_tier[ti] == W.TIER_RANGE:
-            assert bool(d.range_pc_from_size[ti]) == bool(ref.range_pc_from_size[ti]) == True, t   # noqa: E712
+            assert bool(d.range_pc_from_size[ti]) == bool(ref.range_pc_from_size[ti]), t
             assert torch.equal(native.array("range_slot", n, index=ti), ref.range_slot[ti][:n].cpu()), t
             assert torch.equal(native.array("range_pc", n, torch.float32, index=ti), ref.range_pc[ti][:n].cpu()), t
         elif ref.type_tier[ti] == W.TIER_CELL:
@@ -67,7 +67,8 @@ def test_native_build_of_the_sample_world_matches_python(golden_dir):
     data = W.renumber_world(data)
     assert perm is not None and torch.equal(perm, data["agent"].original_index)
     ref = _python_build(data)
-    assert ref.type_tier[data.venue_types().index("household")] == W.TIER_RANGE
+    hi = data.venue_types().index("household")
+    assert ref.type_tier[hi] == W.TIER_RANGE and ref.range_pc_from_size[hi]
     _compare(native, ref, data.venue_types())
     native.close()
 
@@ -93,6 +94,7 @@ def test_native_build_of_a_shuffled_synthetic_world():
     data = W.renumber_world(data)
     assert torch.equal(data["agent"].original_index, torch.arange(n))
     ref = _python_build(data)
+    assert ref.range_pc_from_size[data.venue_types().index("household")]
     _compare(native, ref, data.venue_types())
     assert perm is not None
 
