@@ -118,6 +118,28 @@ __device__ __forceinline__ int64_t noise_agent(const gj_world_desc& w, const gj_
   return w.orig_id ? (int64_t)w.orig_id[a] : (int64_t)p.agent_offset + a;
 }
 
+// results by label (gj_fwd_io.label): add one agent's post-step cases (0..3) and death indicator (0/1), exact small
+// integers, to column label[a] of the integer accumulator acc[n_labels][2].  The warp's values are counted with ballots;
+// a warp without cases or deaths (most warps early in an epidemic) returns before it loads a label.  Lanes that share a
+// label are combined first — without __match_any_sync when the whole warp holds one label, as after renumbering by
+// area — so a warp issues one atomic per distinct label and value; any labels stay correct.  Integer sums are exact
+// and independent of the order of the atomics.
+__device__ __forceinline__ void label_add(uint32_t* __restrict__ acc, const int32_t* __restrict__ label, uint32_t a,
+                                          uint32_t cases, uint32_t deaths) {
+  const unsigned act = __activemask();
+  const unsigned c0 = __ballot_sync(act, cases & 1u), c1 = __ballot_sync(act, cases & 2u);
+  const unsigned dd = __ballot_sync(act, deaths != 0u);
+  if ((c0 | c1 | dd) == 0u) return;
+  const int32_t lab = label[a];
+  const int32_t l0 = __shfl_sync(act, lab, __ffs(act) - 1);
+  const unsigned grp = __all_sync(act, lab == l0) ? act : __match_any_sync(act, lab);
+  if ((int)(threadIdx.x & 31u) == __ffs(grp) - 1) {
+    const uint32_t c = __popc(c0 & grp) + 2u * __popc(c1 & grp), d = __popc(dd & grp);
+    if (c) atomicAdd(acc + 2 * (int64_t)lab, c);
+    if (d) atomicAdd(acc + 2 * (int64_t)lab + 1, d);
+  }
+}
+
 // one standard normal per (agent, call): Box-Muller on stream 1
 __device__ __forceinline__ float draw_step_normal(uint64_t seed, uint32_t call, int64_t agent) {
   uint32_t r[4];

@@ -416,6 +416,7 @@ __device__ __forceinline__ void block_reduce_finish(double (&v)[kR], int nr, dou
 // agent-major kernels for calls WITHOUT the networks phase (stand-alone sampler / infect / symptoms and the
 // seeding step): persistent grid-stride loop, reductions finished by the last CTA
 // ================================================================================================
+template <bool kLabel>
 __global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_step_params p, gj_fwd_io io,
                                                           double* __restrict__ red_part,
                                                           unsigned int* __restrict__ ticket) {
@@ -434,7 +435,7 @@ __global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_st
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
     const float q = io.q_in ? io.q_in[a] : 1.0f;
-    forward_tail(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, redf);
+    forward_tail<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, redf, io.label_acc);
   }
   if (io.red) {
     double red[kMaxRed];
@@ -444,6 +445,7 @@ __global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_st
   }
 }
 
+template <bool kLabel>
 __global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_step_params p, gj_bwd_io io,
                                                            double* __restrict__ red_part,
                                                            unsigned int* __restrict__ ticket) {
@@ -460,7 +462,7 @@ __global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_s
     st.cur = io.cur ? io.cur[a] : 1.0f;
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
-    const BackAgent r = backward_agent(p, io, N, a, noise_agent(w, p, a), cls % 100, st, false);
+    const BackAgent r = backward_agent<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, false);
     if (io.g_q_out) io.g_q_out[a] = r.gq;
     if (io.g_n_out) io.g_n_out[a] = r.gn;
     if (seed_mode) gfrac[0] += (double)(-r.gq);  // q = 1 - fraction
@@ -472,6 +474,19 @@ __global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_s
     if (io.g_ttn) io.g_ttn[a] = r.gttn;
   }
   if (seed_mode && io.g_seed_fraction) block_reduce_finish<1>(gfrac, 1, red_part, ticket, io.g_seed_fraction);
+}
+
+// results by label: the step's integer accumulator -> fp32 table, and back to zero for the next step (sample blockIdx.z)
+__global__ void __launch_bounds__(kBlock) k_label_finish(int64_t n, uint32_t* __restrict__ acc, float* __restrict__ out,
+                                                         int64_t stride) {
+  pdl_launch();
+  pdl_wait();
+  acc += (int64_t)blockIdx.z * stride;
+  out += (int64_t)blockIdx.z * stride;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    out[i] = (float)acc[i];
+    acc[i] = 0u;
+  }
 }
 
 // dL/dbeta_k = sum_g pc_g * S~_g * R_g   (fixed-order two-level sum in fp64)
@@ -570,7 +585,7 @@ static int build_channels(const gj_world_desc* w, const gj_step_params* p, Chann
   return 0;
 }
 
-static const Batch kNoBatch = {1, 0u, 0, 0, 0, 0, nullptr};
+static const Batch kNoBatch = {1, 0u, 0, 0, 0, 0, nullptr, 0};
 // grid of a persistent kernel in a batched launch: the resident wave is split between the samples (block = run * nb +
 // sample), at least one CTA and at most one per tile for each
 static inline int batch_grid(const gj_world_desc* w, int64_t resident, const Batch& bt) {
@@ -888,8 +903,9 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
   }
   if (pipe_enabled() && pipe_aligned_fwd(w, lp, io)) {
     ProfScope ps(K_AGENT_FWD, st);
-    static OccCache occ[12];
+    static OccCache occ[20];
     const bool diag = io->q || io->n;
+    const bool lab = io->label != nullptr;
     const size_t smem = next ? sizeof(PipeFwdSharedT<true, false>)
                              : (batch ? sizeof(PipeFwdSharedT<false, true>) : sizeof(PipeFwdSharedT<false, false>));
     NextStep nx;
@@ -899,25 +915,35 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
       nx.tile_part = sc.tile_part;   // consumed by this step's k_cell_groups before the agent kernel runs
       nx.sct = Scatter{sc.sct_acc, sc.sct_dirty};   // zeroed by this step's finalize pass, which has already run
     }
-#define GJ_PIPE_FWD(Q, D, X, B, I)                                                                                    \
-  launch_pdl(k_pipe_forward<Q, D, X, B>,                                                                              \
-             dim3(pipe_grid(w, k_pipe_forward<Q, D, X, B>, kPipeThreads, smem, &occ[I], bt)), dim3(kPipeThreads), smem, \
-             st, *w, *p, lp, *io, (const float*)sc.cell_buf, sc.red_part, sc.tickets, nx, bt)
-    if (batch) {
-      if (quar && diag) GJ_PIPE_FWD(true, true, false, true, 11);
-      else if (quar) GJ_PIPE_FWD(true, false, false, true, 10);
-      else if (diag) GJ_PIPE_FWD(false, true, false, true, 9);
-      else GJ_PIPE_FWD(false, false, false, true, 8);
+#define GJ_PIPE_FWD(Q, D, X, B, L, I)                                                                                 \
+  launch_pdl(k_pipe_forward<Q, D, X, B, L>,                                                                           \
+             dim3(pipe_grid(w, k_pipe_forward<Q, D, X, B, L>, kPipeThreads, smem, &occ[I], bt)), dim3(kPipeThreads),    \
+             smem, st, *w, *p, lp, *io, (const float*)sc.cell_buf, sc.red_part, sc.tickets, nx, bt)
+    if (lab && batch) {   // a step with a label table never gets a look-ahead (step_forward_impl)
+      if (quar && diag) GJ_PIPE_FWD(true, true, false, true, true, 19);
+      else if (quar) GJ_PIPE_FWD(true, false, false, true, true, 18);
+      else if (diag) GJ_PIPE_FWD(false, true, false, true, true, 17);
+      else GJ_PIPE_FWD(false, false, false, true, true, 16);
+    } else if (lab) {
+      if (quar && diag) GJ_PIPE_FWD(true, true, false, false, true, 15);
+      else if (quar) GJ_PIPE_FWD(true, false, false, false, true, 14);
+      else if (diag) GJ_PIPE_FWD(false, true, false, false, true, 13);
+      else GJ_PIPE_FWD(false, false, false, false, true, 12);
+    } else if (batch) {
+      if (quar && diag) GJ_PIPE_FWD(true, true, false, true, false, 11);
+      else if (quar) GJ_PIPE_FWD(true, false, false, true, false, 10);
+      else if (diag) GJ_PIPE_FWD(false, true, false, true, false, 9);
+      else GJ_PIPE_FWD(false, false, false, true, false, 8);
     } else if (next) {
-      if (quar && diag) GJ_PIPE_FWD(true, true, true, false, 7);
-      else if (quar) GJ_PIPE_FWD(true, false, true, false, 6);
-      else if (diag) GJ_PIPE_FWD(false, true, true, false, 5);
-      else GJ_PIPE_FWD(false, false, true, false, 4);
+      if (quar && diag) GJ_PIPE_FWD(true, true, true, false, false, 7);
+      else if (quar) GJ_PIPE_FWD(true, false, true, false, false, 6);
+      else if (diag) GJ_PIPE_FWD(false, true, true, false, false, 5);
+      else GJ_PIPE_FWD(false, false, true, false, false, 4);
     } else {
-      if (quar && diag) GJ_PIPE_FWD(true, true, false, false, 3);
-      else if (quar) GJ_PIPE_FWD(true, false, false, false, 2);
-      else if (diag) GJ_PIPE_FWD(false, true, false, false, 1);
-      else GJ_PIPE_FWD(false, false, false, false, 0);
+      if (quar && diag) GJ_PIPE_FWD(true, true, false, false, false, 3);
+      else if (quar) GJ_PIPE_FWD(true, false, false, false, false, 2);
+      else if (diag) GJ_PIPE_FWD(false, true, false, false, false, 1);
+      else GJ_PIPE_FWD(false, false, false, false, false, 0);
     }
 #undef GJ_PIPE_FWD
     GJ_CHECK_LAUNCH("k_pipe_forward");
@@ -926,12 +952,23 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
   if (batch) return bad("batched step: the pipelined kernels are off or an array is not 16-byte aligned");
   {
     ProfScope ps(K_AGENT_FWD, st);
-    static OccCache occ[4];
+    static OccCache occ[8];
     const bool diag = io->q || io->n;
-    if (quar && diag) k_lean_forward<true, true><<<lean_grid(w, k_lean_forward<true, true>, &occ[3]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets);
-    else if (quar) k_lean_forward<true, false><<<lean_grid(w, k_lean_forward<true, false>, &occ[2]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets);
-    else if (diag) k_lean_forward<false, true><<<lean_grid(w, k_lean_forward<false, true>, &occ[1]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets);
-    else k_lean_forward<false, false><<<lean_grid(w, k_lean_forward<false, false>, &occ[0]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets);
+#define GJ_LEAN_FWD(Q, D, L, I)                                                                                       \
+  k_lean_forward<Q, D, L><<<lean_grid(w, k_lean_forward<Q, D, L>, &occ[I]), kLeanThreads, 0, st>>>(                   \
+      *w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets)
+    if (io->label) {
+      if (quar && diag) GJ_LEAN_FWD(true, true, true, 7);
+      else if (quar) GJ_LEAN_FWD(true, false, true, 6);
+      else if (diag) GJ_LEAN_FWD(false, true, true, 5);
+      else GJ_LEAN_FWD(false, false, true, 4);
+    } else {
+      if (quar && diag) GJ_LEAN_FWD(true, true, false, 3);
+      else if (quar) GJ_LEAN_FWD(true, false, false, 2);
+      else if (diag) GJ_LEAN_FWD(false, true, false, 1);
+      else GJ_LEAN_FWD(false, false, false, 0);
+    }
+#undef GJ_LEAN_FWD
     GJ_CHECK_LAUNCH("k_lean_forward");
   }
   return 0;
@@ -941,31 +978,46 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
                          const gj_bwd_io* io, const Scratch& sc, cudaStream_t st, const Batch& bt = kNoBatch) {
   const bool quar = p->n_quar > 0;
   const bool batch = bt.nb > 1;
-  static OccCache occ_b[2], occ_g[2];
+  static OccCache occ_b[4], occ_g[2];
+  const bool lab = io->label && io->g_red_label;
   int gather_grid = 1;
   const bool pipe = pipe_enabled() && pipe_aligned_bwd(w, lp, io);
   if (batch && !pipe) return bad("batched step: the pipelined kernels are off or an array is not 16-byte aligned");
   if (p->stage != GJ_STAGE_REST) {
     if (pipe) {
       ProfScope ps(K_AGENT_BWD, st);
-      static OccCache occ[4];
+      static OccCache occ[8];
       const size_t smem = sizeof(PipeBwdShared);
-#define GJ_PIPE_BWD(Q, B, I)                                                                                          \
-  launch_pdl(k_pipe_backward<Q, B>, dim3(pipe_grid(w, k_pipe_backward<Q, B>, kBwdThreads, smem, &occ[I], bt)),          \
+#define GJ_PIPE_BWD(Q, B, L, I)                                                                                       \
+  launch_pdl(k_pipe_backward<Q, B, L>, dim3(pipe_grid(w, k_pipe_backward<Q, B, L>, kBwdThreads, smem, &occ[I], bt)),    \
              dim3(kBwdThreads), smem, st, *w, *p, lp, *io, sc.tile_part, bt)
-      if (batch) {
-        if (quar) GJ_PIPE_BWD(true, true, 3);
-        else GJ_PIPE_BWD(false, true, 2);
+      if (lab && batch) {
+        if (quar) GJ_PIPE_BWD(true, true, true, 7);
+        else GJ_PIPE_BWD(false, true, true, 6);
+      } else if (lab) {
+        if (quar) GJ_PIPE_BWD(true, false, true, 5);
+        else GJ_PIPE_BWD(false, false, true, 4);
+      } else if (batch) {
+        if (quar) GJ_PIPE_BWD(true, true, false, 3);
+        else GJ_PIPE_BWD(false, true, false, 2);
       } else {
-        if (quar) GJ_PIPE_BWD(true, false, 1);
-        else GJ_PIPE_BWD(false, false, 0);
+        if (quar) GJ_PIPE_BWD(true, false, false, 1);
+        else GJ_PIPE_BWD(false, false, false, 0);
       }
 #undef GJ_PIPE_BWD
       GJ_CHECK_LAUNCH("k_pipe_backward");
     } else {
       ProfScope ps(K_AGENT_BWD, st);
-    if (quar) k_lean_backward<true><<<lean_grid(w, k_lean_backward<true>, &occ_b[1]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.tile_part);
-    else k_lean_backward<false><<<lean_grid(w, k_lean_backward<false>, &occ_b[0]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.tile_part);
+#define GJ_LEAN_BWD(Q, L, I) \
+  k_lean_backward<Q, L><<<lean_grid(w, k_lean_backward<Q, L>, &occ_b[I]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.tile_part)
+      if (lab) {
+        if (quar) GJ_LEAN_BWD(true, true, 3);
+        else GJ_LEAN_BWD(false, true, 2);
+      } else {
+        if (quar) GJ_LEAN_BWD(true, false, 1);
+        else GJ_LEAN_BWD(false, false, 0);
+      }
+#undef GJ_LEAN_BWD
       GJ_CHECK_LAUNCH("k_lean_backward");
     }
     if (lp.has_generic)
@@ -1422,14 +1474,49 @@ static int make_batch(const gj_world_desc* w, const gj_step_params* p, const gj_
   bt->sBeta = (int)b->beta_stride;
   bt->sRed = (int)b->red_stride;
   bt->noise = b->noise;
+  bt->sLab = b->label_stride;
   if (b->noise && !aligned16(b->noise)) return bad("batch: noise must be 16-byte aligned");
   return 0;
 }
 
+// results by label: the checks of the header, and the conversion of the step's integer sums
+static int check_labels(const gj_fwd_io* io, const Batch& bt) {
+  if (!io->label) return 0;
+  if (io->n_labels < 1 || io->n_labels > (1 << 30)) return bad("n_labels must lie in [1, 2^30]");
+  if (!io->red_label || !io->label_acc) return bad("label given without red_label / label_acc");
+  if (bt.nb > 1 && bt.sLab < 2 * (int64_t)io->n_labels) return bad("batch: label_stride must be >= 2 * n_labels");
+  return 0;
+}
+static int finish_labels(const gj_fwd_io* io, cudaStream_t st, const Batch& bt) {
+  if (!io->label) return 0;
+  ProfScope ps(K_OTHER, st);
+  const int64_t n = 2 * (int64_t)io->n_labels;
+  const int64_t blocks = (n + kBlock - 1) / kBlock;
+  launch_pdl(k_label_finish, dim3((int)(blocks < kRedBlocks ? blocks : kRedBlocks), 1, bt.nb), dim3(kBlock), 0, st, n,
+             io->label_acc, io->red_label, bt.sLab);
+  GJ_CHECK_LAUNCH("k_label_finish");
+  return 0;
+}
+
+static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, const gj_step_params* next,
+                            const gj_fwd_io* io, void* stream, const gj_batch* batch);
+// the agent kernels accumulate the label table as integers; one small kernel then converts it (and re-zeroes)
 static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, const gj_step_params* next,
                              const gj_fwd_io* io, void* stream, const gj_batch* batch = nullptr) {
   if (int e = check_world(w)) return e;
   if (!p || !io) return bad("params/io is NULL");
+  Batch bt = kNoBatch;
+  if (batch)
+    if (int e = make_batch(w, p, batch, &bt)) return e;
+  if (int e = check_labels(io, bt)) return e;
+  const int rc = step_forward_run(w, p, next, io, stream, batch);
+  if (rc < 0 || p->stage == GJ_STAGE_SUMS) return rc;
+  if (int e = finish_labels(io, (cudaStream_t)stream, bt)) return e;
+  return rc;
+}
+
+static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, const gj_step_params* next,
+                            const gj_fwd_io* io, void* stream, const gj_batch* batch) {
   Batch bt = kNoBatch;
   if (batch)
     if (int e = make_batch(w, p, batch, &bt)) return e;
@@ -1457,19 +1544,29 @@ static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, co
       io->ttn && io->tape_y0 && io->stage_prob && io->s_o && io->inf_o && io->tinf_o && io->cur_o && io->nxt_o &&
       io->ttn_o) {   // Runner.set_initial_cases with in-kernel noise: the throughput-mode seeding kernel
     ProfScope ps(K_SEED, st);
-    static OccCache occ[2];
+    static OccCache occ[4];
     const bool diag = io->n != nullptr;
     int64_t g = (N + (int64_t)kLeanThreads * kLeanBatch - 1) / ((int64_t)kLeanThreads * kLeanBatch);
     gj_world_desc wt = *w;
     wt.n_tiles = g;   // lean_grid clips the persistent grid to the work available
-    if (diag) launch_pdl(k_lean_seed<true>, dim3(lean_grid(&wt, k_lean_seed<true>, &occ[1])), dim3(kLeanThreads), 0, st, *w, pp, *io, sc.red_part, sc.tickets);
-    else launch_pdl(k_lean_seed<false>, dim3(lean_grid(&wt, k_lean_seed<false>, &occ[0])), dim3(kLeanThreads), 0, st, *w, pp, *io, sc.red_part, sc.tickets);
+#define GJ_SEED(D, L, I) \
+  launch_pdl(k_lean_seed<D, L>, dim3(lean_grid(&wt, k_lean_seed<D, L>, &occ[I])), dim3(kLeanThreads), 0, st, *w, pp, *io, \
+             sc.red_part, sc.tickets)
+    if (io->label) {
+      if (diag) GJ_SEED(true, true, 3);
+      else GJ_SEED(false, true, 2);
+    } else {
+      if (diag) GJ_SEED(true, false, 1);
+      else GJ_SEED(false, false, 0);
+    }
+#undef GJ_SEED
     GJ_CHECK_LAUNCH("k_lean_seed");
     return 0;
   }
   if (!(pp.phases & GJ_PHASE_NETWORKS)) {  // stand-alone sampler / infect / symptoms, seeding
     ProfScope ps(K_AGENT_FWD, st);
-    k_agent_forward<<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    if (io->label) k_agent_forward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    else k_agent_forward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
     GJ_CHECK_LAUNCH("k_agent_forward");
     return 0;
   }
@@ -1492,7 +1589,7 @@ static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, co
       // look-ahead: the following step must itself run on the throughput-mode kernels (it then honours t_ready)
       NextStep nx;
       bool have_next = false;
-      if (next && lookahead_enabled() && io->T_next && next->mode == GJ_MODE_STEP && next->phases == GJ_PHASE_ALL &&
+      if (next && !io->label && lookahead_enabled() && io->T_next && next->mode == GJ_MODE_STEP && next->phases == GJ_PHASE_ALL &&
           (next->n_quar <= 0 || io->Tq_next)) {
         Channels chn;
         Plan pln;
@@ -1543,7 +1640,8 @@ static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, co
   if (int e = launch_cell_gather(w, &pp, pl, io->S_scaled, sc, st)) return e;
   {
     ProfScope ps(K_AGENT_FWD, st);
-    k_tile_forward<<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
+    if (io->label) k_tile_forward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
+    else k_tile_forward<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
     GJ_CHECK_LAUNCH("k_tile_forward");
   }
   return 0;
@@ -1587,7 +1685,9 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if ((pp.phases & GJ_PHASE_SAMPLE) && !io->tape_y0) return bad("tape_y0 is NULL");
   if (!(pp.phases & GJ_PHASE_NETWORKS)) {
     ProfScope ps(K_AGENT_BWD, st);
-    k_agent_backward<<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    if (io->label && io->g_red_label)
+      k_agent_backward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    else k_agent_backward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
     GJ_CHECK_LAUNCH("k_agent_backward");
     return 0;
   }
@@ -1614,7 +1714,8 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if (pp.stage != GJ_STAGE_REST) {
     {
       ProfScope ps(K_AGENT_BWD, st);
-      k_tile_backward<<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
+      if (io->label && io->g_red_label) k_tile_backward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
+      else k_tile_backward<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
       GJ_CHECK_LAUNCH("k_tile_backward");
     }
     if (pl.n_generic > 0)

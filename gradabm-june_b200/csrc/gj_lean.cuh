@@ -802,7 +802,7 @@ struct LeanFwdShared {
 
 constexpr int kLeanBatch = 2;  // agents a thread keeps in flight: their loads are issued before any arithmetic
 
-template <bool kQuar, bool kDiag>
+template <bool kQuar, bool kDiag, bool kLabel>
 __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
                                                                   gj_fwd_io io, const float* __restrict__ cell_buf,
                                                                   double* __restrict__ red_part,
@@ -891,8 +891,10 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
         const float gv = lean_generic_finish(w, SP, ent[h], a, gen[h]);
         const float Lc = lp.n_cell > 0 ? L[cls[h]] : 0.0f;
         const uint64_t ga = w.orig_id ? (uint64_t)oid[h] : p.agent_offset + a;
-        lean_forward_agent<kQuar, kDiag>(p, lp, io, a, ga, hs, gv, Lc, beta_r, rpc[h], s[h], inf[h], tinf[h], cur[h],
-                                         nxt[h], ttn[h], cls[h], inv_tau, dead, sh.hist, &sh.deaths);
+        const FwdOut o = lean_forward_agent<kQuar, kDiag>(p, lp, io, a, ga, hs, gv, Lc, beta_r, rpc[h], s[h], inf[h],
+                                                          tinf[h], cur[h], nxt[h], ttn[h], cls[h], inv_tau, dead, sh.hist,
+                                                          &sh.deaths);
+        if (kLabel) label_add(io.label_acc, io.label, a, (uint32_t)o.inf, o.cur == dead ? 1u : 0u);
       }
     }
     tile = tend;
@@ -921,7 +923,7 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
 // variant: same values), first symptoms update, reductions — the arithmetic of lean_forward_core without networks.
 // Replaces the generic k_agent_forward (IEEE libm, 1.45 ms per window at 56 M agents) for Runner.set_initial_cases.
 // =====================================================================================================
-template <bool kDiag>
+template <bool kDiag, bool kLabel>
 __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, gj_step_params p, gj_fwd_io io,
                                                               double* __restrict__ red_part,
                                                               unsigned int* __restrict__ ticket) {
@@ -974,6 +976,7 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
       io.cur_o[a] = o.cur_o;
       io.nxt_o[a] = o.nxt_o;
       io.ttn_o[a] = o.ttn_o;
+      if (kLabel) label_add(io.label_acc, io.label, a, (uint32_t)o.inf_o, o.cur_o == dead ? 1u : 0u);
     }
   }
   if (io.red) {
@@ -997,14 +1000,16 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
 
 // per-agent arithmetic of the backward pass (shared with gj_pipe.cuh): symptoms^T, infect^T, sampler^T, clamp/exp
 // chain -> cotangents of the state, w = dL/dLambda * s (and its quarantine-masked copy), cell-channel sums in acc
-template <bool kQuar>
+// kLabel: glab_i / glab_d are the cotangents of the agent's column of the label table (cases, and deaths / dead)
+template <bool kQuar, bool kLabel = false>
 __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, const LeanPlan& lp, const gj_bwd_io& io,
                                                     uint32_t a, float s, float tinf, float cur, float nxt, float ttn,
                                                     float ty, float v, int cls, float gs_o, float ginf_o, float gtinf_o,
                                                     float gcur_o, float gnxt_o, float gttn_o, float inv_tau, float dead,
                                                     float g_deaths, const float* __restrict__ gred_age,
                                                     const ProbRow* __restrict__ prob, float (&acc)[GJ_MAX_CHANNELS],
-                                                    const uint32_t* __restrict__ orig_id, uint32_t soff = 0u) {
+                                                    const uint32_t* __restrict__ orig_id, uint32_t soff = 0u,
+                                                    float glab_i = 0.0f, float glab_d = 0.0f) {
     // soff: batched ensemble — this sample's offset into the per-sample arrays (outputs below); the agent's id in the
     // world and in the noise stream stays `a`
     const int age = age_of(cls);
@@ -1019,6 +1024,7 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
                                         [&](int) { return draw_step_normal(seed, call, ga()); });
     float gc = gcur_o;
     if (so.cur == dead) gc += g_deaths;
+    if (kLabel && so.cur == dead) gc += glab_d;
     float gcur1 = gc, gnxt1 = gnxt_o;
     if (so.branch == 1) {
       gcur1 += (gnxt_o + gttn_o * so.dwell) / (float)so.stage;
@@ -1032,7 +1038,8 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
     const float g_ttn = gttn_o * (1.0f - n);
     float gn = gnxt1 * (2.0f - nxt) + gttn_o * (p.now - ttn);
     // reductions and infect^T
-    const float gi = ginf_o + gred_age[age];
+    float gi = ginf_o + gred_age[age];
+    if (kLabel) gi += glab_i;
     const float dd = s - n;
     const float wgt = (dd > 0.0f) ? 1.0f : ((dd == 0.0f) ? 0.5f : 0.0f);  // maximum(0, x): ties split 1/2
     float g_s = gs_o * wgt;
@@ -1073,7 +1080,7 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
 // B1  backward, per agent: symptoms^T, infect^T, sampler^T, clamp/exp chain -> cotangents of the state,
 //     w = dL/dLambda * s (and its quarantine-masked copy), partial sums of the cell channels (as in K1)
 // =====================================================================================================
-template <bool kQuar>
+template <bool kQuar, bool kLabel>
 __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
                                                                    gj_bwd_io io, float* __restrict__ tile_part) {
   __shared__ ProbRow prob[200];
@@ -1144,9 +1151,15 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backwar
       for (int h = 0; h < kLeanBatch; ++h) {
         const uint32_t a = base + h * kLeanThreads;
         if (a >= a1) break;
-        lean_backward_agent<kQuar>(p, lp, io, a, s[h], tinf[h], cur[h], nxt[h], ttn[h], ty[h], v[h], cls[h], gs_o[h],
-                                   ginf_o[h], gtinf_o[h], gcur_o[h], gnxt_o[h], gttn_o[h], inv_tau, dead, g_deaths,
-                                   gred_age, prob, acc, w.orig_id);
+        float glab_i = 0.0f, glab_d = 0.0f;
+        if (kLabel) {
+          const int64_t l = io.label[a];
+          glab_i = io.g_red_label[2 * l];
+          glab_d = io.g_red_label[2 * l + 1] / dead;
+        }
+        lean_backward_agent<kQuar, kLabel>(p, lp, io, a, s[h], tinf[h], cur[h], nxt[h], ttn[h], ty[h], v[h], cls[h],
+                                           gs_o[h], ginf_o[h], gtinf_o[h], gcur_o[h], gnxt_o[h], gttn_o[h], inv_tau,
+                                           dead, g_deaths, gred_age, prob, acc, w.orig_id, 0u, glab_i, glab_d);
       }
     }
     if (lp.n_cell > 0) {

@@ -247,13 +247,14 @@ __device__ __forceinline__ void pipe_fwd_issue(PipeFwdStageT<kBatch>& sg, uint64
   bulk_g2s(sg.cls, w.cls + t.lo16, t.hi16 - t.lo16, bar);
 }
 
-template <bool kQuar, bool kDiag, bool kNext, bool kBatch>
+template <bool kQuar, bool kDiag, bool kNext, bool kBatch, bool kLabel>
 __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
                                                                  gj_fwd_io io, const float* __restrict__ cell_buf,
                                                                  double* __restrict__ red_part,
                                                                  unsigned int* __restrict__ ticket, NextStep nx,
                                                                  Batch bt) {
   static_assert(!(kNext && kBatch), "the look-ahead transmission pass is not batched");
+  static_assert(!(kNext && kLabel), "a step with a label table runs without the look-ahead");
   extern __shared__ __align__(128) unsigned char pipe_smem[];
   PipeFwdSharedT<kNext, kBatch>& sh = *reinterpret_cast<PipeFwdSharedT<kNext, kBatch>*>(pipe_smem);
   const BatchCta bc = batch_cta<kBatch>(bt);
@@ -261,11 +262,13 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
   const uint32_t so = bc.so;
   float* __restrict__ red_out = io.red;
   const float* __restrict__ beta_in = io.beta;
+  uint32_t* __restrict__ lacc = io.label_acc;
   if (kBatch) {   // this sample's slices of the scratch and of the small per-sample arrays
     cell_buf = scr_shift(cell_buf, bt, bc.s);
     red_part = scr_shift(red_part, bt, bc.s);
     ticket = scr_shift(ticket, bt, bc.s);
     if (red_out) red_out += (int64_t)bc.s * bt.sRed;
+    if (kLabel) lacc += bc.s * bt.sLab;
     beta_in += (int64_t)bc.s * bt.sBeta;
   }
   const TileRun run = lean_tiles(w, bc);
@@ -345,6 +348,7 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
                                                         sg.s[i], sg.inf[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i], cls,
                                                         inv_tau, dead, sh.hist, &sh.deaths, kBatch && noise != nullptr,
                                                         (kBatch && noise) ? sg.dE[i] : 0.0f);
+      if (kLabel) label_add(lacc, io.label, a, (uint32_t)o.inf, o.cur == dead ? 1u : 0u);
       if (kNext) {   // TransmissionUpdater of the next step (same arithmetic as k_lean_transmission)
         float T = 0.0f;
         if (o.inf != 0.0f) {
@@ -439,7 +443,7 @@ __device__ __forceinline__ void pipe_bwd_issue(PipeBwdStage& sg, uint64_t* bar, 
 constexpr int kBwdThreads = GJ_PIPE_BWD_THREADS;
 constexpr int kBwdPer = kPipeTile / kBwdThreads;
 constexpr int kBwdCtas = kBwdThreads == 256 ? 3 : 2;
-template <bool kQuar, bool kBatch>
+template <bool kQuar, bool kBatch, bool kLabel>
 __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
                                                                   gj_bwd_io io, float* __restrict__ tile_part,
                                                                   Batch bt) {
@@ -448,9 +452,11 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
   const BatchCta bc = batch_cta<kBatch>(bt);
   const uint32_t so = bc.so;
   const float* __restrict__ g_red = io.g_red;
+  const float* __restrict__ g_lab = io.g_red_label;
   if (kBatch) {
     tile_part = scr_shift(tile_part, bt, bc.s);
     if (g_red) g_red += (int64_t)bc.s * bt.sRed;
+    if (kLabel) g_lab += bc.s * bt.sLab;
   }
   const TileRun run = lean_tiles(w, bc);
   const BwdCot cot{{io.g_s_o, io.g_inf_o, io.g_tinf_o, io.g_cur_o, io.g_nxt_o, io.g_ttn_o}};
@@ -493,12 +499,14 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
     mbar_wait(&sh.full[stg], parity);
     // the cotangents of the state outputs stream through registers
     float c[kBwdPer][6];
+    int32_t lab[kBwdPer];   // label codes (kLabel), fetched with the cotangents
 #pragma unroll
     for (int h = 0; h < kBwdPer; ++h) {
       const uint32_t a = a0 + threadIdx.x + h * kBwdThreads;
       const uint32_t al = a < a1 ? a : a0;
 #pragma unroll
       for (int k = 0; k < 6; ++k) c[h][k] = cot.p[k] ? cot.p[k][al + so] : 0.0f;
+      if (kLabel) lab[h] = io.label[al];
     }
     const uint32_t sk = a0 & 3u, sk16 = a0 & 15u;
 #pragma unroll
@@ -506,9 +514,12 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
       const uint32_t j = threadIdx.x + h * kBwdThreads;
       const uint32_t a = a0 + j, i = j + sk;
       if (a >= a1) break;
-      lean_backward_agent<kQuar>(p, lp, io, a, sg.s[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i], sg.ty[i], sg.v[i],
-                                 sg.cls[j + sk16], c[h][0], c[h][1], c[h][2], c[h][3], c[h][4], c[h][5], inv_tau, dead,
-                                 g_deaths, sh.gred_age, sh.prob, acc, w.orig_id, so);
+      const float glab_i = kLabel ? g_lab[2 * (int64_t)lab[h]] : 0.0f;
+      const float glab_d = kLabel ? g_lab[2 * (int64_t)lab[h] + 1] / dead : 0.0f;
+      lean_backward_agent<kQuar, kLabel>(p, lp, io, a, sg.s[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i], sg.ty[i],
+                                         sg.v[i], sg.cls[j + sk16], c[h][0], c[h][1], c[h][2], c[h][3], c[h][4], c[h][5],
+                                         inv_tau, dead, g_deaths, sh.gred_age, sh.prob, acc, w.orig_id, so, glab_i,
+                                         glab_d);
     }
     if (pipe_release() && tile + kPipeStages < run.t1)
       pipe_bwd_issue(sg, &sh.full[stg], w, io, tile + kPipeStages, so);

@@ -43,6 +43,7 @@ struct Batch {
   int64_t sScr;    // stride of the scratch buffers (bytes, multiple of 256)
   int sBeta, sRed; // strides of beta / g_beta and red / g_red (elements)
   const float* noise;  // [n_agents] the draw's Gumbel noise difference, evaluated once for all samples; NULL = in-kernel
+  int64_t sLab;        // stride of red_label / g_red_label / label_acc (elements)
 };
 struct BatchCta {
   int s;           // sample of this CTA
@@ -266,8 +267,11 @@ struct AgentState {
   float s, inf, tinf, cur, nxt, ttn;
 };
 
+// kLabel: also add the agent's cases and death indicator to its label's column of the integer accumulator lacc
+template <bool kLabel = false>
 __device__ __forceinline__ void forward_tail(const gj_step_params& p, const gj_fwd_io& io, int64_t N, int64_t a,
-                                             int64_t ga, int age, float q, AgentState st, float* red) {
+                                             int64_t ga, int age, float q, AgentState st, float* red,
+                                             uint32_t* lacc = nullptr) {
   const int dead = p.n_stages - 1;
   if (p.mode == GJ_MODE_SEED) q = 1.0f - io.seed_fraction[0] * 1.0f;  // infection.py:36-40
   float n = 0.0f;
@@ -321,6 +325,7 @@ __device__ __forceinline__ void forward_tail(const gj_step_params& p, const gj_f
     for (int b = 0; b < GJ_MAX_AGE_BINS; ++b)
       if (b < p.n_age_bins && age > p.age_bins[b] && age < p.age_bins[b + 1]) red[2 + b] += st.inf;
   }
+  if (kLabel) label_add(lacc, io.label, a, (uint32_t)st.inf, st.cur == (float)dead ? 1u : 0u);
 }
 
 struct NetMask {
@@ -427,6 +432,7 @@ __device__ __forceinline__ Pressure agent_pressure(const gj_world_desc& w, const
   return out;
 }
 
+template <bool kLabel>
 __global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_step_params p, Plan pl, gj_fwd_io io,
                                                             const float* __restrict__ cell_buf,
                                                             double* __restrict__ red_part,
@@ -459,7 +465,7 @@ __global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_
     io.tape_v[a] = (st.s == 0.0f) ? pr.X : pr.lam;
     if (io.q) io.q[a] = q;
     if (io.lam) io.lam[a] = pr.lam;
-    forward_tail(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, red);
+    forward_tail<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, red, io.label_acc);
   }
   if (io.red) {
     double redd[kMaxRed];
@@ -480,6 +486,8 @@ struct BackAgent {
 };
 
 // symptoms^T, infect^T, sampler^T and the clamp/exp chain: shared by the generic and the tiled kernels
+// kLabel: fold in the cotangent of the forward's label table (gj_bwd_io.g_red_label) at the agent's label
+template <bool kLabel = false>
 __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, const gj_bwd_io& io, int64_t N, int64_t a,
                                                     int64_t ga, int age, const AgentState& st, bool with_networks) {
   const int dead = p.n_stages - 1;
@@ -493,6 +501,12 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
   float gcur_o = io.g_cur_o ? io.g_cur_o[a] : 0.0f;
   const float gnxt_o = io.g_nxt_o ? io.g_nxt_o[a] : 0.0f;
   const float gttn_o = io.g_ttn_o ? io.g_ttn_o[a] : 0.0f;
+  float glab_i = 0.0f, glab_d = 0.0f;   // label table: cases and deaths cotangents of the agent's column
+  if (kLabel) {
+    const int64_t l = io.label[a];
+    glab_i = io.g_red_label[2 * l];
+    glab_d = io.g_red_label[2 * l + 1] / (float)dead;
+  }
   BackAgent r;
   r.gn = io.g_n ? io.g_n[a] : 0.0f;
   r.gcur = gcur_o;
@@ -511,6 +525,7 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
     });
     // reductions fold in here: deaths = sum (cur' == dead) * cur' / dead   runner.py:204-209
     if (io.g_red && so.cur == (float)dead) gcur_o += io.g_red[1] / (float)dead;
+    if (kLabel && so.cur == (float)dead) gcur_o += glab_d;
     float gcur1 = gcur_o;
     float gnxt1 = gnxt_o;
     const float gttn1 = gttn_o;
@@ -529,6 +544,7 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
   } else if (io.g_red && st.cur == (float)dead) {
     r.gcur += io.g_red[1] / (float)dead;
   }
+  if (kLabel && !(p.phases & GJ_PHASE_SYMPTOMS) && st.cur == (float)dead) r.gcur += glab_d;
   r.gs = gs_o;
   r.ginf = ginf_o;
   r.gtinf = gtinf_o;
@@ -536,6 +552,10 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
     ginf_o += io.g_red[0];
     for (int b = 0; b < p.n_age_bins; ++b)
       if (age > p.age_bins[b] && age < p.age_bins[b + 1]) ginf_o += io.g_red[2 + b];
+    r.ginf = ginf_o;
+  }
+  if (kLabel) {
+    ginf_o += glab_i;
     r.ginf = ginf_o;
   }
   if (p.phases & GJ_PHASE_INFECT) {
@@ -581,6 +601,7 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
   return r;
 }
 
+template <bool kLabel>
 __global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj_step_params p, Plan pl, gj_bwd_io io,
                                                           float* __restrict__ tile_part) {
   __shared__ TileTables tb;
@@ -601,7 +622,7 @@ __global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj
     st.cur = io.cur ? io.cur[a] : 1.0f;
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
-    const BackAgent r = backward_agent(p, io, N, a, noise_agent(w, p, a), cls % 100, st, true);
+    const BackAgent r = backward_agent<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, true);
     const float mq = (p.n_quar > 0) ? quarantine_mask(p, st.cur) : 1.0f;
     const float wv = r.glam * st.s;
     const float wqv = r.glam * (mq * st.s);

@@ -18,7 +18,7 @@ GJ_MAX_STAGES = 16
 GJ_MAX_QUAR = 4
 GJ_MAX_AGE_BINS = 8
 GJ_MAX_CHANNELS = 8
-GJ_ABI_VERSION = 10
+GJ_ABI_VERSION = 11
 
 KIND_PLAIN, KIND_HOUSEHOLD, KIND_LEISURE, KIND_CARE_VISIT = 0, 1, 2, 3
 PHASE_NETWORKS, PHASE_SAMPLE, PHASE_INFECT, PHASE_SYMPTOMS, PHASE_ALL = 1, 2, 4, 8, 15
@@ -103,18 +103,21 @@ _BWD_FIELDS = [
 
 
 class FwdIO(C.Structure):
-    _fields_ = [(name, C.c_void_p) for name in _FWD_FIELDS]
+    # results by label: codes, column count, fp32 table and its integer accumulator
+    _fields_ = [(name, C.c_void_p) for name in _FWD_FIELDS] + [
+        ("label", C.c_void_p), ("n_labels", C.c_int32), ("_pad_label", C.c_int32), ("red_label", C.c_void_p),
+        ("label_acc", C.c_void_p)]
 
 
 class BwdIO(C.Structure):
-    _fields_ = [(name, C.c_void_p) for name in _BWD_FIELDS]
+    _fields_ = [(name, C.c_void_p) for name in _BWD_FIELDS] + [("label", C.c_void_p), ("g_red_label", C.c_void_p)]
 
 
 class Batch(C.Structure):
     """gj_batch: strides of a batched ensemble call (gj_step_forward_batch / gj_step_backward_batch)."""
     _fields_ = [("n_samples", C.c_int32), ("_pad0", C.c_int32), ("agent_stride", C.c_int64),
                 ("group_stride", C.c_int64), ("beta_stride", C.c_int64), ("red_stride", C.c_int64),
-                ("scratch_stride", C.c_int64), ("noise", C.c_void_p)]
+                ("scratch_stride", C.c_int64), ("noise", C.c_void_p), ("label_stride", C.c_int64)]
 
 
 class GradJuneLibraryError(RuntimeError):

@@ -116,6 +116,7 @@ def world_from_june_arrays(f: Mapping, k_leisure: int = 3, load_leisure: bool = 
     agent.socioeconomic_index = torch.as_tensor(
         np.digitize(np.asarray(geo["area_socioeconomic_indices"][:])[area_ids], bins), dtype=torch.int8)
     agent.area = _as_str(np.asarray(geo["area_name"][:])[area_ids])
+    agent.super_area = torch.as_tensor(np.asarray(pop["super_area"][:]).astype(np.int64))   # results_by: super_area
     sexes = _as_str(pop["sex"][:])
     agent.sex = torch.as_tensor((sexes == "f").astype(np.int64))                # "m" -> 0, "f" -> 1
     return data

@@ -91,9 +91,11 @@ class GradJune(torch.nn.Module):
         return spec, nets
 
     def step(self, data, timer, age_bins=None, mode=ops.MODE_STEP, seed_fraction=None, noise=None, want_probs=True,
-             next_timer=None):
+             next_timer=None, label=None):
         """Fused step; returns (data, reductions) where reductions = [cases, deaths, cases by age bin...]
-        (None unless ``age_bins`` is given).  ``want_probs=False`` skips the two diagnostic per-agent outputs
+        (None unless ``age_bins`` is given).  With ``label`` (:class:`grad_june.ops.Labels`) it returns
+        (data, reductions, label_table): the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched),
+        reduced inside the step kernels.  ``want_probs=False`` skips the two diagnostic per-agent outputs
         (``not_infected_probs``, ``new_infected``) that the reference keeps only as locals of its forward.
         ``next_timer``: the timer as it will be at the FOLLOWING call (the driver knows the schedule): the
         kernels then run that step's transmission pass inside this one (used only if the next call matches)."""
@@ -102,7 +104,7 @@ class GradJune(torch.nn.Module):
         dev = agent.susceptibility.device
         if mode == ops.MODE_STEP and self.infection_networks.has_custom(
                 self.infection_networks.active_networks(timer, self.policies)):
-            return self._step_modular(data, timer, age_bins)
+            return self._step_modular(data, timer, age_bins, label)
         static, rows = self._static(data, dev)
         policies = self.policies
         spec, nets = self._spec(timer, rows, age_bins, mode, want_probs)
@@ -114,7 +116,7 @@ class GradJune(torch.nn.Module):
                  "cur": sym["current_stage"], "nxt": sym["next_stage"], "ttn": sym["time_to_next_stage"]}
         beta = beta_vector(nets, policies, timer, dev) if nets else None
         out = ops.infection_step(static, spec, beta, state, seed_fraction=seed_fraction, noise=noise,
-                                 next_spec=next_spec)
+                                 next_spec=next_spec, label=label)
         if out["T"] is not None:
             agent.transmission = out["T"]
         agent.susceptibility = out["s"]
@@ -127,9 +129,11 @@ class GradJune(torch.nn.Module):
             data["agent"]["new_infected"] = out["n"]
         if out["q"] is not None:
             data["agent"]["not_infected_probs"] = out["q"]
+        if label is not None:
+            return data, out["red"], out["red_label"]
         return data, out["red"]
 
-    def _step_modular(self, data, timer, age_bins):
+    def _step_modular(self, data, timer, age_bins, label=None):
         """The reference's own sequencing (model.py:112-144), module by module, for steps with a user-defined network
         subclass (its masking hooks return arbitrary tensors, which the fused kernels cannot evaluate in registers):
         every module is still a CUDA kernel of the library (stand-alone phases), only the fusion is lost."""
@@ -147,6 +151,14 @@ class GradJune(torch.nn.Module):
             red = [inf.sum(), ((cur == dead) * cur / dead).sum()]
             red += [(inf * ((age < hi) * (age > lo))).sum() for lo, hi in zip(age_bins[:-1], age_bins[1:])]
             red = torch.stack(red)
+        if label is not None:         # the label table as index_add of the same per-agent terms
+            cur, inf = agent.symptoms["current_stage"], agent.is_infected
+            dead = float(len(self.symptoms_updater.stages_ids) - 1)
+            idx = label.codes.long()
+            cases = torch.zeros(label.n, dtype=inf.dtype, device=inf.device).index_add(0, idx, inf)
+            deaths = (cur == dead) * cur / dead
+            deaths = torch.zeros(label.n, dtype=deaths.dtype, device=deaths.device).index_add(0, idx, deaths)
+            return data, red, torch.stack((cases, deaths.to(cases.dtype)), dim=1)
         return data, red
 
     def kernel_family(self, data, timer) -> str:

@@ -175,6 +175,45 @@ class StepSpec:
     exact_order: bool = False   # force the reference-order kernels even with in-kernel Philox noise
 
 
+@dataclass(frozen=True)
+class Labels:
+    """Per-agent label codes of a results-by-label table (cases and deaths per region, area, ...): ``codes[a]`` is
+    agent a's column in ``[0, n)``.  Build it with :func:`make_labels`, which checks the range once."""
+    codes: torch.Tensor     # [N] int32
+    n: int
+
+
+def make_labels(codes, n: int, device=None) -> Labels:
+    """Validated :class:`Labels` (the kernels index the table with the codes unchecked)."""
+    codes = torch.as_tensor(codes)
+    if codes.dim() != 1 or codes.dtype.is_floating_point or codes.dtype == torch.bool:
+        raise ValueError("label codes must be a 1-D integer array")
+    n = int(n)
+    if not 1 <= n <= 1 << 30:
+        raise ValueError(f"the number of label columns must lie in [1, 2^30], got {n}")
+    if codes.numel() and (int(codes.min()) < 0 or int(codes.max()) >= n):
+        raise ValueError(f"label codes must lie in [0, {n}), got [{int(codes.min())}, {int(codes.max())}]")
+    return Labels(codes.to(device=device or codes.device, dtype=torch.int32).contiguous(), n)
+
+
+def _label_acc(world: DeviceWorld, n: int):
+    """The integer accumulator of the label table ([n] uint32, zero; every call leaves it zero)."""
+    t = world.__dict__.get("_label_acc")
+    if t is None or t.numel() < n:
+        t = world.__dict__["_label_acc"] = torch.zeros(n, dtype=torch.int32, device=world.device)
+    return t
+
+
+def _set_labels(io, world: DeviceWorld, label: Labels, nb: int = 1):
+    """Point the io struct at the label codes, a new [nb, n, 2] table and the accumulator; returns the table."""
+    if label.codes.numel() != world.n_agents or label.codes.device != world.device:
+        raise ValueError(f"label codes must hold one entry per agent ({world.n_agents}) on {world.device}")
+    table = torch.empty(nb, label.n, 2, dtype=torch.float32, device=world.device)
+    io.label, io.n_labels, io.red_label = label.codes.data_ptr(), label.n, table.data_ptr()
+    io.label_acc = _label_acc(world, nb * 2 * label.n).data_ptr()
+    return table
+
+
 def _scratch(world: DeviceWorld):
     sc = getattr(world, "_scratch", None)
     if sc is None:
@@ -409,7 +448,7 @@ class _Step(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in,
-                seed_fraction, next_spec=None):
+                seed_fraction, next_spec=None, label: Optional[Labels] = None):
         world = static.world
         dev = world.device
         N = world.n_agents
@@ -495,6 +534,7 @@ class _Step(torch.autograd.Function):
         if spec.want_reductions:
             red = torch.empty(2 + p.n_age_bins, dtype=torch.float32, device=dev)
             io.red = red.data_ptr()
+        red_label = _set_labels(io, world, label)[0] if label is not None else None
         io.scratch = _scratch(world).data_ptr()
         desc = world.desc()
         if world.__dict__.get("_scatter_pending"):
@@ -506,7 +546,7 @@ class _Step(torch.autograd.Function):
             p.agent_offset = static.exchange.part.agent_lo
         lean_inputs = E is None and u is None and z is None and T_in is None and lam is None and static.prof4 is not None
         p_next = T_next = Tq_next = None
-        if next_spec is not None and fused_all and lean_inputs and not seed_mode:
+        if next_spec is not None and fused_all and lean_inputs and not seed_mode and label is None:
             # also run the NEXT step's transmission pass inside this step's agent kernel (gj_step_forward_next)
             p_next, _ = _fill_params(world, next_spec, static.symptoms, 0, 0)
             T_next = torch.empty(N, dtype=torch.float32, device=dev)
@@ -524,14 +564,14 @@ class _Step(torch.autograd.Function):
                 tq_name=next_tq_name if Tq_next is not None else "Tq0", inf=out.get("inf_o"), tinf=out.get("tinf_o"),
                 cur=out.get("cur_o"))
 
-        ctx.static, ctx.spec, ctx.noise_key = static, spec, (seed, call_index)
+        ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"],
                               T_in if T_in is not None else T, q_in, n_in,
                               seed_fraction, out.get("inf_o"), tape_v, tape_y0, S_un, E, u, z, q, n)
         ctx.fused_T = fused_T
         outs = (out.get("s_o"), out.get("inf_o"), out.get("tinf_o"), out.get("cur_o"), out.get("nxt_o"),
-                out.get("ttn_o"), T, q, n, red, lam)
+                out.get("ttn_o"), T, q, n, red, lam, red_label)
         nd = [t for t in (T,) if t is not None]
         if (phases & PHASE_SAMPLE) and q is not None:
             nd.append(q)   # fused: q is a by-product; its cotangent path runs through the sampler
@@ -541,7 +581,7 @@ class _Step(torch.autograd.Function):
         return outs
 
     @staticmethod
-    def backward(ctx, g_s_o, g_inf_o, g_tinf_o, g_cur_o, g_nxt_o, g_ttn_o, g_T, g_q, g_n, g_red, g_lam):
+    def backward(ctx, g_s_o, g_inf_o, g_tinf_o, g_cur_o, g_nxt_o, g_ttn_o, g_T, g_q, g_n, g_red, g_lam, g_red_label):
         static, spec = ctx.static, ctx.spec
         world = static.world
         dev, N = world.device, world.n_agents
@@ -586,6 +626,9 @@ class _Step(torch.autograd.Function):
             put("g_lam", g_lam)
         if (phases & PHASE_SAMPLE) and not (phases & PHASE_INFECT):
             put("g_n", g_n)
+        if g_red_label is not None:
+            put("g_red_label", g_red_label)
+            io.label = ctx.label.codes.data_ptr()
 
         need = ctx.needs_input_grad  # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, frac)
 
@@ -630,7 +673,7 @@ class _Step(torch.autograd.Function):
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None)
+                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None)
 
 
 # --------------------------------------------------------------------------------------
@@ -676,7 +719,8 @@ class _BatchStep(torch.autograd.Function):
     run with the same seed and beta[r]."""
 
     @staticmethod
-    def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction):
+    def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction,
+                label: Optional[Labels] = None):
         world = static.world
         dev, N = world.device, world.n_agents
         L = _lib.lib()
@@ -725,11 +769,13 @@ class _BatchStep(torch.autograd.Function):
         if spec.want_reductions:
             red = torch.empty(nb, nr, dtype=torch.float32, device=dev)
             io.red = red.data_ptr()
+        red_label = _set_labels(io, world, label, nb) if label is not None else None
+        n_lab = 2 * label.n if label is not None else 0
         scratch, scr_stride = _scratch_batch(world, nb)
         io.scratch = scratch.data_ptr()
         desc = world.desc()
         strides = {name: 4 * Np for name in _AGENT_FIELDS}
-        strides.update(red=4 * nr, scratch=scr_stride)
+        strides.update(red=4 * nr, scratch=scr_stride, red_label=4 * n_lab, label_acc=4 * n_lab)
         T = tape_v = S_un = None
         sG = K = 0
         if seed_mode:
@@ -757,21 +803,21 @@ class _BatchStep(torch.autograd.Function):
             # the samples share the Philox stream: the draw's Gumbel noise is evaluated once per agent
             noise_buf = _buffer(world, "noise_b", Np) if BATCH_SHARED_NOISE else None
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride, noise=_ptr(noise_buf))
+                            scratch_stride=scr_stride, noise=_ptr(noise_buf), label_stride=n_lab)
             with _on(dev):
                 _lib.check(L.gj_step_forward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_forward_batch")
-        ctx.static, ctx.spec, ctx.noise_key = static, spec, (seed, call_index)
+        ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
         ctx.shape = (nb, Np, sG, K, nr)
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"], T, seed_fraction,
                               out["inf_o"], tape_v, tape_y0, S_un)
         if T is not None:
             ctx.mark_non_differentiable(T)
-        return (out["s_o"], out["inf_o"], out["tinf_o"], out["cur_o"], out["nxt_o"], out["ttn_o"], T, red)
+        return (out["s_o"], out["inf_o"], out["tinf_o"], out["cur_o"], out["nxt_o"], out["ttn_o"], T, red, red_label)
 
     @staticmethod
-    def backward(ctx, g_s_o, g_inf_o, g_tinf_o, g_cur_o, g_nxt_o, g_ttn_o, g_T, g_red):
+    def backward(ctx, g_s_o, g_inf_o, g_tinf_o, g_cur_o, g_nxt_o, g_ttn_o, g_T, g_red, g_red_label):
         static, spec = ctx.static, ctx.spec
         world = static.world
         dev = world.device
@@ -801,6 +847,11 @@ class _BatchStep(torch.autograd.Function):
             g = put(name, g)
             if g is not None and name != "g_red" and tuple(g.shape) != (nb, Np):
                 raise ValueError(f"cotangent {name} has shape {tuple(g.shape)}, expected {(nb, Np)}")
+        n_lab = 0
+        if g_red_label is not None:
+            put("g_red_label", g_red_label)
+            io.label = ctx.label.codes.data_ptr()
+            n_lab = 2 * ctx.label.n
         need = ctx.needs_input_grad   # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction)
 
         def new(name):
@@ -822,7 +873,7 @@ class _BatchStep(torch.autograd.Function):
             g_frac = torch.zeros(nb, dtype=torch.float32, device=dev)
             io.g_seed_fraction = g_frac.data_ptr()
             strides = {name: 4 * Np for name in _AGENT_FIELDS}
-            strides.update(g_red=4 * nr, scratch=scr_stride, g_seed_fraction=4,
+            strides.update(g_red=4 * nr, scratch=scr_stride, g_seed_fraction=4, g_red_label=4 * n_lab,
                            seed_fraction=4 if seed_fraction.numel() == nb else 0)
             _row_calls(L.gj_step_backward, "gj_step_backward", world, desc, p, io, nb, strides, _stream(dev))
             if seed_fraction.numel() != nb:
@@ -839,7 +890,7 @@ class _BatchStep(torch.autograd.Function):
             io.wq = _buffer(world, "wq_b", nb * Np).data_ptr() if p.n_quar > 0 else io.w
             io.R, io.cR = _buffer(world, "R_b", nb * sG).data_ptr(), _buffer(world, "cR_b", nb * sG).data_ptr()
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride)
+                            scratch_stride=scr_stride, label_stride=n_lab)
             with _on(dev):
                 _lib.check(L.gj_step_backward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_backward_batch")
@@ -848,13 +899,14 @@ class _BatchStep(torch.autograd.Function):
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_frac if (seed_mode and need[10]) else None)
+                g_frac if (seed_mode and need[10]) else None, None)
 
 
 def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=None, q_in=None, n_in=None,
-                   seed_fraction=None, noise=None, next_spec=None):
+                   seed_fraction=None, noise=None, next_spec=None, label: Optional[Labels] = None):
     """Run one (fused or partial) step.  ``state``: s, inf, tinf, cur, nxt, ttn (any may be None when
-    the phases do not need it).  Returns a dict with s, inf, tinf, cur, nxt, ttn, T, q, n, red."""
+    the phases do not need it).  Returns a dict with s, inf, tinf, cur, nxt, ttn, T, q, n, red and red_label:
+    with ``label`` the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched), else None."""
     world = static.world
     if world.device.type != "cuda":
         raise _lib.GradJuneLibraryError(
@@ -869,12 +921,13 @@ def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=N
         if T_in is not None or q_in is not None or n_in is not None or static.exchange is not None:
             raise _lib.GradJuneLibraryError("batched ensembles run the whole fused step on an unpartitioned world")
         outs = _BatchStep.apply(static, spec, noise, beta, state["s"], state["inf"], state["tinf"], state["cur"],
-                                state["nxt"], state["ttn"], seed_fraction)
-        names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "red")
+                                state["nxt"], state["ttn"], seed_fraction, label)
+        names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "red", "red_label")
         ret = dict(zip(names, outs))
         ret.update(q=None, n=None, lam=None)
         return ret
     outs = _Step.apply(static, spec, noise, beta, state.get("s"), state.get("inf"), state.get("tinf"),
-                       state.get("cur"), state.get("nxt"), state.get("ttn"), T_in, q_in, n_in, seed_fraction, next_spec)
-    names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "q", "n", "red", "lam")
+                       state.get("cur"), state.get("nxt"), state.get("ttn"), T_in, q_in, n_in, seed_fraction, next_spec,
+                       label)
+    names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "q", "n", "red", "lam", "red_label")
     return dict(zip(names, outs))

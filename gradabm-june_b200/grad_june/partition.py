@@ -401,6 +401,18 @@ def all_reduce_sum(x, part: Optional[Partition]):
     return _AllReduceSum.apply(x, part.process_group)
 
 
+def label_union(values: np.ndarray, part: Optional[Partition]) -> np.ndarray:
+    """Sorted union over the ranks of each rank's distinct label values (one all-gather): every rank of a partitioned
+    world then has the same result columns."""
+    if part is None or part.world_size == 1:
+        return np.unique(values)
+    import torch.distributed as dist
+
+    gathered = [None] * part.world_size
+    dist.all_gather_object(gathered, np.asarray(values), group=part.process_group)
+    return np.unique(np.concatenate(gathered))
+
+
 def exchange_for(data, world):
     """The BoundaryExchange of a partitioned world (cached on the data object), or None."""
     part = data.__dict__.get("_gj_partition")

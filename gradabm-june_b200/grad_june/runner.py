@@ -16,7 +16,7 @@ import yaml
 
 from . import ops
 from .model import GradJune
-from .partition import all_reduce_sum
+from .partition import all_reduce_sum, label_union
 from .paths import ensure_default_config
 from .timer import Timer
 from .transmission import PROFILE_KEYS, TransmissionSampler
@@ -27,9 +27,28 @@ _STATE_KEYS = ("susceptibility", "is_infected", "infection_time", "transmission"
 _SYMPTOM_KEYS = ("current_stage", "next_stage", "time_to_next_stage")
 
 
+def agent_labels(values, n_agents):
+    """A per-agent label attribute (1-D torch / numpy array of integers or strings) as a numpy array of ``n_agents``
+    entries; a one-element array applies to every agent."""
+    a = values.detach().cpu().numpy() if torch.is_tensor(values) else np.asarray(values)
+    if a.ndim != 1 or a.shape[0] not in (1, n_agents):
+        raise ValueError(f"a label attribute must be a 1-D array of 1 or {n_agents} entries, got shape {a.shape}")
+    return np.broadcast_to(a, (n_agents,)) if a.shape[0] == 1 else a
+
+
+def label_codes(labels, columns):
+    """Column of every label in the sorted ``columns``; a label that is not a column raises."""
+    codes = np.searchsorted(columns, labels)
+    hit = codes < len(columns)
+    hit[hit] = columns[codes[hit]] == labels[hit]
+    if not hit.all():
+        raise ValueError(f"label {labels[~hit][0]!r} is not one of the result columns")
+    return codes
+
+
 class Runner(torch.nn.Module):
     def __init__(self, model, data, timer, log_fraction_initial_cases, save_path, parameters,
-                 age_bins=(0, 18, 65, 100)):
+                 age_bins=(0, 18, 65, 100), results_by=None):
         super().__init__()
         self.model = model
         self.data = data
@@ -44,6 +63,14 @@ class Runner(torch.nn.Module):
         self.population_by_age = self.get_people_by_age()
         self.save_path = Path(save_path)
         self.input_parameters = parameters
+        # results by label (``results_by: super_area``): cases and deaths per value of data["agent"][results_by] and
+        # timestep, reduced inside the step kernels.  The columns are the sorted distinct values, over every rank of a
+        # partitioned world.
+        self.results_by = results_by
+        self.result_labels = None
+        if results_by is not None:
+            labels = agent_labels(data["agent"][results_by], self.n_agents)
+            self.result_labels = label_union(np.unique(labels), data.__dict__.get("_gj_partition"))
         # batched ensemble (SURVEY 8e-2): ``runner.batch = b`` makes ``forward()`` step b independent samples of the
         # epidemic at once — the networks' ``log_beta`` then hold b values each, the state tensors are [b, Np] and
         # every result series is [T+1, b].  All samples draw the same noise (common random numbers).
@@ -65,6 +92,7 @@ class Runner(torch.nn.Module):
             save_path=params["save_path"],
             parameters=params,
             age_bins=params.get("age_bins_to_save", (0, 18, 65, 100)),
+            results_by=params.get("results_by"),
         )
 
     @staticmethod
@@ -155,11 +183,25 @@ class Runner(torch.nn.Module):
             return self._fraction_cache[1]
         return fraction.reshape(1).to(device=dev, dtype=torch.float32)
 
+    def _labels(self):
+        """ops.Labels of ``results_by`` on the device (built once per label array and device, like
+        ``_ethnicity_codes``), or None."""
+        if self.results_by is None:
+            return None
+        values = self.data["agent"][self.results_by]
+        dev = self.data["agent"].susceptibility.device
+        hit = self.__dict__.get("_label_codes")
+        if hit is None or hit[0] is not values or hit[1] != dev:
+            codes = label_codes(agent_labels(values, self.n_agents), self.result_labels)
+            hit = self.__dict__["_label_codes"] = (values, dev, ops.make_labels(codes, len(self.result_labels), dev))
+        return hit[2]
+
     def set_initial_cases(self):
-        """infect_fraction_of_people + first symptoms update (runner.py:138-149) as one fused call."""
-        _, red = self.model.step(self.data, self.timer, age_bins=self._age_bins_host, mode=ops.MODE_SEED,
-                                 seed_fraction=self._fraction_tensor())
-        return red
+        """infect_fraction_of_people + first symptoms update (runner.py:138-149) as one fused call (with
+        ``results_by``: returns (reductions, label table))."""
+        out = self.model.step(self.data, self.timer, age_bins=self._age_bins_host, mode=ops.MODE_SEED,
+                              seed_fraction=self._fraction_tensor(), label=self._labels())
+        return out[1] if self.results_by is None else out[1:]
 
     def forward(self):
         timer, model, data = self.timer, self.model, self.data
@@ -170,7 +212,14 @@ class Runner(torch.nn.Module):
             raise RuntimeError("batched ensembles run on a CUDA device only")
         else:
             self.restore_initial_data()
-        reds = [self.set_initial_cases()]
+        label = self._labels()
+        reds, tabs = [], []
+        first = self.set_initial_cases()
+        if label is None:
+            reds.append(first)
+        else:
+            reds.append(first[0])
+            tabs.append(first[1])
         dates = [timer.date]
         while timer.date < timer.final_date:
             next(timer)
@@ -178,11 +227,15 @@ class Runner(torch.nn.Module):
             if timer.date < timer.final_date:      # the schedule is known: tell the step what the next one will be
                 ahead = copy.copy(timer)
                 next(ahead)
-            data, red = model.step(data, timer, age_bins=self._age_bins_host, want_probs=False, next_timer=ahead)
-            reds.append(red)
+            out = model.step(data, timer, age_bins=self._age_bins_host, want_probs=False, next_timer=ahead, label=label)
+            data = out[0]
+            reds.append(out[1])
+            if label is not None:
+                tabs.append(out[2])
             dates.append(timer.date)
+        part = data.__dict__.get("_gj_partition")
         table = torch.stack(reds)                      # [T+1, 2 + n_bins]   (batched: [T+1, b, 2 + n_bins])
-        table = all_reduce_sum(table, data.__dict__.get("_gj_partition"))   # partitioned world: sum over ranks
+        table = all_reduce_sum(table, part)            # partitioned world: sum over ranks
         ex = data.__dict__.get("_gj_cache", {}).get("exchange")
         if ex is not None and not torch.cuda.is_current_stream_capturing():
             ex.check()      # a peer that never arrived at an exchange must not go unnoticed (once per window)
@@ -197,6 +250,10 @@ class Runner(torch.nn.Module):
         }
         for i, key in enumerate(self._age_bins_host[1:]):
             results[f"cases_by_age_{key:02d}"] = table[..., 2 + i]
+        if label is not None:
+            by = all_reduce_sum(torch.stack(tabs), part)   # [T+1, R, 2]   (batched: [T+1, b, R, 2])
+            results[f"cases_by_{self.results_by}"] = by[..., 0]
+            results[f"deaths_by_{self.results_by}"] = by[..., 1]
         is_infected = data["agent"].is_infected
         if is_infected.dim() == 2:                      # batched: [b, Np] -> [b, n_agents] in the loaded order
             is_infected = original_order(data, is_infected[:, : self.n_agents].t()).t()
@@ -205,12 +262,20 @@ class Runner(torch.nn.Module):
 
     def save_results(self, results, is_infected):
         self.save_path.mkdir(exist_ok=True, parents=True)
+        by = () if self.results_by is None else (f"cases_by_{self.results_by}", f"deaths_by_{self.results_by}")
         df = pd.DataFrame(index=results["dates"])
         df.index.name = "date"
         for key, value in results.items():
-            if key != "dates":
+            if key != "dates" and key not in by:
                 df[key] = value.detach().cpu().numpy()
         df.to_csv(self.save_path / "results.csv")
+        if by:      # long format: one row per (date, label)
+            cases, deaths = (results[k].detach().cpu().numpy() for k in by)
+            n_dates, n_labels = cases.shape
+            pd.DataFrame({"date": np.repeat(np.asarray(results["dates"]), n_labels),
+                          "label": np.tile(self.result_labels, n_dates),
+                          "cases": cases.reshape(-1), "deaths": deaths.reshape(-1)}).to_csv(
+                self.save_path / f"results_by_{self.results_by}.csv", index=False)
         pd.DataFrame({"is_infected": is_infected.detach().cpu().numpy()}).to_csv(
             self.save_path / "results_is_infected.csv")
 

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GJ_ABI_VERSION 10
+#define GJ_ABI_VERSION 11
 
 #define GJ_MAX_TYPES 8      /* edge types (household, company, school, university, care_home, leisure, ...) */
 #define GJ_MAX_NETS 16      /* infection networks active in one step */
@@ -291,6 +291,18 @@ typedef struct gj_fwd_io {
    * when the next step has an active quarantine */
   float* T_next;
   float* Tq_next;
+  /* results by label (cases and deaths per region, area, ...; NULL = off): label[a] is agent a's column in
+   * [0, n_labels).  Every kernel that writes `red` also adds the agent's post-step is_infected and its death indicator
+   * (current_stage == dead) to red_label[label[a]][0] / [1].  The sums are exact: they are accumulated as integers in
+   * label_acc and converted to fp32 once per step, so they are independent of the summation order and sum over the
+   * columns to red[0] / red[1].  Label codes must lie in [0, n_labels): they are not checked on the device.  A call with
+   * a label table does not produce the look-ahead of gj_step_forward_next. */
+  const int32_t* label;  /* [N] */
+  int32_t n_labels;      /* 1 .. 2^30 */
+  int32_t _pad_label;
+  float* red_label;      /* [n_labels][2] cases, deaths */
+  uint32_t* label_acc;   /* [n_labels][2] integer workspace, zero-initialised once by the caller; the library leaves it
+                            zeroed (gj_scratch_bytes depends on the world only, so it cannot cover it) */
 } gj_fwd_io;
 
 typedef struct gj_bwd_io {
@@ -331,6 +343,11 @@ typedef struct gj_bwd_io {
   float* R;   /* [sum_k G(type_k) + n_groups], laid out like S_unscaled */
   float* cR;  /* [sum_k G(type_k) + n_groups] */
   void* scratch;
+  /* results by label: the forward's label codes and the cotangent of its red_label ([n_labels][2]); both non-NULL
+   * adds g_red_label[label[a]][0] to the cotangent of agent a's post-step is_infected and g_red_label[label[a]][1] / dead
+   * to that of its post-step current_stage where it equals dead; NULL = no label table */
+  const int32_t* label;
+  const float* g_red_label;
 } gj_bwd_io;
 
 /* ---- library ---------------------------------------------------------------------------- */
@@ -379,8 +396,10 @@ int gj_step_backward(const gj_world_desc* w, const gj_step_params* p, const gj_b
  *   group-sum buffers (S_scaled, S_unscaled, R, cR)                                   + s * group_stride  elements
  *   beta, g_beta                                                                      + s * beta_stride   elements
  *   red, g_red                                                                        + s * red_stride    elements
+ *   red_label, g_red_label, label_acc                                                 + s * label_stride  elements
  *   scratch                                                                           + s * scratch_stride bytes
- * while the world (index words, classes, tiles), the packed infectiousness profile and the lookup tables are shared.
+ * while the world (index words, classes, tiles), the label codes, the packed infectiousness profile and the lookup
+ * tables are shared.
  * The CTAs of the b samples that walk the same run of agent tiles are launched next to each other (block index =
  * run * b + sample) and advance in step, so the tile's index words, class bytes and profile are fetched from HBM once
  * and served to the other b-1 samples out of L2: one index read per b samples.  All samples draw the SAME Philox
@@ -403,6 +422,8 @@ typedef struct gj_batch {
    * buffer, gj_step_forward_batch evaluates it ONCE per agent (one small kernel) and the b samples read it, instead
    * of every sample regenerating it.  Same arithmetic: results are bit-identical.  NULL = every sample computes it. */
   float* noise;
+  /* stride of red_label / g_red_label / label_acc (elements, >= 2 * n_labels when a label table is given) */
+  int64_t label_stride;
 } gj_batch;
 int gj_step_forward_batch(const gj_world_desc* w, const gj_step_params* p, const gj_fwd_io* io, const gj_batch* batch,
                           void* stream);
