@@ -44,12 +44,12 @@ static int bad(const char* what) {
 enum KernelId {
   K_TRANSMISSION = 0, K_GROUP_SMALL_F, K_GROUP_CHUNK_F, K_GROUP_FIX_F, K_AGENT_FWD,
   K_AGENT_BWD, K_GROUP_SMALL_B, K_GROUP_CHUNK_B, K_GROUP_FIX_B, K_DBETA, K_AGENT_BWD_GATHER, K_CELL, K_OTHER, K_SEED,
-  K_EXCHANGE, K_COUNT
+  K_EXCHANGE, K_SEED_GRAD, K_COUNT
 };
 static const char* kKernelNames[K_COUNT] = {
   "transmission", "group_small<fwd>", "group_chunk<fwd>", "group_fix<fwd>", "agent_forward",
   "agent_backward", "group_small<bwd>", "group_chunk<bwd>", "group_fix<bwd>", "dbeta",
-  "backward_gather", "cell_groups+gather", "other", "seeding", "boundary_exchange"};
+  "backward_gather", "cell_groups+gather", "other", "seeding", "boundary_exchange", "seed_label_grad"};
 constexpr int kMaxProfiled = 16384;
 struct Profiler {
   bool on = false;
@@ -416,10 +416,10 @@ __device__ __forceinline__ void block_reduce_finish(double (&v)[kR], int nr, dou
 // agent-major kernels for calls WITHOUT the networks phase (stand-alone sampler / infect / symptoms and the
 // seeding step): persistent grid-stride loop, reductions finished by the last CTA
 // ================================================================================================
-template <bool kLabel>
-__global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_step_params p, gj_fwd_io io,
-                                                          double* __restrict__ red_part,
-                                                          unsigned int* __restrict__ ticket) {
+// kSeed: seeding by label (gj_fwd_io.seed_label / gj_bwd_io.seed_label)
+template <bool kLabel, bool kSeed>
+__device__ __forceinline__ void agent_forward_body(const gj_world_desc& w, const gj_step_params& p, const gj_fwd_io& io,
+                                                   double* __restrict__ red_part, unsigned int* __restrict__ ticket) {
   const int64_t N = w.n_agents;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   float redf[kMaxRed];   // per-thread sums of small integers (<= 2 per agent, < 2^24 agents per thread): exact in fp32
@@ -435,7 +435,7 @@ __global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_st
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
     const float q = io.q_in ? io.q_in[a] : 1.0f;
-    forward_tail<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, redf, io.label_acc);
+    forward_tail<kLabel, kSeed>(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, redf, io.label_acc);
   }
   if (io.red) {
     double red[kMaxRed];
@@ -446,9 +446,24 @@ __global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_st
 }
 
 template <bool kLabel>
-__global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_step_params p, gj_bwd_io io,
-                                                           double* __restrict__ red_part,
-                                                           unsigned int* __restrict__ ticket) {
+__global__ void __launch_bounds__(kBlock) k_agent_forward(gj_world_desc w, gj_step_params p, gj_fwd_io io,
+                                                          double* __restrict__ red_part,
+                                                          unsigned int* __restrict__ ticket) {
+  agent_forward_body<kLabel, false>(w, p, io, red_part, ticket);
+}
+
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock) k_agent_seed_forward(gj_world_desc w, gj_step_params p, gj_fwd_io io,
+                                                               double* __restrict__ red_part,
+                                                               unsigned int* __restrict__ ticket) {
+  agent_forward_body<kLabel, true>(w, p, io, red_part, ticket);
+}
+
+// kSeed: each agent's d/dseed_fraction goes to the scratch row io.seed_work (reduced per label by k_seed_label_grad)
+// instead of the single fp64 sum
+template <bool kLabel, bool kSeed>
+__device__ __forceinline__ void agent_backward_body(const gj_world_desc& w, const gj_step_params& p, const gj_bwd_io& io,
+                                                    double* __restrict__ red_part, unsigned int* __restrict__ ticket) {
   const int64_t N = w.n_agents;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   double gfrac[1] = {0.0};
@@ -462,10 +477,11 @@ __global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_s
     st.cur = io.cur ? io.cur[a] : 1.0f;
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
-    const BackAgent r = backward_agent<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, false);
+    const BackAgent r = backward_agent<kLabel, kSeed>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, false);
     if (io.g_q_out) io.g_q_out[a] = r.gq;
     if (io.g_n_out) io.g_n_out[a] = r.gn;
-    if (seed_mode) gfrac[0] += (double)(-r.gq);  // q = 1 - fraction
+    if (kSeed) io.seed_work[a] = -r.gq;
+    else if (seed_mode) gfrac[0] += (double)(-r.gq);  // q = 1 - fraction
     if (io.g_s) io.g_s[a] = r.gs;
     if (io.g_inf) io.g_inf[a] = r.ginf;
     if (io.g_tinf) io.g_tinf[a] = r.gtinf;
@@ -473,7 +489,85 @@ __global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_s
     if (io.g_nxt) io.g_nxt[a] = r.gnxt;
     if (io.g_ttn) io.g_ttn[a] = r.gttn;
   }
-  if (seed_mode && io.g_seed_fraction) block_reduce_finish<1>(gfrac, 1, red_part, ticket, io.g_seed_fraction);
+  if (!kSeed && seed_mode && io.g_seed_fraction) block_reduce_finish<1>(gfrac, 1, red_part, ticket, io.g_seed_fraction);
+}
+
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock) k_agent_backward(gj_world_desc w, gj_step_params p, gj_bwd_io io,
+                                                           double* __restrict__ red_part,
+                                                           unsigned int* __restrict__ ticket) {
+  agent_backward_body<kLabel, false>(w, p, io, red_part, ticket);
+}
+
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock) k_agent_seed_backward(gj_world_desc w, gj_step_params p, gj_bwd_io io,
+                                                                double* __restrict__ red_part,
+                                                                unsigned int* __restrict__ ticket) {
+  agent_backward_body<kLabel, true>(w, p, io, red_part, ticket);
+}
+
+// ================================================================================================
+// seeding by label: g_seed_fraction[l] = sum of seed_work over the agents of label l, deterministically.
+// seed_order lists the agents stably sorted by label; label l owns positions [offsets[l], offsets[l+1]).  The positions
+// are cut into fixed chunks of `chunk` (a power of two that depends on the world only).  One warp per chunk sums, in
+// fp64 with a fixed lane order and shuffle tree, each label's piece of the chunk: a label that lies inside the chunk is
+// finished there; a label that crosses a chunk boundary leaves its piece in one of the chunk's two partial slots —
+// slot 0 for the label that holds the chunk's first position, slot 1 for a label that starts inside the chunk and
+// runs past its end.  k_seed_label_fix then adds a crossing label's pieces in chunk order.  Nothing depends on the
+// launch grid, and there are no floating-point atomics.
+// ================================================================================================
+__global__ void __launch_bounds__(kBlock) k_seed_label_grad(int64_t N, int64_t chunk, const int32_t* __restrict__ order,
+                                                            const int32_t* __restrict__ offsets, int n_labels,
+                                                            const float* __restrict__ work, double* __restrict__ part,
+                                                            float* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n_chunks = (N + chunk - 1) / chunk;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < n_chunks; c += warps) {
+    const int64_t lo = c * chunk, hi = lo + chunk < N ? lo + chunk : N;
+    int l0 = 0, l1 = n_labels;   // the label holding position lo: the last l with offsets[l] <= lo
+    while (l1 - l0 > 1) {
+      const int m = (l0 + l1) >> 1;
+      if ((int64_t)offsets[m] <= lo) l0 = m;
+      else l1 = m;
+    }
+    int l = l0;
+    int64_t pos = lo;
+    while (pos < hi) {
+      while ((int64_t)offsets[l + 1] <= pos) ++l;   // skip empty labels
+      const int64_t b = offsets[l], e = offsets[l + 1];
+      const int64_t end = e < hi ? e : hi;
+      double v = 0.0;
+      for (int64_t j = pos + lane; j < end; j += 32) v += (double)work[order[j]];
+      v = warp_sum(v);
+      if (lane == 0) {
+        if (b >= lo && e <= hi) out[l] = (float)v;
+        else part[2 * c + (b <= lo ? 0 : 1)] = v;
+      }
+      pos = end;
+    }
+  }
+}
+
+// one warp per label that crosses a chunk boundary: its pieces in chunk order; empty labels get 0
+__global__ void __launch_bounds__(kBlock) k_seed_label_fix(int64_t chunk, const int32_t* __restrict__ offsets,
+                                                           int n_labels, const double* __restrict__ part,
+                                                           float* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t l = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; l < n_labels; l += warps) {
+    const int64_t b = offsets[l], e = offsets[l + 1];
+    if (b == e) {
+      if (lane == 0) out[l] = 0.0f;
+      continue;
+    }
+    const int64_t c0 = b / chunk, c1 = (e - 1) / chunk;
+    if (c0 == c1) continue;   // finished by k_seed_label_grad
+    double v = 0.0;
+    for (int64_t c = c0 + lane; c <= c1; c += 32) v += part[2 * c + ((c == c0 && b != c0 * chunk) ? 1 : 0)];
+    v = warp_sum(v);
+    if (lane == 0) out[l] = (float)v;
+  }
 }
 
 // results by label: the step's integer accumulator -> fp32 table, and back to zero for the next step (sample blockIdx.z)
@@ -1538,7 +1632,10 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
   if (p->mode == GJ_MODE_SEED) {
     pp.phases &= ~GJ_PHASE_NETWORKS;
     if (!io->seed_fraction) return bad("seed_fraction is NULL");
+    if (io->seed_label && (io->n_seed_labels < 1 || io->n_seed_labels > (1 << 30)))
+      return bad("n_seed_labels must lie in [1, 2^30]");
   }
+  const bool seed_by = p->mode == GJ_MODE_SEED && io->seed_label != nullptr;
   if (p->mode == GJ_MODE_SEED && pp.phases == (GJ_PHASE_SAMPLE | GJ_PHASE_INFECT | GJ_PHASE_SYMPTOMS) &&
       !p->exact_order && !io->inj_E && !io->inj_u && !io->inj_z && io->s && io->inf && io->tinf && io->cur && io->nxt &&
       io->ttn && io->tape_y0 && io->stage_prob && io->s_o && io->inf_o && io->tinf_o && io->cur_o && io->nxt_o &&
@@ -1549,15 +1646,24 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
     int64_t g = (N + (int64_t)kLeanThreads * kLeanBatch - 1) / ((int64_t)kLeanThreads * kLeanBatch);
     gj_world_desc wt = *w;
     wt.n_tiles = g;   // lean_grid clips the persistent grid to the work available
-#define GJ_SEED(D, L, I) \
-  launch_pdl(k_lean_seed<D, L>, dim3(lean_grid(&wt, k_lean_seed<D, L>, &occ[I])), dim3(kLeanThreads), 0, st, *w, pp, *io, \
-             sc.red_part, sc.tickets)
-    if (io->label) {
-      if (diag) GJ_SEED(true, true, 3);
-      else GJ_SEED(false, true, 2);
+#define GJ_SEED(K, C, D, L, I) \
+  launch_pdl(K<D, L>, dim3(lean_grid(&wt, K<D, L>, &C[I])), dim3(kLeanThreads), 0, st, *w, pp, *io, sc.red_part, \
+             sc.tickets)
+    if (io->seed_label) {   // seeding by label
+      static OccCache occ_by[4];
+      if (io->label) {
+        if (diag) GJ_SEED(k_lean_seed_by, occ_by, true, true, 3);
+        else GJ_SEED(k_lean_seed_by, occ_by, false, true, 2);
+      } else {
+        if (diag) GJ_SEED(k_lean_seed_by, occ_by, true, false, 1);
+        else GJ_SEED(k_lean_seed_by, occ_by, false, false, 0);
+      }
+    } else if (io->label) {
+      if (diag) GJ_SEED(k_lean_seed, occ, true, true, 3);
+      else GJ_SEED(k_lean_seed, occ, false, true, 2);
     } else {
-      if (diag) GJ_SEED(true, false, 1);
-      else GJ_SEED(false, false, 0);
+      if (diag) GJ_SEED(k_lean_seed, occ, true, false, 1);
+      else GJ_SEED(k_lean_seed, occ, false, false, 0);
     }
 #undef GJ_SEED
     GJ_CHECK_LAUNCH("k_lean_seed");
@@ -1565,8 +1671,14 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
   }
   if (!(pp.phases & GJ_PHASE_NETWORKS)) {  // stand-alone sampler / infect / symptoms, seeding
     ProfScope ps(K_AGENT_FWD, st);
-    if (io->label) k_agent_forward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
-    else k_agent_forward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    if (seed_by) {
+      if (io->label) k_agent_seed_forward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+      else k_agent_seed_forward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    } else if (io->label) {
+      k_agent_forward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    } else {
+      k_agent_forward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    }
     GJ_CHECK_LAUNCH("k_agent_forward");
     return 0;
   }
@@ -1665,6 +1777,43 @@ int gj_step_forward_batch(const gj_world_desc* w, const gj_step_params* p, const
   return rc > 0 ? 0 : rc;
 }
 
+// seeding by label, backward: the per-agent pass writes d/dseed_fraction to seed_work, then the per-label reduction.
+// The reduction's chunk partials live in the scratch's reduction partials (free once the agent pass is done); the chunk
+// is the smallest power of two >= kSeedChunk whose partials fit there, so it depends on the world only.
+constexpr int64_t kSeedChunk = 2048;
+static int64_t seed_chunk(const gj_world_desc* w) {
+  const int64_t n_tiles = w->n_tiles > 0 ? w->n_tiles : 1;
+  const int64_t slots = (n_tiles > kRedBlocks ? n_tiles : kRedBlocks) * kMaxRed;   // doubles in Scratch::red_part
+  int64_t chunk = kSeedChunk;
+  while (2 * ((w->n_agents + chunk - 1) / chunk) > slots) chunk *= 2;
+  return chunk;
+}
+static int seed_backward(const gj_world_desc* w, const gj_step_params& pp, const gj_bwd_io* io, const Scratch& sc,
+                         cudaStream_t st) {
+  if (io->n_seed_labels < 1 || io->n_seed_labels > (1 << 30)) return bad("n_seed_labels must lie in [1, 2^30]");
+  if (!io->seed_order || !io->seed_offsets || !io->seed_work) return bad("seed_label given without seed_order / seed_offsets / seed_work");
+  const int64_t N = w->n_agents;
+  {
+    ProfScope ps(K_AGENT_BWD, st);
+    if (io->label && io->g_red_label)
+      k_agent_seed_backward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    else k_agent_seed_backward<false><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);
+    GJ_CHECK_LAUNCH("k_agent_seed_backward");
+  }
+  if (!io->g_seed_fraction) return 0;
+  ProfScope ps(K_SEED_GRAD, st);
+  const int64_t chunk = seed_chunk(w);
+  const int64_t n_chunks = (N + chunk - 1) / chunk;
+  k_seed_label_grad<<<blocks_for(n_chunks * 32, kBlock), kBlock, 0, st>>>(N, chunk, io->seed_order, io->seed_offsets,
+                                                                         io->n_seed_labels, io->seed_work, sc.red_part,
+                                                                         io->g_seed_fraction);
+  GJ_CHECK_LAUNCH("k_seed_label_grad");
+  k_seed_label_fix<<<blocks_for((int64_t)io->n_seed_labels * 32, kBlock), kBlock, 0, st>>>(
+      chunk, io->seed_offsets, io->n_seed_labels, sc.red_part, io->g_seed_fraction);
+  GJ_CHECK_LAUNCH("k_seed_label_fix");
+  return 0;
+}
+
 static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, const gj_bwd_io* io, void* stream,
                               const gj_batch* batch) {
   if (int e = check_world(w)) return e;
@@ -1684,6 +1833,7 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if (p->mode == GJ_MODE_SEED) pp.phases &= ~GJ_PHASE_NETWORKS;
   if ((pp.phases & GJ_PHASE_SAMPLE) && !io->tape_y0) return bad("tape_y0 is NULL");
   if (!(pp.phases & GJ_PHASE_NETWORKS)) {
+    if (p->mode == GJ_MODE_SEED && io->seed_label) return seed_backward(w, pp, io, sc, st);
     ProfScope ps(K_AGENT_BWD, st);
     if (io->label && io->g_red_label)
       k_agent_backward<true><<<agent_grid(N), kBlock, 0, st>>>(*w, pp, *io, sc.red_part, sc.tickets);

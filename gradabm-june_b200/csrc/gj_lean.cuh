@@ -922,11 +922,12 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
 // seeding step in throughput mode (GJ_MODE_SEED with in-kernel noise): sample with q = 1 - fraction, infect (clamp
 // variant: same values), first symptoms update, reductions — the arithmetic of lean_forward_core without networks.
 // Replaces the generic k_agent_forward (IEEE libm, 1.45 ms per window at 56 M agents) for Runner.set_initial_cases.
+// kSeed: seeding by label, q = 1 - seed_fraction[seed_label[a]]; the code and the region's fraction are loaded with the
+// other per-agent operands of the batch, outside the draw loop.
 // =====================================================================================================
-template <bool kDiag, bool kLabel>
-__global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, gj_step_params p, gj_fwd_io io,
-                                                              double* __restrict__ red_part,
-                                                              unsigned int* __restrict__ ticket) {
+template <bool kDiag, bool kLabel, bool kSeed>
+__device__ __forceinline__ void lean_seed_body(const gj_world_desc& w, const gj_step_params& p, const gj_fwd_io& io,
+                                               double* __restrict__ red_part, unsigned int* __restrict__ ticket) {
   __shared__ float hist[100];
   __shared__ float deaths;
   pdl_launch();
@@ -945,6 +946,8 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
     float s[kLeanBatch], inf[kLeanBatch], tinf[kLeanBatch], cur[kLeanBatch], nxt[kLeanBatch], ttn[kLeanBatch];
     uint32_t oid[kLeanBatch];
     int cls[kLeanBatch];
+    int32_t lab[kLeanBatch];
+    float qs[kLeanBatch];
 #pragma unroll
     for (int h = 0; h < kLeanBatch; ++h) {
       const uint32_t a = base + h * kLeanThreads;
@@ -957,6 +960,11 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
       ttn[h] = io.ttn[al];
       cls[h] = w.cls ? w.cls[al] : 0;
       oid[h] = w.orig_id ? w.orig_id[al] : 0u;
+      if (kSeed) lab[h] = io.seed_label[al];
+    }
+    if (kSeed) {
+#pragma unroll
+      for (int h = 0; h < kLeanBatch; ++h) qs[h] = 1.0f - io.seed_fraction[lab[h]] * 1.0f;
     }
 #pragma unroll
     for (int h = 0; h < kLeanBatch; ++h) {
@@ -967,7 +975,7 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
       philox_step_pair(p.seed, p.call_index, ga, r);
       const FwdRes o = lean_forward_core<false>(p, lp, io.stage_prob, ga, lean_noise_dE(r[0], r[1]), 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, s[h],
                                                 inf[h], tinf[h], cur[h], nxt[h], ttn[h], cls[h], inv_tau, dead, hist,
-                                                &deaths, q_seed);
+                                                &deaths, kSeed ? qs[h] : q_seed);
       io.tape_y0[a] = o.tape_y0;
       if (kDiag && io.n) io.n[a] = o.n;
       io.s_o[a] = o.s_o;
@@ -996,6 +1004,21 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, 
     }
     finish_partials<kMaxRed>(nr, red_part, gridDim.x, ticket, io.red);
   }
+}
+
+template <bool kDiag, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed(gj_world_desc w, gj_step_params p, gj_fwd_io io,
+                                                              double* __restrict__ red_part,
+                                                              unsigned int* __restrict__ ticket) {
+  lean_seed_body<kDiag, kLabel, false>(w, p, io, red_part, ticket);
+}
+
+// the same with seeding by label (gj_fwd_io.seed_label)
+template <bool kDiag, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed_by(gj_world_desc w, gj_step_params p, gj_fwd_io io,
+                                                                 double* __restrict__ red_part,
+                                                                 unsigned int* __restrict__ ticket) {
+  lean_seed_body<kDiag, kLabel, true>(w, p, io, red_part, ticket);
 }
 
 // per-agent arithmetic of the backward pass (shared with gj_pipe.cuh): symptoms^T, infect^T, sampler^T, clamp/exp

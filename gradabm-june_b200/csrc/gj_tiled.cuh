@@ -268,12 +268,13 @@ struct AgentState {
 };
 
 // kLabel: also add the agent's cases and death indicator to its label's column of the integer accumulator lacc
-template <bool kLabel = false>
+// kSeed: seeding by label, the agent's fraction is seed_fraction[seed_label[a]]
+template <bool kLabel = false, bool kSeed = false>
 __device__ __forceinline__ void forward_tail(const gj_step_params& p, const gj_fwd_io& io, int64_t N, int64_t a,
                                              int64_t ga, int age, float q, AgentState st, float* red,
                                              uint32_t* lacc = nullptr) {
   const int dead = p.n_stages - 1;
-  if (p.mode == GJ_MODE_SEED) q = 1.0f - io.seed_fraction[0] * 1.0f;  // infection.py:36-40
+  if (p.mode == GJ_MODE_SEED) q = 1.0f - io.seed_fraction[kSeed ? io.seed_label[a] : 0] * 1.0f;  // infection.py:36-40
   float n = 0.0f;
   StepNoise nz;
   nz.E0 = nz.E1 = 1.0f;
@@ -487,7 +488,8 @@ struct BackAgent {
 
 // symptoms^T, infect^T, sampler^T and the clamp/exp chain: shared by the generic and the tiled kernels
 // kLabel: fold in the cotangent of the forward's label table (gj_bwd_io.g_red_label) at the agent's label
-template <bool kLabel = false>
+// kSeed: seeding by label, the agent's fraction is seed_fraction[seed_label[a]]
+template <bool kLabel = false, bool kSeed = false>
 __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, const gj_bwd_io& io, int64_t N, int64_t a,
                                                     int64_t ga, int age, const AgentState& st, bool with_networks) {
   const int dead = p.n_stages - 1;
@@ -575,7 +577,7 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
     lam = (st.s == 0.0f) ? 0.0f : v;
     q = not_infected_prob(lam, p.dt);
   }
-  if (seed_mode) q = 1.0f - io.seed_fraction[0] * 1.0f;
+  if (seed_mode) q = 1.0f - io.seed_fraction[kSeed ? io.seed_label[a] : 0] * 1.0f;
   if (p.phases & GJ_PHASE_SAMPLE) {
     if (!with_networks && !seed_mode && io.q_in) q = io.q_in[a];  // stand-alone sampler
     float y0, y1;

@@ -18,7 +18,7 @@ GJ_MAX_STAGES = 16
 GJ_MAX_QUAR = 4
 GJ_MAX_AGE_BINS = 8
 GJ_MAX_CHANNELS = 8
-GJ_ABI_VERSION = 11
+GJ_ABI_VERSION = 12
 
 KIND_PLAIN, KIND_HOUSEHOLD, KIND_LEISURE, KIND_CARE_VISIT = 0, 1, 2, 3
 PHASE_NETWORKS, PHASE_SAMPLE, PHASE_INFECT, PHASE_SYMPTOMS, PHASE_ALL = 1, 2, 4, 8, 15
@@ -106,11 +106,15 @@ class FwdIO(C.Structure):
     # results by label: codes, column count, fp32 table and its integer accumulator
     _fields_ = [(name, C.c_void_p) for name in _FWD_FIELDS] + [
         ("label", C.c_void_p), ("n_labels", C.c_int32), ("_pad_label", C.c_int32), ("red_label", C.c_void_p),
-        ("label_acc", C.c_void_p)]
+        ("label_acc", C.c_void_p),
+        # seeding by label: region codes and their count
+        ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32)]
 
 
 class BwdIO(C.Structure):
-    _fields_ = [(name, C.c_void_p) for name in _BWD_FIELDS] + [("label", C.c_void_p), ("g_red_label", C.c_void_p)]
+    _fields_ = [(name, C.c_void_p) for name in _BWD_FIELDS] + [("label", C.c_void_p), ("g_red_label", C.c_void_p)] + [
+        ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32), ("seed_order", C.c_void_p),
+        ("seed_offsets", C.c_void_p), ("seed_work", C.c_void_p)]
 
 
 class Batch(C.Structure):

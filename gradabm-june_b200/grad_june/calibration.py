@@ -89,14 +89,18 @@ class Calibrator:
 
         cal = Calibrator(runner, loss_fn=lambda r: ((r["cases_per_timestep"] - target) ** 2).mean())
         history = cal.fit(50)              # pandas DataFrame: iteration, loss, log_beta_<network>..., grad_<network>...
+                                           # (fit_seed=True: also log_fraction_<label>..., grad_log_fraction_<label>...)
         cal.save(history)                  # <save_path>/calibration.csv + the reference's results.csv of the last run
     """
 
     def __init__(self, runner, loss_fn: Callable[[dict], torch.Tensor], networks: Optional[Sequence[str]] = None,
-                 lr: float = 0.05, optimizer: str = "adam", seed: int = 0, reseed_every: int = 0):
+                 lr: float = 0.05, optimizer: str = "adam", seed: int = 0, reseed_every: int = 0, fit_seed: bool = False):
+        """``fit_seed=True`` also calibrates the initial-case log-fractions (one national value, or one per region of
+        ``runner.seed_labels``): they sit after the log-betas in the parameter vector."""
         self.runner = runner
-        self.graphed = GraphedRunner(runner, loss_fn, networks=networks, seed=seed)
+        self.graphed = GraphedRunner(runner, loss_fn, networks=networks, seed=seed, fit_seed=fit_seed)
         self.names = self.graphed.names
+        self.seed_names = self.graphed.seed_names
         dev = self.graphed.device
         self.log_beta = self.graphed.log_beta.detach().clone().requires_grad_(True)
         opt = {"adam": torch.optim.Adam, "sgd": torch.optim.SGD}[optimizer.lower()]
@@ -123,8 +127,11 @@ class Calibrator:
         for _ in range(n_iterations):
             loss, lb, grads = self.step()
             row = {"iteration": self.iteration, "loss": loss}
+            K = len(self.names)
             row.update({f"log_beta_{k}": v for k, v in zip(self.names, lb)})
             row.update({f"grad_{k}": v for k, v in zip(self.names, grads)})
+            row.update({f"log_fraction_{k}": v for k, v in zip(self.seed_names, lb[K:])})
+            row.update({f"grad_log_fraction_{k}": v for k, v in zip(self.seed_names, grads[K:])})
             rows.append(row)
             if callback is not None:
                 callback(row)

@@ -9,6 +9,10 @@ the NCCL all-reduces of a partitioned world — is capturable with ``torch.cuda.
     graphed = GraphedRunner(runner, loss_fn=lambda r: r["cases_per_timestep"].sum())
     loss, grads, results = graphed(log_beta_vector)       # replay: one graph launch
 
+``fit_seed=True`` calibrates the seeding too: the initial-case log-fractions go next to the log-betas in the parameter
+vector — one value for a national seed, one per region of ``runner.seed_labels`` with ``seed_by`` — so a replay takes
+[K + R] values ([b, K + R] batched) and returns their gradient.
+
 Noise: the Philox key and call indices are kernel arguments, so every replay draws the SAME noise (common random
 numbers across parameter samples — the usual variance reduction for calibration gradients); ``recapture(seed)``
 re-records the graph with another key.
@@ -23,6 +27,7 @@ replay is bit-identical to an unbatched replay with ``log_beta[r]`` (same Philox
 import warnings
 from typing import Callable, Optional, Sequence
 
+import numpy as np
 import torch
 
 from . import ops
@@ -30,8 +35,9 @@ from . import ops
 
 class GraphedRunner:
     def __init__(self, runner, loss_fn: Callable[[dict], torch.Tensor], networks: Optional[Sequence[str]] = None,
-                 seed: int = 0, warmup: int = 1, batch: Optional[int] = None):
+                 seed: int = 0, warmup: int = 1, batch: Optional[int] = None, fit_seed: bool = False):
         self.runner = runner
+        self.fit_seed = bool(fit_seed)
         self.loss_fn = loss_fn
         self.batch = int(batch) if batch else None
         runner.batch = self.batch
@@ -41,6 +47,18 @@ class GraphedRunner:
         ops.require_cuda(agent.susceptibility, "data['agent'].susceptibility")
         self.device = agent.susceptibility.device
         init = [float(torch.as_tensor(nets[k].log_beta).detach().reshape(-1)[0]) for k in self.names]
+        self.n_beta = len(init)
+        self.seed_names = []
+        if self.fit_seed:   # the log-fractions follow the log-betas: one per region, or one national value
+            lf = runner.log_fraction_initial_cases
+            lf = lf.detach().cpu().numpy() if torch.is_tensor(lf) else np.asarray(lf, dtype=np.float64)
+            if runner.seed_by is None:
+                self.seed_names = ["national"]
+                init += [float(lf.reshape(-1)[0])]
+            else:
+                R = len(runner.seed_labels)
+                self.seed_names = [str(v) for v in runner.seed_labels]
+                init += [float(v) for v in np.broadcast_to(lf.reshape(-1)[:R] if lf.size >= R else lf, (R,))]
         self.log_beta = torch.tensor(init, dtype=torch.float32).to(self.device)
         if self.batch:
             self.log_beta = self.log_beta.repeat(self.batch, 1)          # [b, K]
@@ -63,6 +81,13 @@ class GraphedRunner:
             # refuses to assign a plain tensor over one: unregister it first
             nets[k]._parameters.pop("log_beta", None)
             nets[k].log_beta = self.log_beta[:, i] if self.batch else self.log_beta[i]
+        if self.fit_seed:
+            K = self.n_beta
+            self.runner._parameters.pop("log_fraction_initial_cases", None)   # an nn.Parameter is replaced like log_beta
+            if self.runner.seed_by is None:
+                self.runner.log_fraction_initial_cases = self.log_beta[:, K] if self.batch else self.log_beta[K]
+            else:
+                self.runner.log_fraction_initial_cases = self.log_beta[:, K:] if self.batch else self.log_beta[K:]
         with ops.philox_seed(self.seed):
             results, is_infected = self.runner()
         loss = self.loss_fn(results)
@@ -73,7 +98,8 @@ class GraphedRunner:
         part = self.runner.data.__dict__.get("_gj_partition")
         if part is not None and part.world_size > 1:
             # geographic partition: every rank holds the d/dbeta terms of the groups it owns; the sum over ranks
-            # is part of the captured iteration (one more NCCL kernel in the graph, no eager collective per replay)
+            # is part of the captured iteration (one more NCCL kernel in the graph, no eager collective per replay);
+            # with fit_seed the seeding gradients (each rank's own agents) are summed in the same all-reduce
             import torch.distributed as dist
             dist.all_reduce(self.log_beta.grad, group=part.process_group)
         return loss.detach(), results, is_infected
@@ -107,8 +133,9 @@ class GraphedRunner:
 
     @torch.no_grad()
     def __call__(self, log_beta: Optional[torch.Tensor] = None):
-        """Replay with ``log_beta`` ([K], or [b, K] for a batched window; any device; None = keep).  Returns
-        (loss, d loss / d log_beta, results): static device tensors that the next replay overwrites."""
+        """Replay with ``log_beta`` ([K], or [b, K] for a batched window; [K + R] / [b, K + R] with ``fit_seed``, the
+        log-fractions last; any device; None = keep).  Returns (loss, d loss / d log_beta, results): static device
+        tensors that the next replay overwrites."""
         if log_beta is not None:
             self.log_beta.copy_(log_beta.to(dtype=torch.float32), non_blocking=True)
         self.graph.replay()

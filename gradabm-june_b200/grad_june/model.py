@@ -91,12 +91,14 @@ class GradJune(torch.nn.Module):
         return spec, nets
 
     def step(self, data, timer, age_bins=None, mode=ops.MODE_STEP, seed_fraction=None, noise=None, want_probs=True,
-             next_timer=None, label=None):
+             next_timer=None, label=None, seed_label=None):
         """Fused step; returns (data, reductions) where reductions = [cases, deaths, cases by age bin...]
         (None unless ``age_bins`` is given).  With ``label`` (:class:`grad_june.ops.Labels`) it returns
         (data, reductions, label_table): the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched),
         reduced inside the step kernels.  ``want_probs=False`` skips the two diagnostic per-agent outputs
         (``not_infected_probs``, ``new_infected``) that the reference keeps only as locals of its forward.
+        ``seed_label`` (:class:`grad_june.ops.SeedLabels`, seeding step only): ``seed_fraction`` holds one fraction per
+        region and every agent is seeded with its region's.
         ``next_timer``: the timer as it will be at the FOLLOWING call (the driver knows the schedule): the
         kernels then run that step's transmission pass inside this one (used only if the next call matches)."""
         agent = data["agent"]
@@ -116,7 +118,7 @@ class GradJune(torch.nn.Module):
                  "cur": sym["current_stage"], "nxt": sym["next_stage"], "ttn": sym["time_to_next_stage"]}
         beta = beta_vector(nets, policies, timer, dev) if nets else None
         out = ops.infection_step(static, spec, beta, state, seed_fraction=seed_fraction, noise=noise,
-                                 next_spec=next_spec, label=label)
+                                 next_spec=next_spec, label=label, seed_label=seed_label)
         if out["T"] is not None:
             agent.transmission = out["T"]
         agent.susceptibility = out["s"]

@@ -196,6 +196,44 @@ def make_labels(codes, n: int, device=None) -> Labels:
     return Labels(codes.to(device=device or codes.device, dtype=torch.int32).contiguous(), n)
 
 
+@dataclass(frozen=True)
+class SeedLabels:
+    """Per-agent region codes of seeding by label: ``codes[a]`` in ``[0, n)`` picks agent a's initial-case fraction.
+    ``order`` lists the agents stably sorted by code and ``offsets[l]`` is where region l starts in it ([n + 1]):
+    the backward's deterministic per-region reduction walks them.  Build it with :func:`make_seed_labels`."""
+    codes: torch.Tensor     # [N] int32
+    n: int
+    order: torch.Tensor     # [N] int32
+    offsets: torch.Tensor   # [n + 1] int32
+
+
+def make_seed_labels(codes, n: int, device=None) -> SeedLabels:
+    """Validated :class:`SeedLabels` (range-checked like :func:`make_labels`); ``codes`` may be the codes of a
+    :class:`Labels` already on the device, which are then shared."""
+    lab = make_labels(codes, n, device)
+    if lab.codes.numel() >= 1 << 31:
+        raise ValueError("seeding by label supports fewer than 2^31 agents per world")
+    order = torch.sort(lab.codes, stable=True).indices.to(torch.int32)
+    counts = torch.bincount(lab.codes.long(), minlength=lab.n)
+    offsets = torch.zeros(lab.n + 1, dtype=torch.int64, device=lab.codes.device)
+    offsets[1:] = torch.cumsum(counts, 0)
+    return SeedLabels(lab.codes, lab.n, order.contiguous(), offsets.to(torch.int32).contiguous())
+
+
+def _set_seed_labels(io, world: DeviceWorld, seed_label: SeedLabels, seed_fraction, nb: int = 1):
+    """Point the io struct at the region codes; checks the fraction tensor holds ``n`` values per sample (or ``n``
+    shared by the samples)."""
+    if seed_label.codes.numel() != world.n_agents or seed_label.codes.device != world.device:
+        raise ValueError(f"seed label codes must hold one entry per agent ({world.n_agents}) on {world.device}")
+    if seed_fraction.numel() not in (seed_label.n, nb * seed_label.n):
+        raise ValueError(f"seed_fraction must hold {seed_label.n} values (one per region)"
+                         + (f" or {nb} x {seed_label.n}" if nb > 1 else "") + f", got {seed_fraction.numel()}")
+    io.seed_label, io.n_seed_labels = seed_label.codes.data_ptr(), seed_label.n
+    if hasattr(io, "seed_order"):
+        io.seed_order, io.seed_offsets = seed_label.order.data_ptr(), seed_label.offsets.data_ptr()
+        io.seed_work = _buffer(world, "seed_work", world.n_agents).data_ptr()
+
+
 def _label_acc(world: DeviceWorld, n: int):
     """The integer accumulator of the label table ([n] uint32, zero; every call leaves it zero)."""
     t = world.__dict__.get("_label_acc")
@@ -448,7 +486,7 @@ class _Step(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in,
-                seed_fraction, next_spec=None, label: Optional[Labels] = None):
+                seed_fraction, next_spec=None, label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None):
         world = static.world
         dev = world.device
         N = world.n_agents
@@ -475,6 +513,9 @@ class _Step(torch.autograd.Function):
         if static.symptoms is not None:
             put("stage_prob", static.symptoms.stage_prob)
         seed_fraction = put("seed_fraction", seed_fraction) if seed_mode else None
+        seed_label = seed_label if seed_mode else None
+        if seed_label is not None:
+            _set_seed_labels(io, world, seed_label, seed_fraction)
         put("inj_E", E), put("inj_u", u), put("inj_z", z)
         st = {}
         for name, t in zip(_STATE, (s, inf, tinf, cur, nxt, ttn)):
@@ -565,6 +606,7 @@ class _Step(torch.autograd.Function):
                 cur=out.get("cur_o"))
 
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
+        ctx.seed_label = seed_label
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"],
                               T_in if T_in is not None else T, q_in, n_in,
@@ -651,7 +693,12 @@ class _Step(torch.autograd.Function):
         g_q_in = new("g_q_out") if (q_in is not None and need[11]) else None
         g_n_in = new("g_n_out") if (n_in is not None and need[12]) else None
         g_beta = new("g_beta", max(p.n_nets, 1), zero=True) if nets_on else None
-        g_frac = new("g_seed_fraction", 1, zero=True) if seed_mode else None
+        g_frac = None
+        if seed_mode and ctx.seed_label is not None:   # one gradient per region
+            _set_seed_labels(io, world, ctx.seed_label, seed_fraction)
+            g_frac = new("g_seed_fraction", ctx.seed_label.n).reshape(seed_fraction.shape)
+        elif seed_mode:
+            g_frac = new("g_seed_fraction", 1, zero=True)
         R_buf = cR_buf = None
         if nets_on:
             s_total += world.n_groups
@@ -673,7 +720,7 @@ class _Step(torch.autograd.Function):
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None)
+                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None, None)
 
 
 # --------------------------------------------------------------------------------------
@@ -720,7 +767,7 @@ class _BatchStep(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction,
-                label: Optional[Labels] = None):
+                label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None):
         world = static.world
         dev, N = world.device, world.n_agents
         L = _lib.lib()
@@ -778,11 +825,17 @@ class _BatchStep(torch.autograd.Function):
         strides.update(red=4 * nr, scratch=scr_stride, red_label=4 * n_lab, label_acc=4 * n_lab)
         T = tape_v = S_un = None
         sG = K = 0
+        if not seed_mode:
+            seed_label = None
         if seed_mode:
             seed_fraction = put("seed_fraction", seed_fraction)
-            if seed_fraction.numel() not in (1, nb):
+            R = 1
+            if seed_label is not None:   # seeding by label: [R] shared by the samples or [b, R]
+                _set_seed_labels(io, world, seed_label, seed_fraction, nb)
+                R = seed_label.n
+            elif seed_fraction.numel() not in (1, nb):
                 raise ValueError("seed_fraction must hold 1 or b values")
-            strides["seed_fraction"] = 4 if seed_fraction.numel() == nb else 0
+            strides["seed_fraction"] = 4 * R if seed_fraction.numel() == nb * R else 0
             beta = None
             _row_calls(L.gj_step_forward, "gj_step_forward", world, desc, p, io, nb, strides, _stream(dev))
         else:
@@ -808,6 +861,7 @@ class _BatchStep(torch.autograd.Function):
                 _lib.check(L.gj_step_forward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_forward_batch")
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
+        ctx.seed_label = seed_label
         ctx.shape = (nb, Np, sG, K, nr)
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"], T, seed_fraction,
@@ -870,14 +924,18 @@ class _BatchStep(torch.autograd.Function):
         desc = world.desc()
         g_beta = g_frac = None
         if seed_mode:
-            g_frac = torch.zeros(nb, dtype=torch.float32, device=dev)
+            R = 1
+            if ctx.seed_label is not None:
+                _set_seed_labels(io, world, ctx.seed_label, seed_fraction, nb)
+                R = ctx.seed_label.n
+            g_frac = torch.zeros(nb, R, dtype=torch.float32, device=dev)
             io.g_seed_fraction = g_frac.data_ptr()
             strides = {name: 4 * Np for name in _AGENT_FIELDS}
-            strides.update(g_red=4 * nr, scratch=scr_stride, g_seed_fraction=4, g_red_label=4 * n_lab,
-                           seed_fraction=4 if seed_fraction.numel() == nb else 0)
+            strides.update(g_red=4 * nr, scratch=scr_stride, g_seed_fraction=4 * R, g_red_label=4 * n_lab,
+                           seed_fraction=4 * R if seed_fraction.numel() == nb * R else 0)
             _row_calls(L.gj_step_backward, "gj_step_backward", world, desc, p, io, nb, strides, _stream(dev))
-            if seed_fraction.numel() != nb:
-                g_frac = g_frac.sum().reshape(seed_fraction.shape)    # one fraction shared by the samples
+            if seed_fraction.numel() != nb * R:
+                g_frac = g_frac.sum(0).reshape(seed_fraction.shape)    # one fraction (per region) shared by the samples
             else:
                 g_frac = g_frac.reshape(seed_fraction.shape)
         else:
@@ -899,14 +957,17 @@ class _BatchStep(torch.autograd.Function):
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_frac if (seed_mode and need[10]) else None, None)
+                g_frac if (seed_mode and need[10]) else None, None, None)
 
 
 def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=None, q_in=None, n_in=None,
-                   seed_fraction=None, noise=None, next_spec=None, label: Optional[Labels] = None):
+                   seed_fraction=None, noise=None, next_spec=None, label: Optional[Labels] = None,
+                   seed_label: Optional[SeedLabels] = None):
     """Run one (fused or partial) step.  ``state``: s, inf, tinf, cur, nxt, ttn (any may be None when
     the phases do not need it).  Returns a dict with s, inf, tinf, cur, nxt, ttn, T, q, n, red and red_label:
-    with ``label`` the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched), else None."""
+    with ``label`` the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched), else None.
+    ``seed_label`` (seeding step only): ``seed_fraction`` then holds one fraction per region ([n], or [b, n]
+    batched) and agent a is seeded with ``seed_fraction[seed_label.codes[a]]``."""
     world = static.world
     if world.device.type != "cuda":
         raise _lib.GradJuneLibraryError(
@@ -921,13 +982,13 @@ def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=N
         if T_in is not None or q_in is not None or n_in is not None or static.exchange is not None:
             raise _lib.GradJuneLibraryError("batched ensembles run the whole fused step on an unpartitioned world")
         outs = _BatchStep.apply(static, spec, noise, beta, state["s"], state["inf"], state["tinf"], state["cur"],
-                                state["nxt"], state["ttn"], seed_fraction, label)
+                                state["nxt"], state["ttn"], seed_fraction, label, seed_label)
         names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "red", "red_label")
         ret = dict(zip(names, outs))
         ret.update(q=None, n=None, lam=None)
         return ret
     outs = _Step.apply(static, spec, noise, beta, state.get("s"), state.get("inf"), state.get("tinf"),
                        state.get("cur"), state.get("nxt"), state.get("ttn"), T_in, q_in, n_in, seed_fraction, next_spec,
-                       label)
+                       label, seed_label)
     names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "q", "n", "red", "lam", "red_label")
     return dict(zip(names, outs))

@@ -46,9 +46,43 @@ def label_codes(labels, columns):
     return codes
 
 
+def seed_log_fractions(mapping, labels):
+    """A per-region log-fraction mapping ``{label: value, ..., "default": value}`` (the YAML form) as a list in the
+    order of the sorted ``labels``.  Labels the mapping does not list take ``default``; a label in the mapping that no
+    agent carries raises, and so does a missing ``default`` when some label is not listed."""
+    mapping = dict(mapping)
+    default = mapping.pop("default", None)
+    labels = np.asarray(labels)
+    out = [None] * len(labels)
+    for key, value in mapping.items():
+        if labels.dtype.kind in "iu" and not isinstance(key, (int, np.integer)):
+            try:
+                key = int(key)
+            except (TypeError, ValueError):
+                raise ValueError(f"seeding: label {key!r} is not carried by any agent") from None
+        elif labels.dtype.kind in "US" and not isinstance(key, str):
+            key = str(key)
+        i = int(np.searchsorted(labels, key))
+        if i >= len(labels) or labels[i] != key:
+            raise ValueError(f"seeding: label {key!r} is not carried by any agent")
+        out[i] = float(value)
+    missing = [labels[i] for i, v in enumerate(out) if v is None]
+    if missing and default is None:
+        raise ValueError(f"seeding: no log-fraction for label {missing[0]!r} and no 'default'")
+    return [float(default) if v is None else v for v in out]
+
+
 class Runner(torch.nn.Module):
     def __init__(self, model, data, timer, log_fraction_initial_cases, save_path, parameters,
-                 age_bins=(0, 18, 65, 100), results_by=None):
+                 age_bins=(0, 18, 65, 100), results_by=None, seed_by=None):
+        """``seed_by`` (``infection_seed: {by: super_area}`` in the YAML): seed the initial cases per value of
+        ``data["agent"][seed_by]`` (``runner.seed_labels``, the sorted distinct values over every rank of a partitioned
+        world).  ``log_fraction_initial_cases`` is then a scalar (every region), a list or tensor of one value per
+        region in ``seed_labels`` order ([b, R] or [R] when ``runner.batch = b``; may be an ``nn.Parameter``: the
+        gradient reaches every region), or a mapping ``{label: value, "default": value}``.  A region's fraction below
+        about 2^-24 (log-fraction < -7.2) rounds its q = 1 - fraction to exactly 1 in fp32: none of its agents is
+        infected, and its gradient is NaN (the sampler's d/dq divides 0 by 0, as the reference's torch code does);
+        the other regions' gradients are unaffected."""
         super().__init__()
         self.model = model
         self.data = data
@@ -71,6 +105,21 @@ class Runner(torch.nn.Module):
         if results_by is not None:
             labels = agent_labels(data["agent"][results_by], self.n_agents)
             self.result_labels = label_union(np.unique(labels), data.__dict__.get("_gj_partition"))
+        # seeding by label: one initial-case fraction per value of data["agent"][seed_by]
+        self.seed_by = seed_by
+        self.seed_labels = None
+        if seed_by is not None:
+            if seed_by == results_by:
+                self.seed_labels = self.result_labels
+            else:
+                labels = agent_labels(data["agent"][seed_by], self.n_agents)
+                self.seed_labels = label_union(np.unique(labels), data.__dict__.get("_gj_partition"))
+            if isinstance(log_fraction_initial_cases, dict):
+                log_fraction_initial_cases = seed_log_fractions(log_fraction_initial_cases, self.seed_labels)
+            self.log_fraction_initial_cases = log_fraction_initial_cases
+            self._seed_fraction_shape(log_fraction_initial_cases)
+        elif isinstance(log_fraction_initial_cases, dict):
+            raise ValueError("a per-region log_fraction_initial_cases mapping needs infection_seed.by (seed_by)")
         # batched ensemble (SURVEY 8e-2): ``runner.batch = b`` makes ``forward()`` step b independent samples of the
         # epidemic at once — the networks' ``log_beta`` then hold b values each, the state tensors are [b, Np] and
         # every result series is [T+1, b].  All samples draw the same noise (common random numbers).
@@ -93,6 +142,7 @@ class Runner(torch.nn.Module):
             parameters=params,
             age_bins=params.get("age_bins_to_save", (0, 18, 65, 100)),
             results_by=params.get("results_by"),
+            seed_by=params["infection_seed"].get("by"),
         )
 
     @staticmethod
@@ -172,7 +222,19 @@ class Runner(torch.nn.Module):
         agent.symptoms = dict(hit[2])
         self.data["results"] = {"deaths_per_timestep": None}
 
+    def _seed_fraction_shape(self, value):
+        """Check a per-region log-fraction's shape; returns the number of values it holds per sample."""
+        R = len(self.seed_labels)
+        shape = tuple(value.shape) if torch.is_tensor(value) else np.shape(value)
+        batch = self.__dict__.get("batch")
+        if shape in ((), (1,), (R,)) or (batch and shape == (batch, R)):
+            return R
+        raise ValueError(f"seeding by {self.seed_by!r}: log_fraction_initial_cases must be a scalar or hold one value "
+                         f"per region ({R}, or [b, {R}] batched), got shape {shape}")
+
     def _fraction_tensor(self):
+        if self.seed_by is not None:
+            return self._seed_fraction_tensor()
         fraction = 10.0 ** self.log_fraction_initial_cases
         dev = self.data["agent"].susceptibility.device
         if not torch.is_tensor(fraction):
@@ -181,7 +243,41 @@ class Runner(torch.nn.Module):
             if getattr(self, "_fraction_cache", (None, None))[0] != key:
                 self._fraction_cache = (key, torch.tensor([float(fraction)], dtype=torch.float32).to(dev))
             return self._fraction_cache[1]
-        return fraction.reshape(1).to(device=dev, dtype=torch.float32)
+        return fraction.reshape(-1).to(device=dev, dtype=torch.float32)   # [1], or [b] per sample
+
+    def _seed_fraction_tensor(self):
+        """The per-region fractions 10^log_fraction on the device: [R] ([b, R] for a per-sample batch)."""
+        lf = self.log_fraction_initial_cases
+        R = len(self.seed_labels)
+        self._seed_fraction_shape(lf)
+        dev = self.data["agent"].susceptibility.device
+        if not torch.is_tensor(lf):
+            # plain numbers: evaluated like the national scalar (host fp64, then fp32), the device copy kept
+            vals = np.broadcast_to(np.asarray(lf, dtype=np.float64), (R,) if np.ndim(lf) < 2 else np.shape(lf))
+            key = (tuple(float(10.0 ** v) for v in vals.reshape(-1)), vals.shape, str(dev))
+            if getattr(self, "_seed_fraction_cache", (None, None))[0] != key:
+                self._seed_fraction_cache = (key, torch.tensor(key[0], dtype=torch.float32).reshape(vals.shape).to(dev))
+            return self._seed_fraction_cache[1]
+        fraction = (10.0 ** lf).to(device=dev, dtype=torch.float32)
+        if fraction.numel() == 1:
+            fraction = fraction.reshape(1).expand(R)
+        return fraction.contiguous()
+
+    def _seed_label_codes(self):
+        """ops.SeedLabels of ``seed_by`` on the device (built once per label array and device; shares the device codes
+        of ``results_by`` when both name the same attribute), or None."""
+        if self.seed_by is None:
+            return None
+        values = self.data["agent"][self.seed_by]
+        dev = self.data["agent"].susceptibility.device
+        hit = self.__dict__.get("_seed_codes")
+        if hit is None or hit[0] is not values or hit[1] != dev:
+            if self.seed_by == self.results_by:
+                codes = self._labels().codes
+            else:
+                codes = label_codes(agent_labels(values, self.n_agents), self.seed_labels)
+            hit = self.__dict__["_seed_codes"] = (values, dev, ops.make_seed_labels(codes, len(self.seed_labels), dev))
+        return hit[2]
 
     def _labels(self):
         """ops.Labels of ``results_by`` on the device (built once per label array and device, like
@@ -200,7 +296,8 @@ class Runner(torch.nn.Module):
         """infect_fraction_of_people + first symptoms update (runner.py:138-149) as one fused call (with
         ``results_by``: returns (reductions, label table))."""
         out = self.model.step(self.data, self.timer, age_bins=self._age_bins_host, mode=ops.MODE_SEED,
-                              seed_fraction=self._fraction_tensor(), label=self._labels())
+                              seed_fraction=self._fraction_tensor(), label=self._labels(),
+                              seed_label=self._seed_label_codes())
         return out[1] if self.results_by is None else out[1:]
 
     def forward(self):

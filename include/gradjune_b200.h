@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GJ_ABI_VERSION 11
+#define GJ_ABI_VERSION 12
 
 #define GJ_MAX_TYPES 8      /* edge types (household, company, school, university, care_home, leisure, ...) */
 #define GJ_MAX_NETS 16      /* infection networks active in one step */
@@ -255,7 +255,7 @@ typedef struct gj_fwd_io {
   const float* beta;         /* [n_nets] beta_eff per network (base.py:36-42 evaluated on the host) */
   const float* leisure_prob; /* [n_tables][2][2][100] */
   const float* stage_prob;   /* [n_stages][100] */
-  const float* seed_fraction; /* [1] (GJ_MODE_SEED) */
+  const float* seed_fraction; /* [1] (GJ_MODE_SEED), or [n_seed_labels] with seed_label */
   /* injected noise (NULL -> Philox) */
   const float* inj_E; /* [2][N] */
   const float* inj_u; /* [N] */
@@ -303,6 +303,13 @@ typedef struct gj_fwd_io {
   float* red_label;      /* [n_labels][2] cases, deaths */
   uint32_t* label_acc;   /* [n_labels][2] integer workspace, zero-initialised once by the caller; the library leaves it
                             zeroed (gj_scratch_bytes depends on the world only, so it cannot cover it) */
+  /* seeding by label (GJ_MODE_SEED only; NULL = one national fraction): seed_label[a] is agent a's region in
+   * [0, n_seed_labels), and the seeding step draws agent a with q = 1 - seed_fraction[seed_label[a]] instead of
+   * 1 - seed_fraction[0].  The Philox counter is unchanged, so an agent whose region holds the national value draws
+   * exactly what it draws without a label table.  Codes are not checked on the device. */
+  const int32_t* seed_label;  /* [N] */
+  int32_t n_seed_labels;      /* 1 .. 2^30 */
+  int32_t _pad_seed;
 } gj_fwd_io;
 
 typedef struct gj_bwd_io {
@@ -336,7 +343,7 @@ typedef struct gj_bwd_io {
   float* g_q_out;   /* cotangent of q_in (stand-alone SAMPLE) */
   float* g_n_out;   /* cotangent of n_in (stand-alone INFECT / SYMPTOMS) */
   float* g_beta;    /* [n_nets] */
-  float* g_seed_fraction; /* [1] */
+  float* g_seed_fraction; /* [1], or [n_seed_labels] with seed_label */
   /* workspaces */
   float* w;   /* [N] */
   float* wq;  /* [N], may alias w when n_quar <= 0 */
@@ -348,6 +355,21 @@ typedef struct gj_bwd_io {
    * to that of its post-step current_stage where it equals dead; NULL = no label table */
   const int32_t* label;
   const float* g_red_label;
+  /* seeding by label (GJ_MODE_SEED only; NULL = one national fraction): the forward's seed_label / n_seed_labels.  The
+   * per-agent pass writes each agent's d/dseed_fraction (-dL/dq) to seed_work instead of folding it into one sum, and a
+   * reduction then writes g_seed_fraction[l] = sum over the agents of label l.  The library never allocates, so the
+   * caller passes the agents in label order: seed_order holds the agent ids stably sorted by label and seed_offsets
+   * the start of every label in it (seed_offsets[0] = 0, seed_offsets[n_seed_labels] = N; empty labels allowed).  The
+   * sum runs in fp64 over fixed chunks of seed_order whose partials are combined in chunk order: it is bit-reproducible
+   * and independent of the launch grid.  Each agent's fraction is q = 1 - seed_fraction[l]; a fraction below ~2^-24
+   * rounds q to 1 in fp32, and the sampler's d/dq then divides 0 by 0 for that agent, as the reference's torch code
+   * does (DESIGN.md, "Seeding by label"). */
+  const int32_t* seed_label;    /* [N] */
+  int32_t n_seed_labels;
+  int32_t _pad_seed;
+  const int32_t* seed_order;    /* [N] */
+  const int32_t* seed_offsets;  /* [n_seed_labels + 1] */
+  float* seed_work;             /* [N] workspace */
 } gj_bwd_io;
 
 /* ---- library ---------------------------------------------------------------------------- */
