@@ -44,12 +44,13 @@ static int bad(const char* what) {
 enum KernelId {
   K_TRANSMISSION = 0, K_GROUP_SMALL_F, K_GROUP_CHUNK_F, K_GROUP_FIX_F, K_AGENT_FWD,
   K_AGENT_BWD, K_GROUP_SMALL_B, K_GROUP_CHUNK_B, K_GROUP_FIX_B, K_DBETA, K_AGENT_BWD_GATHER, K_CELL, K_OTHER, K_SEED,
-  K_EXCHANGE, K_SEED_GRAD, K_COUNT
+  K_EXCHANGE, K_SEED_GRAD, K_REGION_GRAD, K_COUNT
 };
 static const char* kKernelNames[K_COUNT] = {
   "transmission", "group_small<fwd>", "group_chunk<fwd>", "group_fix<fwd>", "agent_forward",
   "agent_backward", "group_small<bwd>", "group_chunk<bwd>", "group_fix<bwd>", "dbeta",
-  "backward_gather", "cell_groups+gather", "other", "seeding", "boundary_exchange", "seed_label_grad"};
+  "backward_gather", "cell_groups+gather", "other", "seeding", "boundary_exchange", "seed_label_grad",
+  "region_factor_grad"};
 constexpr int kMaxProfiled = 16384;
 struct Profiler {
   bool on = false;
@@ -746,12 +747,12 @@ static bool pipe_aligned_fwd(const gj_world_desc* w, const LeanPlan& lp, const g
   return aligned16(io->s) && aligned16(io->inf) && aligned16(io->tinf) && aligned16(io->cur) && aligned16(io->nxt) &&
          aligned16(io->ttn) && aligned16(io->T) && aligned16(io->Tq) && aligned16(w->ent1) && aligned16(w->cls) &&
          aligned16(w->orig_id) &&
-         aligned16(lp.r_slot) && aligned16(lp.r_pc);
+         aligned16(lp.r_slot) && aligned16(lp.r_pc) && aligned16(io->region);
 }
 static bool pipe_aligned_bwd(const gj_world_desc* w, const LeanPlan& lp, const gj_bwd_io* io) {
   const void* ptrs[] = {io->s, io->inf, io->tinf, io->cur, io->nxt, io->ttn, io->tape_y0, io->tape_v, io->g_s_o,
                         io->g_inf_o, io->g_tinf_o, io->g_cur_o, io->g_nxt_o, io->g_ttn_o, io->prof4, io->g_inf,
-                        io->g_tinf, io->T_in, io->w, io->wq, w->ent1, w->cls, lp.r_slot, lp.r_pc};
+                        io->g_tinf, io->T_in, io->w, io->wq, w->ent1, w->cls, lp.r_slot, lp.r_pc, io->region};
   for (const void* q : ptrs)
     if (!aligned16(q)) return false;   // NULL counts as aligned
   return true;
@@ -1000,8 +1001,10 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
     static OccCache occ[20];
     const bool diag = io->q || io->n;
     const bool lab = io->label != nullptr;
+    const bool region = io->region != nullptr;   // a step with a regional factor never gets a look-ahead
     const size_t smem = next ? sizeof(PipeFwdSharedT<true, false>)
-                             : (batch ? sizeof(PipeFwdSharedT<false, true>) : sizeof(PipeFwdSharedT<false, false>));
+                             : (batch ? sizeof(PipeFwdSharedT<false, true>) : sizeof(PipeFwdSharedT<false, false>)) +
+                                   (region ? kPipeRegionBytes : 0);
     NextStep nx;
     memset(&nx, 0, sizeof(nx));
     if (next) {
@@ -1013,7 +1016,32 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
   launch_pdl(k_pipe_forward<Q, D, X, B, L>,                                                                           \
              dim3(pipe_grid(w, k_pipe_forward<Q, D, X, B, L>, kPipeThreads, smem, &occ[I], bt)), dim3(kPipeThreads),    \
              smem, st, *w, *p, lp, *io, (const float*)sc.cell_buf, sc.red_part, sc.tickets, nx, bt)
-    if (lab && batch) {   // a step with a label table never gets a look-ahead (step_forward_impl)
+#define GJ_PIPE_FWD_R(Q, D, B, L, I)                                                                                  \
+  launch_pdl(k_pipe_forward_region<Q, D, B, L>,                                                                       \
+             dim3(pipe_grid(w, k_pipe_forward_region<Q, D, B, L>, kPipeThreads, smem, &occ_r[I], bt)),                \
+             dim3(kPipeThreads), smem, st, *w, *p, lp, *io, (const float*)sc.cell_buf, sc.red_part, sc.tickets, nx, bt)
+    static OccCache occ_r[16];
+    if (region) {
+      const int i = (quar ? 8 : 0) | (diag ? 4 : 0) | (batch ? 2 : 0) | (lab ? 1 : 0);
+      switch (i) {
+        case 0: GJ_PIPE_FWD_R(false, false, false, false, 0); break;
+        case 1: GJ_PIPE_FWD_R(false, false, false, true, 1); break;
+        case 2: GJ_PIPE_FWD_R(false, false, true, false, 2); break;
+        case 3: GJ_PIPE_FWD_R(false, false, true, true, 3); break;
+        case 4: GJ_PIPE_FWD_R(false, true, false, false, 4); break;
+        case 5: GJ_PIPE_FWD_R(false, true, false, true, 5); break;
+        case 6: GJ_PIPE_FWD_R(false, true, true, false, 6); break;
+        case 7: GJ_PIPE_FWD_R(false, true, true, true, 7); break;
+        case 8: GJ_PIPE_FWD_R(true, false, false, false, 8); break;
+        case 9: GJ_PIPE_FWD_R(true, false, false, true, 9); break;
+        case 10: GJ_PIPE_FWD_R(true, false, true, false, 10); break;
+        case 11: GJ_PIPE_FWD_R(true, false, true, true, 11); break;
+        case 12: GJ_PIPE_FWD_R(true, true, false, false, 12); break;
+        case 13: GJ_PIPE_FWD_R(true, true, false, true, 13); break;
+        case 14: GJ_PIPE_FWD_R(true, true, true, false, 14); break;
+        default: GJ_PIPE_FWD_R(true, true, true, true, 15); break;
+      }
+    } else if (lab && batch) {   // a step with a label table never gets a look-ahead (step_forward_impl)
       if (quar && diag) GJ_PIPE_FWD(true, true, false, true, true, 19);
       else if (quar) GJ_PIPE_FWD(true, false, false, true, true, 18);
       else if (diag) GJ_PIPE_FWD(false, true, false, true, true, 17);
@@ -1040,6 +1068,7 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
       else GJ_PIPE_FWD(false, false, false, false, false, 0);
     }
 #undef GJ_PIPE_FWD
+#undef GJ_PIPE_FWD_R
     GJ_CHECK_LAUNCH("k_pipe_forward");
     return next ? 1 : 0;
   }
@@ -1051,7 +1080,23 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
 #define GJ_LEAN_FWD(Q, D, L, I)                                                                                       \
   k_lean_forward<Q, D, L><<<lean_grid(w, k_lean_forward<Q, D, L>, &occ[I]), kLeanThreads, 0, st>>>(                   \
       *w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets)
-    if (io->label) {
+#define GJ_LEAN_FWD_R(Q, D, L, I)                                                                                     \
+  k_lean_forward_region<Q, D, L><<<lean_grid(w, k_lean_forward_region<Q, D, L>, &occ_r[I]), kLeanThreads, 0, st>>>(     \
+      *w, *p, lp, *io, sc.cell_buf, sc.red_part, sc.tickets)
+    static OccCache occ_r[8];
+    if (io->region) {
+      if (io->label) {
+        if (quar && diag) GJ_LEAN_FWD_R(true, true, true, 7);
+        else if (quar) GJ_LEAN_FWD_R(true, false, true, 6);
+        else if (diag) GJ_LEAN_FWD_R(false, true, true, 5);
+        else GJ_LEAN_FWD_R(false, false, true, 4);
+      } else {
+        if (quar && diag) GJ_LEAN_FWD_R(true, true, false, 3);
+        else if (quar) GJ_LEAN_FWD_R(true, false, false, 2);
+        else if (diag) GJ_LEAN_FWD_R(false, true, false, 1);
+        else GJ_LEAN_FWD_R(false, false, false, 0);
+      }
+    } else if (io->label) {
       if (quar && diag) GJ_LEAN_FWD(true, true, true, 7);
       else if (quar) GJ_LEAN_FWD(true, false, true, 6);
       else if (diag) GJ_LEAN_FWD(false, true, true, 5);
@@ -1063,6 +1108,7 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
       else GJ_LEAN_FWD(false, false, false, 0);
     }
 #undef GJ_LEAN_FWD
+#undef GJ_LEAN_FWD_R
     GJ_CHECK_LAUNCH("k_lean_forward");
   }
   return 0;
@@ -1074,6 +1120,7 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
   const bool batch = bt.nb > 1;
   static OccCache occ_b[4], occ_g[2];
   const bool lab = io->label && io->g_red_label;
+  const bool region = io->region != nullptr;
   int gather_grid = 1;
   const bool pipe = pipe_enabled() && pipe_aligned_bwd(w, lp, io);
   if (batch && !pipe) return bad("batched step: the pipelined kernels are off or an array is not 16-byte aligned");
@@ -1081,11 +1128,28 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
     if (pipe) {
       ProfScope ps(K_AGENT_BWD, st);
       static OccCache occ[8];
-      const size_t smem = sizeof(PipeBwdShared);
+      const size_t smem = sizeof(PipeBwdShared) + (region ? kPipeRegionBytes : 0);
 #define GJ_PIPE_BWD(Q, B, L, I)                                                                                       \
   launch_pdl(k_pipe_backward<Q, B, L>, dim3(pipe_grid(w, k_pipe_backward<Q, B, L>, kBwdThreads, smem, &occ[I], bt)),    \
              dim3(kBwdThreads), smem, st, *w, *p, lp, *io, sc.tile_part, bt)
-      if (lab && batch) {
+#define GJ_PIPE_BWD_R(Q, B, L, I)                                                                                     \
+  launch_pdl(k_pipe_backward_region<Q, B, L>,                                                                         \
+             dim3(pipe_grid(w, k_pipe_backward_region<Q, B, L>, kBwdThreads, smem, &occ_r[I], bt)), dim3(kBwdThreads), \
+             smem, st, *w, *p, lp, *io, sc.tile_part, bt)
+      static OccCache occ_r[8];
+      if (region) {
+        const int i = (quar ? 4 : 0) | (batch ? 2 : 0) | (lab ? 1 : 0);
+        switch (i) {
+          case 0: GJ_PIPE_BWD_R(false, false, false, 0); break;
+          case 1: GJ_PIPE_BWD_R(false, false, true, 1); break;
+          case 2: GJ_PIPE_BWD_R(false, true, false, 2); break;
+          case 3: GJ_PIPE_BWD_R(false, true, true, 3); break;
+          case 4: GJ_PIPE_BWD_R(true, false, false, 4); break;
+          case 5: GJ_PIPE_BWD_R(true, false, true, 5); break;
+          case 6: GJ_PIPE_BWD_R(true, true, false, 6); break;
+          default: GJ_PIPE_BWD_R(true, true, true, 7); break;
+        }
+      } else if (lab && batch) {
         if (quar) GJ_PIPE_BWD(true, true, true, 7);
         else GJ_PIPE_BWD(false, true, true, 6);
       } else if (lab) {
@@ -1099,12 +1163,25 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
         else GJ_PIPE_BWD(false, false, false, 0);
       }
 #undef GJ_PIPE_BWD
+#undef GJ_PIPE_BWD_R
       GJ_CHECK_LAUNCH("k_pipe_backward");
     } else {
       ProfScope ps(K_AGENT_BWD, st);
 #define GJ_LEAN_BWD(Q, L, I) \
   k_lean_backward<Q, L><<<lean_grid(w, k_lean_backward<Q, L>, &occ_b[I]), kLeanThreads, 0, st>>>(*w, *p, lp, *io, sc.tile_part)
-      if (lab) {
+#define GJ_LEAN_BWD_R(Q, L, I)                                                                                        \
+  k_lean_backward_region<Q, L><<<lean_grid(w, k_lean_backward_region<Q, L>, &occ_br[I]), kLeanThreads, 0, st>>>(        \
+      *w, *p, lp, *io, sc.tile_part)
+      static OccCache occ_br[4];
+      if (region) {
+        if (lab) {
+          if (quar) GJ_LEAN_BWD_R(true, true, 3);
+          else GJ_LEAN_BWD_R(false, true, 2);
+        } else {
+          if (quar) GJ_LEAN_BWD_R(true, false, 1);
+          else GJ_LEAN_BWD_R(false, false, 0);
+        }
+      } else if (lab) {
         if (quar) GJ_LEAN_BWD(true, true, 3);
         else GJ_LEAN_BWD(false, true, 2);
       } else {
@@ -1112,6 +1189,7 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
         else GJ_LEAN_BWD(false, false, 0);
       }
 #undef GJ_LEAN_BWD
+#undef GJ_LEAN_BWD_R
       GJ_CHECK_LAUNCH("k_lean_backward");
     }
     if (lp.has_generic)
@@ -1569,6 +1647,8 @@ static int make_batch(const gj_world_desc* w, const gj_step_params* p, const gj_
   bt->sRed = (int)b->red_stride;
   bt->noise = b->noise;
   bt->sLab = b->label_stride;
+  bt->sReg = b->region_stride;
+  if (b->region_stride < 0) return bad("batch: region_stride must be >= 0");
   if (b->noise && !aligned16(b->noise)) return bad("batch: noise must be 16-byte aligned");
   return 0;
 }
@@ -1579,6 +1659,14 @@ static int check_labels(const gj_fwd_io* io, const Batch& bt) {
   if (io->n_labels < 1 || io->n_labels > (1 << 30)) return bad("n_labels must lie in [1, 2^30]");
   if (!io->red_label || !io->label_acc) return bad("label given without red_label / label_acc");
   if (bt.nb > 1 && bt.sLab < 2 * (int64_t)io->n_labels) return bad("batch: label_stride must be >= 2 * n_labels");
+  return 0;
+}
+// regional transmission factor: the checks of the header (the codes and factors themselves are not checked)
+static int check_region(const int32_t* region, int n_regions, const float* factor, const Batch& bt) {
+  if (!region) return 0;
+  if (n_regions < 1 || n_regions > (1 << 30)) return bad("n_regions must lie in [1, 2^30]");
+  if (!factor) return bad("region given without region_factor");
+  if (bt.nb > 1 && bt.sReg < (int64_t)n_regions) return bad("batch: region_stride must be >= n_regions");
   return 0;
 }
 static int finish_labels(const gj_fwd_io* io, cudaStream_t st, const Batch& bt) {
@@ -1603,6 +1691,7 @@ static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, co
   if (batch)
     if (int e = make_batch(w, p, batch, &bt)) return e;
   if (int e = check_labels(io, bt)) return e;
+  if (int e = check_region(io->region, io->n_regions, io->region_factor, bt)) return e;
   const int rc = step_forward_run(w, p, next, io, stream, batch);
   if (rc < 0 || p->stage == GJ_STAGE_SUMS) return rc;
   if (int e = finish_labels(io, (cudaStream_t)stream, bt)) return e;
@@ -1701,7 +1790,7 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
       // look-ahead: the following step must itself run on the throughput-mode kernels (it then honours t_ready)
       NextStep nx;
       bool have_next = false;
-      if (next && !io->label && lookahead_enabled() && io->T_next && next->mode == GJ_MODE_STEP && next->phases == GJ_PHASE_ALL &&
+      if (next && !io->label && !io->region && lookahead_enabled() && io->T_next && next->mode == GJ_MODE_STEP && next->phases == GJ_PHASE_ALL &&
           (next->n_quar <= 0 || io->Tq_next)) {
         Channels chn;
         Plan pln;
@@ -1752,7 +1841,11 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
   if (int e = launch_cell_gather(w, &pp, pl, io->S_scaled, sc, st)) return e;
   {
     ProfScope ps(K_AGENT_FWD, st);
-    if (io->label) k_tile_forward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
+    if (io->region && io->label)
+      k_tile_forward_region<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
+    else if (io->region)
+      k_tile_forward_region<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
+    else if (io->label) k_tile_forward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
     else k_tile_forward<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.cell_buf, sc.red_part, sc.tickets);
     GJ_CHECK_LAUNCH("k_tile_forward");
   }
@@ -1788,6 +1881,22 @@ static int64_t seed_chunk(const gj_world_desc* w) {
   while (2 * ((w->n_agents + chunk - 1) / chunk) > slots) chunk *= 2;
   return chunk;
 }
+// out[l] = sum of work over the agents of label l (order / offsets: the agents stably sorted by label), in fp64 over
+// fixed chunks combined in chunk order: bit-reproducible and independent of the launch grid
+static int label_sums(const gj_world_desc* w, const int32_t* order, const int32_t* offsets, int n_labels,
+                      const float* work, const Scratch& sc, float* out, cudaStream_t st) {
+  const int64_t N = w->n_agents;
+  const int64_t chunk = seed_chunk(w);
+  const int64_t n_chunks = (N + chunk - 1) / chunk;
+  k_seed_label_grad<<<blocks_for(n_chunks * 32, kBlock), kBlock, 0, st>>>(N, chunk, order, offsets, n_labels, work,
+                                                                         sc.red_part, out);
+  GJ_CHECK_LAUNCH("k_seed_label_grad");
+  k_seed_label_fix<<<blocks_for((int64_t)n_labels * 32, kBlock), kBlock, 0, st>>>(chunk, offsets, n_labels, sc.red_part,
+                                                                                  out);
+  GJ_CHECK_LAUNCH("k_seed_label_fix");
+  return 0;
+}
+
 static int seed_backward(const gj_world_desc* w, const gj_step_params& pp, const gj_bwd_io* io, const Scratch& sc,
                          cudaStream_t st) {
   if (io->n_seed_labels < 1 || io->n_seed_labels > (1 << 30)) return bad("n_seed_labels must lie in [1, 2^30]");
@@ -1802,15 +1911,20 @@ static int seed_backward(const gj_world_desc* w, const gj_step_params& pp, const
   }
   if (!io->g_seed_fraction) return 0;
   ProfScope ps(K_SEED_GRAD, st);
-  const int64_t chunk = seed_chunk(w);
-  const int64_t n_chunks = (N + chunk - 1) / chunk;
-  k_seed_label_grad<<<blocks_for(n_chunks * 32, kBlock), kBlock, 0, st>>>(N, chunk, io->seed_order, io->seed_offsets,
-                                                                         io->n_seed_labels, io->seed_work, sc.red_part,
-                                                                         io->g_seed_fraction);
-  GJ_CHECK_LAUNCH("k_seed_label_grad");
-  k_seed_label_fix<<<blocks_for((int64_t)io->n_seed_labels * 32, kBlock), kBlock, 0, st>>>(
-      chunk, io->seed_offsets, io->n_seed_labels, sc.red_part, io->g_seed_fraction);
-  GJ_CHECK_LAUNCH("k_seed_label_fix");
+  return label_sums(w, io->seed_order, io->seed_offsets, io->n_seed_labels, io->seed_work, sc, io->g_seed_fraction, st);
+}
+
+// regional transmission factor, backward: the agent kernels wrote d/dlam' * lam to region_work; the same per-label
+// reduction as seeding by label sums it per region, once per sample (after the agent pass, so sample 0's reduction
+// partials are free).  With a partitioned world it runs in the second stage, after every agent has written its term.
+static int region_backward(const gj_world_desc* w, const gj_bwd_io* io, const Scratch& sc, const Batch& bt,
+                           cudaStream_t st) {
+  if (!io->region || !io->g_region_factor) return 0;
+  ProfScope ps(K_REGION_GRAD, st);
+  for (int s = 0; s < bt.nb; ++s)
+    if (int e = label_sums(w, io->region_order, io->region_offsets, io->n_regions, io->region_work + (int64_t)s * bt.sN,
+                           sc, io->g_region_factor + (int64_t)s * bt.sReg, st))
+      return e;
   return 0;
 }
 
@@ -1845,6 +1959,11 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if (!io->w || !io->wq || !io->R || !io->cR || !io->tape_v || !io->S_unscaled || !io->beta || !io->s || !io->T_in)
     return bad("backward workspaces are NULL");
   if (p->n_quar > 0 && !io->cur) return bad("cur is NULL with an active quarantine");
+  if (int e = check_region(io->region, io->n_regions, io->region_factor, bt)) return e;
+  if (io->region && !io->region_work) return bad("region given without region_work");
+  if (io->region && io->g_region_factor && (!io->region_order || !io->region_offsets))
+    return bad("g_region_factor given without region_order / region_offsets");
+  const bool region_last = io->region && pp.stage != GJ_STAGE_SUMS;   // the per-region reduction ends the call
   if (!io->g_T && (!io->tinf || !io->inf || !io->maxinf || !io->k0 || !io->g_inf || !io->g_tinf))
     return bad("state arrays are NULL");
   {
@@ -1856,7 +1975,8 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
         return bad("fused step backward: state / tape arrays are NULL");
       if (batch && batch->n_samples > 1 && batch->group_stride < lp.gen_base + w->n_groups)
         return bad("batch: group_stride smaller than the group-sum buffers");
-      return lean_backward(w, &pp, pl, lp, io, sc, st, bt);
+      if (int e = lean_backward(w, &pp, pl, lp, io, sc, st, bt)) return e;
+      return region_last ? region_backward(w, io, sc, bt, st) : 0;
     }
   }
   if (batch) return bad("batch: this step does not run on the throughput-mode kernels (gj_step_plan = 0, injected noise, or no packed profile)");
@@ -1864,7 +1984,10 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if (pp.stage != GJ_STAGE_REST) {
     {
       ProfScope ps(K_AGENT_BWD, st);
-      if (io->label && io->g_red_label) k_tile_backward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
+      const bool lab = io->label && io->g_red_label;
+      if (io->region && lab) k_tile_backward_region<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
+      else if (io->region) k_tile_backward_region<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
+      else if (lab) k_tile_backward<true><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
       else k_tile_backward<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
       GJ_CHECK_LAUNCH("k_tile_backward");
     }
@@ -1890,7 +2013,7 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
                                       io->g_beta, kNoBatch);
     GJ_CHECK_LAUNCH("k_dbeta");
   }
-  return 0;
+  return region_last ? region_backward(w, io, sc, bt, st) : 0;
 }
 
 int gj_step_backward(const gj_world_desc* w, const gj_step_params* p, const gj_bwd_io* io, void* stream) {

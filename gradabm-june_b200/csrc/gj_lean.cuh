@@ -692,23 +692,26 @@ __device__ __forceinline__ float lean_noise_dE(uint32_t r0, uint32_t r1) {
   return lg2_fast(fmaxf(-lg2_fast(u01_open(r0)), kMinE2)) - lg2_fast(fmaxf(-lg2_fast(u01_open(r1)), kMinE2));
 }
 // dE: lean_noise_dE of the agent's Philox pair; ga = its id in the noise stream
-template <bool kQuar>
+// kRegion: the pressure is multiplied by the agent's regional factor mreg before the clamp (the tape keeps lam)
+template <bool kQuar, bool kRegion = false>
 __device__ __forceinline__ FwdRes lean_forward_core(const gj_step_params& p, const LeanPlan& lp,
                                                     const float* __restrict__ stage_prob, uint64_t ga, float dE,
                                                     float hs, float gv, float Lc, float beta_r, float rpc,
                                                     float s, float inf, float tinf, float cur, float nxt, float ttn,
                                                     int cls, float inv_tau, float dead, float* __restrict__ hist,
-                                                    float* __restrict__ deaths, float q_seed = -1.0f) {
+                                                    float* __restrict__ deaths, float q_seed = -1.0f,
+                                                    float mreg = 1.0f) {
   FwdRes o;
   const float rv = (beta_r * rpc) * hs;
   const float house = lp.r_house ? rv : 0.0f;
   const float plain = (gv + Lc) + (lp.r_house ? 0.0f : rv);
   const float mq = kQuar ? quar_mask(p, cur) : 1.0f;
   const float X = fmaf(mq, plain, house);  // pressure per unit susceptibility
-  const float lam = X * s;
+  const float lam0 = X * s;
+  const float lam = kRegion ? lam0 * mreg : lam0;
   // q_seed >= 0: the seeding step (infect_fraction_of_people, infection.py:31-42): a uniform q = 1 - fraction
   const float q = (q_seed >= 0.0f) ? q_seed : not_infected_prob(lam, p.dt);
-  o.tape_v = (s == 0.0f) ? X : lam;
+  o.tape_v = (s == 0.0f) ? X : lam0;
   // Gumbel-softmax hard draw from Philox bits (same stream as draw_step_noise):
   // x0 - x1 = (ln2 / tau) * d,  d = lg2 q - lg2(1-q) - lg2 E0 + lg2 E1, E = -ln u (the ln2 factors cancel)
   const float d = (lg2_fast(q) - lg2_fast(1.0f - q)) - dE;
@@ -741,21 +744,22 @@ __device__ __forceinline__ FwdRes lean_forward_core(const gj_step_params& p, con
 }
 
 // one agent: noise, core, stores
-template <bool kQuar, bool kDiag>
+template <bool kQuar, bool kDiag, bool kRegion = false>
 __device__ __forceinline__ FwdOut lean_forward_agent(const gj_step_params& p, const LeanPlan& lp, const gj_fwd_io& io,
                                                    uint32_t a, uint64_t ga, float hs, float gv, float Lc, float beta_r, float rpc,
                                                    float s, float inf, float tinf, float cur, float nxt, float ttn,
                                                    int cls, float inv_tau, float dead, float* __restrict__ hist,
                                                    float* __restrict__ deaths, bool noise_given = false,
-                                                   float dE_given = 0.0f) {
+                                                   float dE_given = 0.0f, float mreg = 1.0f) {
   float dE = dE_given;   // batched ensemble: evaluated once for all samples (k_batch_noise)
   if (!noise_given) {
     uint32_t r[2];
     philox_step_pair(p.seed, p.call_index, ga, r);   // ga: the agent's id in the noise stream (noise_agent())
     dE = lean_noise_dE(r[0], r[1]);
   }
-  const FwdRes o = lean_forward_core<kQuar>(p, lp, io.stage_prob, ga, dE, hs, gv, Lc, beta_r, rpc, s, inf, tinf,
-                                            cur, nxt, ttn, cls, inv_tau, dead, hist, deaths);
+  const FwdRes o = lean_forward_core<kQuar, kRegion>(p, lp, io.stage_prob, ga, dE, hs, gv, Lc, beta_r, rpc, s, inf,
+                                                     tinf, cur, nxt, ttn, cls, inv_tau, dead, hist, deaths, -1.0f,
+                                                     mreg);
   io.tape_v[a] = o.tape_v;
   io.tape_y0[a] = o.tape_y0;
   if (kDiag) {
@@ -802,11 +806,12 @@ struct LeanFwdShared {
 
 constexpr int kLeanBatch = 2;  // agents a thread keeps in flight: their loads are issued before any arithmetic
 
-template <bool kQuar, bool kDiag, bool kLabel>
-__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
-                                                                  gj_fwd_io io, const float* __restrict__ cell_buf,
-                                                                  double* __restrict__ red_part,
-                                                                  unsigned int* __restrict__ ticket) {
+// kRegion: regional transmission factor (gj_fwd_io.region): the code is loaded with the batch's other per-agent
+// operands, the factor gathered (R floats, L1/L2-resident) before the arithmetic
+template <bool kQuar, bool kDiag, bool kLabel, bool kRegion>
+__device__ __forceinline__ void lean_forward_body(const gj_world_desc& w, const gj_step_params& p, const LeanPlan& lp,
+                                                  const gj_fwd_io& io, const float* __restrict__ cell_buf,
+                                                  double* __restrict__ red_part, unsigned int* __restrict__ ticket) {
   __shared__ LeanFwdShared sh;
   lean_load_prob<true>(sh.prob, p, lp, io.leisure_prob);
   if (threadIdx.x < p.n_nets) sh.beta[threadIdx.x] = io.beta[threadIdx.x];
@@ -858,6 +863,7 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
       RangeLoads rl[kLeanBatch];
       uint32_t ent[kLeanBatch], slot[kLeanBatch], oid[kLeanBatch];
       int cls[kLeanBatch];
+      int32_t reg[kLeanBatch];
       // ---- issue every load of the batch: gathers (addresses known from the previous iteration), streaming
       //      loads, and the next batch's index words --------------------------------------------------------
 #pragma unroll
@@ -877,11 +883,15 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
         cls[h] = w.cls[al];
         rpc[h] = has_range ? lp.r_pc[al] : 0.0f;
         oid[h] = w.orig_id ? w.orig_id[al] : 0u;
+        if (kRegion) reg[h] = io.region[al];
         const uint32_t an = a + kLeanBatch * kLeanThreads;
         const uint32_t anl = (an < a1) ? an : a0;
         ent_n[h] = has_gen ? i_ent[anl] : kEntNone;
         slot_n[h] = has_range ? i_slot[anl] : kNoSlot;
       }
+      float mreg[kLeanBatch];
+#pragma unroll
+      for (int h = 0; h < kLeanBatch; ++h) mreg[h] = kRegion ? __ldg(io.region_factor + reg[h]) : 1.0f;
       // ---- arithmetic and stores ------------------------------------------------------------------------------
 #pragma unroll
       for (int h = 0; h < kLeanBatch; ++h) {
@@ -891,9 +901,9 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
         const float gv = lean_generic_finish(w, SP, ent[h], a, gen[h]);
         const float Lc = lp.n_cell > 0 ? L[cls[h]] : 0.0f;
         const uint64_t ga = w.orig_id ? (uint64_t)oid[h] : p.agent_offset + a;
-        const FwdOut o = lean_forward_agent<kQuar, kDiag>(p, lp, io, a, ga, hs, gv, Lc, beta_r, rpc[h], s[h], inf[h],
-                                                          tinf[h], cur[h], nxt[h], ttn[h], cls[h], inv_tau, dead, sh.hist,
-                                                          &sh.deaths);
+        const FwdOut o = lean_forward_agent<kQuar, kDiag, kRegion>(p, lp, io, a, ga, hs, gv, Lc, beta_r, rpc[h], s[h],
+                                                                   inf[h], tinf[h], cur[h], nxt[h], ttn[h], cls[h], inv_tau,
+                                                                   dead, sh.hist, &sh.deaths, false, 0.0f, mreg[h]);
         if (kLabel) label_add(io.label_acc, io.label, a, (uint32_t)o.inf, o.cur == dead ? 1u : 0u);
       }
     }
@@ -916,6 +926,24 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward
     }
     finish_partials<kMaxRed>(nr, red_part, gridDim.x, ticket, io.red);
   }
+}
+
+template <bool kQuar, bool kDiag, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
+                                                                  gj_fwd_io io, const float* __restrict__ cell_buf,
+                                                                  double* __restrict__ red_part,
+                                                                  unsigned int* __restrict__ ticket) {
+  lean_forward_body<kQuar, kDiag, kLabel, false>(w, p, lp, io, cell_buf, red_part, ticket);
+}
+
+// the same with the regional transmission factor (gj_fwd_io.region)
+template <bool kQuar, bool kDiag, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_FWD) k_lean_forward_region(gj_world_desc w, gj_step_params p,
+                                                                  LeanPlan lp, gj_fwd_io io,
+                                                                  const float* __restrict__ cell_buf,
+                                                                  double* __restrict__ red_part,
+                                                                  unsigned int* __restrict__ ticket) {
+  lean_forward_body<kQuar, kDiag, kLabel, true>(w, p, lp, io, cell_buf, red_part, ticket);
 }
 
 // =====================================================================================================
@@ -1024,7 +1052,9 @@ __global__ void __launch_bounds__(kLeanThreads, 4) k_lean_seed_by(gj_world_desc 
 // per-agent arithmetic of the backward pass (shared with gj_pipe.cuh): symptoms^T, infect^T, sampler^T, clamp/exp
 // chain -> cotangents of the state, w = dL/dLambda * s (and its quarantine-masked copy), cell-channel sums in acc
 // kLabel: glab_i / glab_d are the cotangents of the agent's column of the label table (cases, and deaths / dead)
-template <bool kQuar, bool kLabel = false>
+// kRegion: the forward multiplied the pressure by the regional factor mreg before the clamp: the clamp gates d/dlam',
+// d/dlam' * lam goes to io.region_work and d/dlam' * mreg down the chain
+template <bool kQuar, bool kLabel = false, bool kRegion = false>
 __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, const LeanPlan& lp, const gj_bwd_io& io,
                                                     uint32_t a, float s, float tinf, float cur, float nxt, float ttn,
                                                     float ty, float v, int cls, float gs_o, float ginf_o, float gtinf_o,
@@ -1032,7 +1062,7 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
                                                     float g_deaths, const float* __restrict__ gred_age,
                                                     const ProbRow* __restrict__ prob, float (&acc)[GJ_MAX_CHANNELS],
                                                     const uint32_t* __restrict__ orig_id, uint32_t soff = 0u,
-                                                    float glab_i = 0.0f, float glab_d = 0.0f) {
+                                                    float glab_i = 0.0f, float glab_d = 0.0f, float mreg = 1.0f) {
     // soff: batched ensemble — this sample's offset into the per-sample arrays (outputs below); the agent's id in the
     // world and in the noise stream stays `a`
     const int age = age_of(cls);
@@ -1070,7 +1100,8 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
     const float g_tinf = gtinf_o * (1.0f - n);
     // sampler^T and the clamp / exp chain: dL/dq = gl0/q - gl1/(1-q), dL/dLambda = dL/dq * q * (-dt)
     // evaluated as (gl1 * q/(1-q) - gl0) * dt
-    const float lam = (s == 0.0f) ? 0.0f : v;
+    const float lam0 = (s == 0.0f) ? 0.0f : v;
+    const float lam = kRegion ? lam0 * mreg : lam0;
     const float q = not_infected_prob(lam, p.dt);
     float y0, y1;
     decode_soft(ty, y0, y1);
@@ -1079,11 +1110,15 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
     const float gl0 = ((gret0 - dot) * y0) * inv_tau, gl1 = ((0.0f - dot) * y1) * inv_tau;
     float glam = 0.0f;
     if (lam >= 1e-6f && lam <= 100.0f) glam = (gl1 * (q * rcp_fast(1.0f - q)) - gl0) * p.dt;
+    const uint32_t ao = a + soff;
+    if (kRegion) {
+      io.region_work[ao] = glam * lam0;
+      glam = glam * mreg;
+    }
     const float X = (s == 0.0f) ? v : ((s == 1.0f) ? v : v * rcp_fast(s));
     g_s += glam * X;
     // outputs
     const float wv = glam * s;
-    const uint32_t ao = a + soff;
     io.w[ao] = wv;
     float wqv = wv;
     if (kQuar) {
@@ -1103,9 +1138,9 @@ __device__ __forceinline__ void lean_backward_agent(const gj_step_params& p, con
 // B1  backward, per agent: symptoms^T, infect^T, sampler^T, clamp/exp chain -> cotangents of the state,
 //     w = dL/dLambda * s (and its quarantine-masked copy), partial sums of the cell channels (as in K1)
 // =====================================================================================================
-template <bool kQuar, bool kLabel>
-__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
-                                                                   gj_bwd_io io, float* __restrict__ tile_part) {
+template <bool kQuar, bool kLabel, bool kRegion>
+__device__ __forceinline__ void lean_backward_body(const gj_world_desc& w, const gj_step_params& p, const LeanPlan& lp,
+                                                   const gj_bwd_io& io, float* __restrict__ tile_part) {
   __shared__ ProbRow prob[200];
   __shared__ float gred_age[100];  // cotangent of is_infected from the cases / cases-by-age reductions
   lean_load_prob<true>(prob, p, lp, io.leisure_prob);
@@ -1151,10 +1186,12 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backwar
       float gs_o[kLeanBatch], ginf_o[kLeanBatch], gtinf_o[kLeanBatch], gcur_o[kLeanBatch], gnxt_o[kLeanBatch],
           gttn_o[kLeanBatch];
       int cls[kLeanBatch];
+      int32_t reg[kLeanBatch];
 #pragma unroll
       for (int h = 0; h < kLeanBatch; ++h) {
         const uint32_t a = base + h * kLeanThreads;
         const uint32_t al = (a < a1) ? a : a0;
+        if (kRegion) reg[h] = io.region[al];
         s[h] = i_s[al];
         tinf[h] = i_tinf[al];
         cur[h] = i_cur[al];
@@ -1180,9 +1217,11 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backwar
           glab_i = io.g_red_label[2 * l];
           glab_d = io.g_red_label[2 * l + 1] / dead;
         }
-        lean_backward_agent<kQuar, kLabel>(p, lp, io, a, s[h], tinf[h], cur[h], nxt[h], ttn[h], ty[h], v[h], cls[h],
-                                           gs_o[h], ginf_o[h], gtinf_o[h], gcur_o[h], gnxt_o[h], gttn_o[h], inv_tau,
-                                           dead, g_deaths, gred_age, prob, acc, w.orig_id, 0u, glab_i, glab_d);
+        const float mreg = kRegion ? __ldg(io.region_factor + reg[h]) : 1.0f;
+        lean_backward_agent<kQuar, kLabel, kRegion>(p, lp, io, a, s[h], tinf[h], cur[h], nxt[h], ttn[h], ty[h], v[h],
+                                                    cls[h], gs_o[h], ginf_o[h], gtinf_o[h], gcur_o[h], gnxt_o[h],
+                                                    gttn_o[h], inv_tau, dead, g_deaths, gred_age, prob, acc, w.orig_id,
+                                                    0u, glab_i, glab_d, mreg);
       }
     }
     if (lp.n_cell > 0) {
@@ -1196,6 +1235,20 @@ __global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backwar
       }
     }
   }
+}
+
+template <bool kQuar, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
+                                                                   gj_bwd_io io, float* __restrict__ tile_part) {
+  lean_backward_body<kQuar, kLabel, false>(w, p, lp, io, tile_part);
+}
+
+// the same with the regional transmission factor (gj_bwd_io.region)
+template <bool kQuar, bool kLabel>
+__global__ void __launch_bounds__(kLeanThreads, GJ_LEAN_MINB_BWD) k_lean_backward_region(gj_world_desc w, gj_step_params p,
+                                                                   LeanPlan lp, gj_bwd_io io,
+                                                                   float* __restrict__ tile_part) {
+  lean_backward_body<kQuar, kLabel, true>(w, p, lp, io, tile_part);
 }
 
 // per-agent arithmetic of the backward gather (shared with gj_pipe.cuh): dL/dT from the three tiers ->

@@ -217,19 +217,22 @@ struct PipeFwdSharedT {
 
 // so: batched ensemble — this sample's offset into the per-sample arrays (a multiple of four agents: the copies stay
 // 16-byte aligned); the world's arrays are shared
-template <bool kBatch>
+// kRegion: also the region codes (gj_fwd_io.region) into `reg`, the stage's slice of the region staging area
+template <bool kBatch, bool kRegion = false>
 __device__ __forceinline__ void pipe_fwd_issue(PipeFwdStageT<kBatch>& sg, uint64_t* bar, const gj_world_desc& w,
                                                const LeanPlan& lp, const gj_fwd_io& io, const float* Tr, int64_t tile,
                                                bool has_gen, bool has_range, uint32_t so = 0u,
-                                               const float* noise = nullptr) {
+                                               const float* noise = nullptr, int32_t* reg = nullptr) {
   const TileSpan t = tile_span(w, tile);
   uint32_t total = 6u * t.n4 + (t.hi16 - t.lo16);
+  if (kRegion) total += t.n4;
   if (kBatch && noise) total += t.n4;
   if (has_gen) total += t.n4;
   if (w.orig_id) total += t.n4;
   if (has_range) total += (lp.r_pc_lut ? 1u : 2u) * t.n4 + (t.thi - t.tlo) * 4u;
   mbar_expect_tx(bar, total);
   const Copier c{bar};
+  if (kRegion) c.f4(reg, io.region, t);
   if (kBatch && noise) c.f4(sg.dE, noise, t);
   if (w.orig_id) c.f4(sg.oid, w.orig_id, t);
   c.f4(sg.s, io.s + so, t);
@@ -247,28 +250,37 @@ __device__ __forceinline__ void pipe_fwd_issue(PipeFwdStageT<kBatch>& sg, uint64
   bulk_g2s(sg.cls, w.cls + t.lo16, t.hi16 - t.lo16, bar);
 }
 
-template <bool kQuar, bool kDiag, bool kNext, bool kBatch, bool kLabel>
-__global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
-                                                                 gj_fwd_io io, const float* __restrict__ cell_buf,
-                                                                 double* __restrict__ red_part,
-                                                                 unsigned int* __restrict__ ticket, NextStep nx,
-                                                                 Batch bt) {
+// region staging (kRegion): kPipeStages slices of kPipeF region codes, in the dynamic shared memory right after the
+// kernel's shared struct (whose size is a multiple of 16), so the other instantiations keep their layout
+constexpr size_t kPipeRegionBytes = sizeof(int32_t) * kPipeStages * kPipeF;
+
+// kRegion: regional transmission factor (gj_fwd_io.region): the code is staged with the tile's other operands and the
+// factor gathered from region_factor (R floats, cached)
+template <bool kQuar, bool kDiag, bool kNext, bool kBatch, bool kLabel, bool kRegion>
+__device__ __forceinline__ void pipe_forward_body(const gj_world_desc& w, const gj_step_params& p, const LeanPlan& lp,
+                                                  const gj_fwd_io& io, const float* __restrict__ cell_buf,
+                                                  double* __restrict__ red_part, unsigned int* __restrict__ ticket,
+                                                  NextStep nx, const Batch& bt) {
   static_assert(!(kNext && kBatch), "the look-ahead transmission pass is not batched");
   static_assert(!(kNext && kLabel), "a step with a label table runs without the look-ahead");
+  static_assert(!(kNext && kRegion), "a step with a regional factor runs without the look-ahead");
   extern __shared__ __align__(128) unsigned char pipe_smem[];
   PipeFwdSharedT<kNext, kBatch>& sh = *reinterpret_cast<PipeFwdSharedT<kNext, kBatch>*>(pipe_smem);
+  int32_t* const reg_st = reinterpret_cast<int32_t*>(pipe_smem + sizeof(PipeFwdSharedT<kNext, kBatch>));
   const BatchCta bc = batch_cta<kBatch>(bt);
   const float* noise = kBatch ? bt.noise : nullptr;
   const uint32_t so = bc.so;
   float* __restrict__ red_out = io.red;
   const float* __restrict__ beta_in = io.beta;
   uint32_t* __restrict__ lacc = io.label_acc;
+  const float* __restrict__ rfac = io.region_factor;
   if (kBatch) {   // this sample's slices of the scratch and of the small per-sample arrays
     cell_buf = scr_shift(cell_buf, bt, bc.s);
     red_part = scr_shift(red_part, bt, bc.s);
     ticket = scr_shift(ticket, bt, bc.s);
     if (red_out) red_out += (int64_t)bc.s * bt.sRed;
     if (kLabel) lacc += bc.s * bt.sLab;
+    if (kRegion) rfac += bc.s * bt.sReg;
     beta_in += (int64_t)bc.s * bt.sBeta;
   }
   const TileRun run = lean_tiles(w, bc);
@@ -292,7 +304,8 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
   if (threadIdx.x == 0) {
     for (int i = 0; i < kPipeStages; ++i)
       if (run.t0 + i < run.t1)
-        pipe_fwd_issue<kBatch>(sh.st[i], &sh.full[i], w, lp, io, Tr, run.t0 + i, has_gen, has_range, so, noise);
+        pipe_fwd_issue<kBatch, kRegion>(sh.st[i], &sh.full[i], w, lp, io, Tr, run.t0 + i, has_gen, has_range, so,
+                                        noise, reg_st + i * kPipeF);
   }
   const float* __restrict__ SP = io.S_scaled + lp.gen_base + (kBatch ? (int64_t)bc.s * bt.sG : (int64_t)0);
   const float dead = (float)(p.n_stages - 1);
@@ -344,10 +357,11 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
       const uint64_t ga = w.orig_id ? (uint64_t)sg.oid[i] : p.agent_offset + a;
       const float rpc = !has_range ? 0.0f : (lp.r_pc_lut ? ((sg.slot[i] == kNoSlot) ? 0.0f : sh.pc_lut[sg.slot[i] & 0xFFFFu])
                                                          : sg.rpc[i]);
-      const FwdOut o = lean_forward_agent<kQuar, kDiag>(p, lp, io, a + so, ga, hs, gv, Lc, beta_r, rpc,
+      const float mreg = kRegion ? __ldg(rfac + reg_st[stg * kPipeF + i]) : 1.0f;
+      const FwdOut o = lean_forward_agent<kQuar, kDiag, kRegion>(p, lp, io, a + so, ga, hs, gv, Lc, beta_r, rpc,
                                                         sg.s[i], sg.inf[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i], cls,
                                                         inv_tau, dead, sh.hist, &sh.deaths, kBatch && noise != nullptr,
-                                                        (kBatch && noise) ? sg.dE[i] : 0.0f);
+                                                        (kBatch && noise) ? sg.dE[i] : 0.0f, mreg);
       if (kLabel) label_add(lacc, io.label, a, (uint32_t)o.inf, o.cur == dead ? 1u : 0u);
       if (kNext) {   // TransmissionUpdater of the next step (same arithmetic as k_lean_transmission)
         float T = 0.0f;
@@ -368,7 +382,8 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
       }
     }
     if (pipe_release() && tile + kPipeStages < run.t1)
-      pipe_fwd_issue<kBatch>(sg, &sh.full[stg], w, lp, io, Tr, tile + kPipeStages, has_gen, has_range, so, noise);
+      pipe_fwd_issue<kBatch, kRegion>(sg, &sh.full[stg], w, lp, io, Tr, tile + kPipeStages, has_gen, has_range, so,
+                                      noise, reg_st + stg * kPipeF);
     if (++stg == kPipeStages) {
       stg = 0;
       parity ^= 1u;
@@ -402,6 +417,25 @@ __global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc 
   }
 }
 
+template <bool kQuar, bool kDiag, bool kNext, bool kBatch, bool kLabel>
+__global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward(gj_world_desc w, gj_step_params p, LeanPlan lp,
+                                                                 gj_fwd_io io, const float* __restrict__ cell_buf,
+                                                                 double* __restrict__ red_part,
+                                                                 unsigned int* __restrict__ ticket, NextStep nx,
+                                                                 Batch bt) {
+  pipe_forward_body<kQuar, kDiag, kNext, kBatch, kLabel, false>(w, p, lp, io, cell_buf, red_part, ticket, nx, bt);
+}
+
+// the same with the regional transmission factor (gj_fwd_io.region); dynamic shared memory + kPipeRegionBytes
+template <bool kQuar, bool kDiag, bool kBatch, bool kLabel>
+__global__ void __launch_bounds__(kPipeThreads, 2) k_pipe_forward_region(gj_world_desc w, gj_step_params p, LeanPlan lp,
+                                                                        gj_fwd_io io, const float* __restrict__ cell_buf,
+                                                                        double* __restrict__ red_part,
+                                                                        unsigned int* __restrict__ ticket, NextStep nx,
+                                                                        Batch bt) {
+  pipe_forward_body<kQuar, kDiag, false, kBatch, kLabel, true>(w, p, lp, io, cell_buf, red_part, ticket, nx, bt);
+}
+
 // =====================================================================================================
 // B1p  backward, per agent
 // =====================================================================================================
@@ -421,12 +455,15 @@ struct BwdCot {
   const float* p[6];
 };
 
+template <bool kRegion = false>
 __device__ __forceinline__ void pipe_bwd_issue(PipeBwdStage& sg, uint64_t* bar, const gj_world_desc& w,
-                                               const gj_bwd_io& io, int64_t tile, uint32_t so = 0u) {
+                                               const gj_bwd_io& io, int64_t tile, uint32_t so = 0u,
+                                               int32_t* reg = nullptr) {
   const TileSpan t = tile_span(w, tile);
-  const uint32_t total = 7u * t.n4 + (t.hi16 - t.lo16);
+  const uint32_t total = (kRegion ? 8u : 7u) * t.n4 + (t.hi16 - t.lo16);
   mbar_expect_tx(bar, total);
   const Copier c{bar};
+  if (kRegion) c.f4(reg, io.region, t);
   c.f4(sg.s, io.s + so, t);
   c.f4(sg.tinf, io.tinf + so, t);
   c.f4(sg.cur, io.cur + so, t);
@@ -443,20 +480,23 @@ __device__ __forceinline__ void pipe_bwd_issue(PipeBwdStage& sg, uint64_t* bar, 
 constexpr int kBwdThreads = GJ_PIPE_BWD_THREADS;
 constexpr int kBwdPer = kPipeTile / kBwdThreads;
 constexpr int kBwdCtas = kBwdThreads == 256 ? 3 : 2;
-template <bool kQuar, bool kBatch, bool kLabel>
-__global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
-                                                                  gj_bwd_io io, float* __restrict__ tile_part,
-                                                                  Batch bt) {
+// kRegion: regional transmission factor; the region codes are staged like in the forward (after PipeBwdShared)
+template <bool kQuar, bool kBatch, bool kLabel, bool kRegion>
+__device__ __forceinline__ void pipe_backward_body(const gj_world_desc& w, const gj_step_params& p, const LeanPlan& lp,
+                                                   const gj_bwd_io& io, float* __restrict__ tile_part, const Batch& bt) {
   extern __shared__ __align__(128) unsigned char pipe_smem[];
   PipeBwdShared& sh = *reinterpret_cast<PipeBwdShared*>(pipe_smem);
+  int32_t* const reg_st = reinterpret_cast<int32_t*>(pipe_smem + sizeof(PipeBwdShared));
   const BatchCta bc = batch_cta<kBatch>(bt);
   const uint32_t so = bc.so;
   const float* __restrict__ g_red = io.g_red;
   const float* __restrict__ g_lab = io.g_red_label;
+  const float* __restrict__ rfac = io.region_factor;
   if (kBatch) {
     tile_part = scr_shift(tile_part, bt, bc.s);
     if (g_red) g_red += (int64_t)bc.s * bt.sRed;
     if (kLabel) g_lab += bc.s * bt.sLab;
+    if (kRegion) rfac += bc.s * bt.sReg;
   }
   const TileRun run = lean_tiles(w, bc);
   const BwdCot cot{{io.g_s_o, io.g_inf_o, io.g_tinf_o, io.g_cur_o, io.g_nxt_o, io.g_ttn_o}};
@@ -477,7 +517,7 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
   __syncthreads();
   if (threadIdx.x == 0) {
     for (int i = 0; i < kPipeStages; ++i)
-      if (run.t0 + i < run.t1) pipe_bwd_issue(sh.st[i], &sh.full[i], w, io, run.t0 + i, so);
+      if (run.t0 + i < run.t1) pipe_bwd_issue<kRegion>(sh.st[i], &sh.full[i], w, io, run.t0 + i, so, reg_st + i * kPipeF);
   }
   const float dead = (float)(p.n_stages - 1);
   const float g_deaths = g_red ? g_red[1] / dead : 0.0f;
@@ -516,13 +556,14 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
       if (a >= a1) break;
       const float glab_i = kLabel ? g_lab[2 * (int64_t)lab[h]] : 0.0f;
       const float glab_d = kLabel ? g_lab[2 * (int64_t)lab[h] + 1] / dead : 0.0f;
-      lean_backward_agent<kQuar, kLabel>(p, lp, io, a, sg.s[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i], sg.ty[i],
-                                         sg.v[i], sg.cls[j + sk16], c[h][0], c[h][1], c[h][2], c[h][3], c[h][4], c[h][5],
-                                         inv_tau, dead, g_deaths, sh.gred_age, sh.prob, acc, w.orig_id, so, glab_i,
-                                         glab_d);
+      const float mreg = kRegion ? __ldg(rfac + reg_st[stg * kPipeF + i]) : 1.0f;
+      lean_backward_agent<kQuar, kLabel, kRegion>(p, lp, io, a, sg.s[i], sg.tinf[i], sg.cur[i], sg.nxt[i], sg.ttn[i],
+                                                  sg.ty[i], sg.v[i], sg.cls[j + sk16], c[h][0], c[h][1], c[h][2], c[h][3],
+                                                  c[h][4], c[h][5], inv_tau, dead, g_deaths, sh.gred_age, sh.prob, acc,
+                                                  w.orig_id, so, glab_i, glab_d, mreg);
     }
     if (pipe_release() && tile + kPipeStages < run.t1)
-      pipe_bwd_issue(sg, &sh.full[stg], w, io, tile + kPipeStages, so);
+      pipe_bwd_issue<kRegion>(sg, &sh.full[stg], w, io, tile + kPipeStages, so, reg_st + stg * kPipeF);
     const bool ends_cell = lp.n_cell > 0 && (tile + 1 == run.t1 || (sh.next_flag[stg] & 1u));   // after the barrier
     if (++stg == kPipeStages) {
       stg = 0;
@@ -538,6 +579,21 @@ __global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_worl
       }
     }
   }
+}
+
+template <bool kQuar, bool kBatch, bool kLabel>
+__global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward(gj_world_desc w, gj_step_params p, LeanPlan lp,
+                                                                  gj_bwd_io io, float* __restrict__ tile_part,
+                                                                  Batch bt) {
+  pipe_backward_body<kQuar, kBatch, kLabel, false>(w, p, lp, io, tile_part, bt);
+}
+
+// the same with the regional transmission factor (gj_bwd_io.region); dynamic shared memory + kPipeRegionBytes
+template <bool kQuar, bool kBatch, bool kLabel>
+__global__ void __launch_bounds__(kBwdThreads, kBwdCtas) k_pipe_backward_region(gj_world_desc w, gj_step_params p,
+                                                                         LeanPlan lp, gj_bwd_io io,
+                                                                         float* __restrict__ tile_part, Batch bt) {
+  pipe_backward_body<kQuar, kBatch, kLabel, true>(w, p, lp, io, tile_part, bt);
 }
 
 // =====================================================================================================

@@ -44,6 +44,7 @@ struct Batch {
   int sBeta, sRed; // strides of beta / g_beta and red / g_red (elements)
   const float* noise;  // [n_agents] the draw's Gumbel noise difference, evaluated once for all samples; NULL = in-kernel
   int64_t sLab;        // stride of red_label / g_red_label / label_acc (elements)
+  int64_t sReg;        // stride of region_factor / g_region_factor (elements, >= n_regions: a row per sample)
 };
 struct BatchCta {
   int s;           // sample of this CTA
@@ -433,11 +434,12 @@ __device__ __forceinline__ Pressure agent_pressure(const gj_world_desc& w, const
   return out;
 }
 
-template <bool kLabel>
-__global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_step_params p, Plan pl, gj_fwd_io io,
-                                                            const float* __restrict__ cell_buf,
-                                                            double* __restrict__ red_part,
-                                                            unsigned int* __restrict__ ticket) {
+// kRegion: the pressure is multiplied by the agent's regional factor before the clamp (gj_fwd_io.region); the tape
+// keeps the pre-factor value, the diagnostic lam is the product
+template <bool kLabel, bool kRegion>
+__device__ __forceinline__ void tile_forward_body(const gj_world_desc& w, const gj_step_params& p, const Plan& pl,
+                                                  const gj_fwd_io& io, const float* __restrict__ cell_buf,
+                                                  double* __restrict__ red_part, unsigned int* __restrict__ ticket) {
   __shared__ TileTables tb;
   const int64_t N = w.n_agents;
   const int64_t tile = blockIdx.x;
@@ -462,10 +464,11 @@ __global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
     const float mq = (p.n_quar > 0) ? quarantine_mask(p, st.cur) : 1.0f;
     const Pressure pr = agent_pressure(w, p, pl, tb, io.S_scaled, Tsrc, Tq, a, cls, st.s, mq);
-    const float q = not_infected_prob(pr.lam, p.dt);
+    const float lam = kRegion ? pr.lam * __ldg(io.region_factor + io.region[a]) : pr.lam;
+    const float q = not_infected_prob(lam, p.dt);
     io.tape_v[a] = (st.s == 0.0f) ? pr.X : pr.lam;
     if (io.q) io.q[a] = q;
-    if (io.lam) io.lam[a] = pr.lam;
+    if (io.lam) io.lam[a] = lam;
     forward_tail<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, q, st, red, io.label_acc);
   }
   if (io.red) {
@@ -475,6 +478,23 @@ __global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_
     block_sums<double, kMaxRed>(redd, 2 + p.n_age_bins, red_part + tile * kMaxRed);
     finish_partials<kMaxRed>(2 + p.n_age_bins, red_part, gridDim.x, ticket, io.red);
   }
+}
+
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock, 4) k_tile_forward(gj_world_desc w, gj_step_params p, Plan pl, gj_fwd_io io,
+                                                            const float* __restrict__ cell_buf,
+                                                            double* __restrict__ red_part,
+                                                            unsigned int* __restrict__ ticket) {
+  tile_forward_body<kLabel, false>(w, p, pl, io, cell_buf, red_part, ticket);
+}
+
+// the same with the regional transmission factor (gj_fwd_io.region)
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock, 4) k_tile_forward_region(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                   gj_fwd_io io, const float* __restrict__ cell_buf,
+                                                                   double* __restrict__ red_part,
+                                                                   unsigned int* __restrict__ ticket) {
+  tile_forward_body<kLabel, true>(w, p, pl, io, cell_buf, red_part, ticket);
 }
 
 // =====================================================================================================
@@ -489,7 +509,9 @@ struct BackAgent {
 // symptoms^T, infect^T, sampler^T and the clamp/exp chain: shared by the generic and the tiled kernels
 // kLabel: fold in the cotangent of the forward's label table (gj_bwd_io.g_red_label) at the agent's label
 // kSeed: seeding by label, the agent's fraction is seed_fraction[seed_label[a]]
-template <bool kLabel = false, bool kSeed = false>
+// kRegion: regional transmission factor m (gj_bwd_io.region): glam (with g_lam, the cotangent of lam' = lam * m) times
+// lam goes to io.region_work, and r.glam = glam * m is what the chain below sees
+template <bool kLabel = false, bool kSeed = false, bool kRegion = false>
 __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, const gj_bwd_io& io, int64_t N, int64_t a,
                                                     int64_t ga, int age, const AgentState& st, bool with_networks) {
   const int dead = p.n_stages - 1;
@@ -571,10 +593,12 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
     r.gtinf = gtinf_o * (1.0f - n);
   }
   r.gq = io.g_q ? io.g_q[a] : 0.0f;
-  float lam = 0.0f, q = 1.0f, v = 0.0f;
+  float lam = 0.0f, q = 1.0f, v = 0.0f, lam0 = 0.0f, mreg = 1.0f;
   if (with_networks) {
     v = io.tape_v[a];
-    lam = (st.s == 0.0f) ? 0.0f : v;
+    lam0 = (st.s == 0.0f) ? 0.0f : v;
+    if (kRegion) mreg = __ldg(io.region_factor + io.region[a]);
+    lam = kRegion ? lam0 * mreg : lam0;
     q = not_infected_prob(lam, p.dt);
   }
   if (seed_mode) q = 1.0f - io.seed_fraction[kSeed ? io.seed_label[a] : 0] * 1.0f;
@@ -597,15 +621,19 @@ __device__ __forceinline__ BackAgent backward_agent(const gj_step_params& p, con
       if (lam >= 1e-6f && lam <= 100.0f) r.glam = glc;
     }
     if (io.g_lam) r.glam += io.g_lam[a];
+    if (kRegion) {
+      io.region_work[a] = r.glam * lam0;
+      r.glam = r.glam * mreg;
+    }
     const float X = (st.s == 0.0f) ? v : v / st.s;
     r.gs += r.glam * X;
   }
   return r;
 }
 
-template <bool kLabel>
-__global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj_step_params p, Plan pl, gj_bwd_io io,
-                                                          float* __restrict__ tile_part) {
+template <bool kLabel, bool kRegion>
+__device__ __forceinline__ void tile_backward_body(const gj_world_desc& w, const gj_step_params& p, const Plan& pl,
+                                                   const gj_bwd_io& io, float* __restrict__ tile_part) {
   __shared__ TileTables tb;
   const int64_t N = w.n_agents;
   const int64_t tile = blockIdx.x;
@@ -624,7 +652,7 @@ __global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj
     st.cur = io.cur ? io.cur[a] : 1.0f;
     st.nxt = io.nxt ? io.nxt[a] : 1.0f;
     st.ttn = io.ttn ? io.ttn[a] : 0.0f;
-    const BackAgent r = backward_agent<kLabel>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, true);
+    const BackAgent r = backward_agent<kLabel, false, kRegion>(p, io, N, a, noise_agent(w, p, a), cls % 100, st, true);
     const float mq = (p.n_quar > 0) ? quarantine_mask(p, st.cur) : 1.0f;
     const float wv = r.glam * st.s;
     const float wqv = r.glam * (mq * st.s);
@@ -650,6 +678,19 @@ __global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj
     if (io.g_ttn) io.g_ttn[a] = r.gttn;
   }
   if (pl.n_t2 > 0) block_sums<float, GJ_MAX_CHANNELS>(acc, pl.n_t2, tile_part + tile * GJ_MAX_CHANNELS);
+}
+
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock, 3) k_tile_backward(gj_world_desc w, gj_step_params p, Plan pl, gj_bwd_io io,
+                                                          float* __restrict__ tile_part) {
+  tile_backward_body<kLabel, false>(w, p, pl, io, tile_part);
+}
+
+// the same with the regional transmission factor (gj_bwd_io.region)
+template <bool kLabel>
+__global__ void __launch_bounds__(kBlock, 3) k_tile_backward_region(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                    gj_bwd_io io, float* __restrict__ tile_part) {
+  tile_backward_body<kLabel, true>(w, p, pl, io, tile_part);
 }
 
 // =====================================================================================================

@@ -18,7 +18,7 @@ GJ_MAX_STAGES = 16
 GJ_MAX_QUAR = 4
 GJ_MAX_AGE_BINS = 8
 GJ_MAX_CHANNELS = 8
-GJ_ABI_VERSION = 12
+GJ_ABI_VERSION = 13
 
 KIND_PLAIN, KIND_HOUSEHOLD, KIND_LEISURE, KIND_CARE_VISIT = 0, 1, 2, 3
 PHASE_NETWORKS, PHASE_SAMPLE, PHASE_INFECT, PHASE_SYMPTOMS, PHASE_ALL = 1, 2, 4, 8, 15
@@ -108,20 +108,26 @@ class FwdIO(C.Structure):
         ("label", C.c_void_p), ("n_labels", C.c_int32), ("_pad_label", C.c_int32), ("red_label", C.c_void_p),
         ("label_acc", C.c_void_p),
         # seeding by label: region codes and their count
-        ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32)]
+        ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32),
+        # regional transmission factor: region codes, their count, the factor per region
+        ("region", C.c_void_p), ("n_regions", C.c_int32), ("_pad_region", C.c_int32), ("region_factor", C.c_void_p)]
 
 
 class BwdIO(C.Structure):
     _fields_ = [(name, C.c_void_p) for name in _BWD_FIELDS] + [("label", C.c_void_p), ("g_red_label", C.c_void_p)] + [
         ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32), ("seed_order", C.c_void_p),
-        ("seed_offsets", C.c_void_p), ("seed_work", C.c_void_p)]
+        ("seed_offsets", C.c_void_p), ("seed_work", C.c_void_p)] + [
+        ("region", C.c_void_p), ("n_regions", C.c_int32), ("_pad_region", C.c_int32), ("region_factor", C.c_void_p),
+        ("region_order", C.c_void_p), ("region_offsets", C.c_void_p), ("region_work", C.c_void_p),
+        ("g_region_factor", C.c_void_p)]
 
 
 class Batch(C.Structure):
     """gj_batch: strides of a batched ensemble call (gj_step_forward_batch / gj_step_backward_batch)."""
     _fields_ = [("n_samples", C.c_int32), ("_pad0", C.c_int32), ("agent_stride", C.c_int64),
                 ("group_stride", C.c_int64), ("beta_stride", C.c_int64), ("red_stride", C.c_int64),
-                ("scratch_stride", C.c_int64), ("noise", C.c_void_p), ("label_stride", C.c_int64)]
+                ("scratch_stride", C.c_int64), ("noise", C.c_void_p), ("label_stride", C.c_int64),
+                ("region_stride", C.c_int64)]
 
 
 class GradJuneLibraryError(RuntimeError):

@@ -13,6 +13,11 @@ the NCCL all-reduces of a partitioned world — is capturable with ``torch.cuda.
 vector — one value for a national seed, one per region of ``runner.seed_labels`` with ``seed_by`` — so a replay takes
 [K + R] values ([b, K + R] batched) and returns their gradient.
 
+``fit_regional=True`` calibrates the regional policies too: the log10 of every ``RegionalSocialDistancing`` policy's
+factors, R values per policy (``runner.region_labels`` order) in the order the policies were given, follow the
+log-betas and the seeding values; a factor of 0 has no log10 and is rejected.  Regional factors that are not fitted
+are constants of the graph, used through a device copy made at construction; the policies themselves are not changed.
+
 Noise: the Philox key and call indices are kernel arguments, so every replay draws the SAME noise (common random
 numbers across parameter samples — the usual variance reduction for calibration gradients); ``recapture(seed)``
 re-records the graph with another key.
@@ -35,9 +40,11 @@ from . import ops
 
 class GraphedRunner:
     def __init__(self, runner, loss_fn: Callable[[dict], torch.Tensor], networks: Optional[Sequence[str]] = None,
-                 seed: int = 0, warmup: int = 1, batch: Optional[int] = None, fit_seed: bool = False):
+                 seed: int = 0, warmup: int = 1, batch: Optional[int] = None, fit_seed: bool = False,
+                 fit_regional: bool = False):
         self.runner = runner
         self.fit_seed = bool(fit_seed)
+        self.fit_regional = bool(fit_regional)
         self.loss_fn = loss_fn
         self.batch = int(batch) if batch else None
         runner.batch = self.batch
@@ -59,6 +66,26 @@ class GraphedRunner:
                 R = len(runner.seed_labels)
                 self.seed_names = [str(v) for v in runner.seed_labels]
                 init += [float(v) for v in np.broadcast_to(lf.reshape(-1)[:R] if lf.size >= R else lf, (R,))]
+        self.n_seed = len(init) - self.n_beta
+        rp = getattr(runner.model.policies, "regional_policies", None)
+        self.regional = list(rp.policies) if (rp is not None and runner.region_by is not None) else []
+        self.regional_names = []
+        if self.fit_regional:   # log10 of each regional policy's factors, R per policy, after the seeding values
+            if not self.regional:
+                raise ValueError("fit_regional=True needs at least one regional policy")
+            for i, pol in enumerate(self.regional):
+                f = pol.factors(runner.region_labels, "cpu").detach().reshape(-1, len(runner.region_labels))[0]
+                if not bool((f > 0).all()):
+                    zero = runner.region_labels[int(torch.nonzero(f <= 0)[0])]
+                    raise ValueError(f"fit_regional=True fits log10 of the factors: regional policy {i} has factor "
+                                     f"{float(f[f <= 0][0])} for region {zero!r}; start the fit from a factor > 0")
+                init += [float(v) for v in torch.log10(f.double())]
+                self.regional_names += [f"{i}_{v}" for v in runner.region_labels]
+        # factors that are not fitted are constants of the graph: a tensor is used through a detached copy on the device
+        # (a host-to-device copy cannot be captured).  The policies themselves are left as the caller built them: each
+        # iteration swaps the values in and restores the originals afterwards.
+        self._fixed_factors = [pol.beta_factors.detach().to(device=self.device, dtype=torch.float32)
+                               if torch.is_tensor(pol.beta_factors) else None for pol in self.regional]
         self.log_beta = torch.tensor(init, dtype=torch.float32).to(self.device)
         if self.batch:
             self.log_beta = self.log_beta.repeat(self.batch, 1)          # [b, K]
@@ -87,9 +114,28 @@ class GraphedRunner:
             if self.runner.seed_by is None:
                 self.runner.log_fraction_initial_cases = self.log_beta[:, K] if self.batch else self.log_beta[K]
             else:
-                self.runner.log_fraction_initial_cases = self.log_beta[:, K:] if self.batch else self.log_beta[K:]
-        with ops.philox_seed(self.seed):
-            results, is_infected = self.runner()
+                self.runner.log_fraction_initial_cases = (self.log_beta[:, K:K + self.n_seed] if self.batch
+                                                          else self.log_beta[K:K + self.n_seed])
+        originals = [pol.beta_factors for pol in self.regional]
+        R = len(self.runner.region_labels) if self.regional else 0
+        off = self.n_beta + self.n_seed
+        for i, pol in enumerate(self.regional):
+            if self.fit_regional:
+                value = 10.0 ** (self.log_beta[:, off + i * R:off + (i + 1) * R] if self.batch
+                                 else self.log_beta[off + i * R:off + (i + 1) * R])
+            elif self._fixed_factors[i] is not None:
+                value = self._fixed_factors[i]
+            else:
+                continue
+            pol._parameters.pop("beta_factors", None)   # an nn.Parameter is unregistered first, like log_beta
+            pol.beta_factors = value
+        try:
+            with ops.philox_seed(self.seed):
+                results, is_infected = self.runner()
+        finally:
+            for pol, value in zip(self.regional, originals):
+                pol._parameters.pop("beta_factors", None)
+                pol.beta_factors = value
         loss = self.loss_fn(results)
         if self.batch and tuple(loss.shape) != (self.batch,):
             raise ValueError(f"batched window: loss_fn must return one loss per sample, shape ({self.batch},); "
@@ -99,7 +145,8 @@ class GraphedRunner:
         if part is not None and part.world_size > 1:
             # geographic partition: every rank holds the d/dbeta terms of the groups it owns; the sum over ranks
             # is part of the captured iteration (one more NCCL kernel in the graph, no eager collective per replay);
-            # with fit_seed the seeding gradients (each rank's own agents) are summed in the same all-reduce
+            # with fit_seed / fit_regional the seeding and regional gradients (each rank's own agents) are summed in the
+            # same all-reduce
             import torch.distributed as dist
             dist.all_reduce(self.log_beta.grad, group=part.process_group)
         return loss.detach(), results, is_infected
@@ -134,7 +181,8 @@ class GraphedRunner:
     @torch.no_grad()
     def __call__(self, log_beta: Optional[torch.Tensor] = None):
         """Replay with ``log_beta`` ([K], or [b, K] for a batched window; [K + R] / [b, K + R] with ``fit_seed``, the
-        log-fractions last; any device; None = keep).  Returns (loss, d loss / d log_beta, results): static device
+        log-fractions after the log-betas; then, with ``fit_regional``, R log10-factors per regional policy; any device;
+        None = keep).  Returns (loss, d loss / d log_beta, results): static device
         tensors that the next replay overwrites."""
         if log_beta is not None:
             self.log_beta.copy_(log_beta.to(dtype=torch.float32), non_blocking=True)

@@ -178,7 +178,7 @@ def beta_vector(networks, policies, timer, device):
                         for net in networks])
 
 
-def _run_networks(networks, data, timer, policies, device, want_lam=False):
+def _run_networks(networks, data, timer, policies, device, want_lam=False, region=None):
     agent = data["agent"]
     ops.require_cuda(agent.susceptibility, "data['agent'].susceptibility")
     dev = agent.susceptibility.device
@@ -196,7 +196,7 @@ def _run_networks(networks, data, timer, policies, device, want_lam=False):
 
     static = ops.StepStatic(world=world, leisure_prob=table, exchange=exchange_for(data, world))
     return ops.infection_step(static, spec, beta_vector(networks, policies, timer, dev), state,
-                              T_in=agent.transmission)
+                              T_in=agent.transmission, region=region)
 
 
 class InfectionNetworks(torch.nn.Module):
@@ -235,16 +235,20 @@ class InfectionNetworks(torch.nn.Module):
     def has_custom(self, nets=None):
         return any(net.is_custom() for net in (self.networks.values() if nets is None else nets))
 
-    def forward(self, data, timer, policies):
+    def forward(self, data, timer, policies, region=None):
+        """not_infected_probs of the step.  ``region`` (:class:`grad_june.ops.Region`): every agent's summed pressure is
+        multiplied by its region's factor before the clamp (the regional policies active at this step)."""
         policies.apply(timer=timer, data=data)
         nets = self.active_networks(timer, policies)
         if not self.has_custom(nets):
-            return _run_networks(nets, data, timer, policies, self.device)["q"]
+            return _run_networks(nets, data, timer, policies, self.device, region=region)["q"]
         # a user-defined network among them: network by network in the activity order, then the reference's clamp /
         # exp chain (base.py:133-140) in torch
         agent = data["agent"]
         lam = torch.zeros_like(agent.susceptibility)
         for net in nets:
             lam = lam + net(data=data, timer=timer, policies=policies)
+        if region is not None:
+            lam = lam * region.factor.to(lam.device)[region.labels.codes.long()]
         lam = torch.clamp(lam, min=1e-6, max=100)
         return torch.clamp(torch.exp(-lam * timer.duration), min=0.0, max=1.0)

@@ -234,6 +234,40 @@ def _set_seed_labels(io, world: DeviceWorld, seed_label: SeedLabels, seed_fracti
         io.seed_work = _buffer(world, "seed_work", world.n_agents).data_ptr()
 
 
+@dataclass(frozen=True)
+class Region:
+    """Regional transmission factor of one step: every agent's summed pressure is multiplied by
+    ``factor[labels.codes[a]]`` before the clamp.  ``labels`` (:class:`SeedLabels`) holds the per-agent region codes
+    and the order / offsets of the backward's deterministic per-region reduction; ``factor`` is [n] ([n] or [b, n]
+    batched), differentiable."""
+    labels: SeedLabels
+    factor: torch.Tensor
+
+
+def _set_region(io, world: DeviceWorld, labels: SeedLabels, factor):
+    """Point the io struct at the region codes and the factors (and, on the backward's struct, at the reduction's order,
+    offsets and the per-agent workspace of ``nb`` rows)."""
+    if labels.codes.numel() != world.n_agents or labels.codes.device != world.device:
+        raise ValueError(f"region codes must hold one entry per agent ({world.n_agents}) on {world.device}")
+    io.region, io.n_regions, io.region_factor = labels.codes.data_ptr(), labels.n, factor.data_ptr()
+    if hasattr(io, "region_order"):
+        io.region_order, io.region_offsets = labels.order.data_ptr(), labels.offsets.data_ptr()
+
+
+def _region_factor(region: Region, dev, nb: int = 0):
+    """The factors as a contiguous fp32 tensor on ``dev``: [n], or [nb, n] for a batch of ``nb`` samples."""
+    f = _f32(region.factor, dev)
+    n = region.labels.n
+    if nb:
+        if tuple(f.shape) not in ((n,), (nb, n)):
+            raise ValueError(f"a regional factor must hold {n} values (one per region) or {nb} x {n}, got "
+                             f"{tuple(f.shape)}")
+        return f.expand(nb, n).contiguous()
+    if tuple(f.shape) != (n,):
+        raise ValueError(f"a regional factor must hold {n} values (one per region), got {tuple(f.shape)}")
+    return f.contiguous()
+
+
 def _label_acc(world: DeviceWorld, n: int):
     """The integer accumulator of the label table ([n] uint32, zero; every call leaves it zero)."""
     t = world.__dict__.get("_label_acc")
@@ -486,7 +520,8 @@ class _Step(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in,
-                seed_fraction, next_spec=None, label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None):
+                seed_fraction, next_spec=None, label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None,
+                region_labels: Optional[SeedLabels] = None, region_factor=None):
         world = static.world
         dev = world.device
         N = world.n_agents
@@ -509,6 +544,13 @@ class _Step(torch.autograd.Function):
         phases, seed_mode = spec.phases, spec.mode == MODE_SEED
         nets_on = bool(phases & PHASE_NETWORKS) and not seed_mode
         beta = put("beta", beta) if nets_on else None
+        region_labels = region_labels if nets_on else None
+        if region_labels is not None:
+            region_factor = _region_factor(Region(region_labels, region_factor), dev)
+            keep.append(region_factor)
+            _set_region(io, world, region_labels, region_factor)
+        else:
+            region_factor = None
         put("leisure_prob", static.leisure_prob)
         if static.symptoms is not None:
             put("stage_prob", static.symptoms.stage_prob)
@@ -587,7 +629,8 @@ class _Step(torch.autograd.Function):
             p.agent_offset = static.exchange.part.agent_lo
         lean_inputs = E is None and u is None and z is None and T_in is None and lam is None and static.prof4 is not None
         p_next = T_next = Tq_next = None
-        if next_spec is not None and fused_all and lean_inputs and not seed_mode and label is None:
+        if (next_spec is not None and fused_all and lean_inputs and not seed_mode and label is None
+                and region_labels is None):
             # also run the NEXT step's transmission pass inside this step's agent kernel (gj_step_forward_next)
             p_next, _ = _fill_params(world, next_spec, static.symptoms, 0, 0)
             T_next = torch.empty(N, dtype=torch.float32, device=dev)
@@ -606,11 +649,11 @@ class _Step(torch.autograd.Function):
                 cur=out.get("cur_o"))
 
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
-        ctx.seed_label = seed_label
+        ctx.seed_label, ctx.region_labels = seed_label, region_labels
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"],
                               T_in if T_in is not None else T, q_in, n_in,
-                              seed_fraction, out.get("inf_o"), tape_v, tape_y0, S_un, E, u, z, q, n)
+                              seed_fraction, out.get("inf_o"), tape_v, tape_y0, S_un, E, u, z, q, n, region_factor)
         ctx.fused_T = fused_T
         outs = (out.get("s_o"), out.get("inf_o"), out.get("tinf_o"), out.get("cur_o"), out.get("nxt_o"),
                 out.get("ttn_o"), T, q, n, red, lam, red_label)
@@ -628,7 +671,7 @@ class _Step(torch.autograd.Function):
         world = static.world
         dev, N = world.device, world.n_agents
         (beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, seed_fraction, inf_o, tape_v, tape_y0, S_un, E, u, z,
-         q_saved, n_saved) = ctx.saved_tensors
+         q_saved, n_saved, region_factor) = ctx.saved_tensors
         seed, call_index = ctx.noise_key
         p, s_total = _fill_params(world, spec, static.symptoms, seed, call_index)
         phases, seed_mode = spec.phases, spec.mode == MODE_SEED
@@ -672,7 +715,15 @@ class _Step(torch.autograd.Function):
             put("g_red_label", g_red_label)
             io.label = ctx.label.codes.data_ptr()
 
-        need = ctx.needs_input_grad  # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, frac)
+        need = ctx.needs_input_grad  # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, frac,
+        #                                next_spec, label, seed_label, region_labels, region_factor)
+        g_region = None
+        if ctx.region_labels is not None:   # the per-agent terms always; their per-region sums when wanted
+            _set_region(io, world, ctx.region_labels, region_factor)
+            io.region_work = _buffer(world, "region_work", N).data_ptr()
+            if need[18]:
+                g_region = torch.empty(ctx.region_labels.n, dtype=torch.float32, device=dev)
+                io.g_region_factor = g_region.data_ptr()
 
         def new(name, n=N, zero=False):
             t = (torch.zeros if zero else torch.empty)(n, dtype=torch.float32, device=dev)
@@ -720,7 +771,8 @@ class _Step(torch.autograd.Function):
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None, None)
+                g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None, None, None,
+                g_region)
 
 
 # --------------------------------------------------------------------------------------
@@ -767,7 +819,8 @@ class _BatchStep(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction,
-                label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None):
+                label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None,
+                region_labels: Optional[SeedLabels] = None, region_factor=None):
         world = static.world
         dev, N = world.device, world.n_agents
         L = _lib.lib()
@@ -828,6 +881,14 @@ class _BatchStep(torch.autograd.Function):
         if not seed_mode:
             seed_label = None
         if seed_mode:
+            region_labels = None
+        rf, n_reg = None, 0
+        if region_labels is not None:   # [b, R]: every sample its own row of factors
+            rf = _region_factor(Region(region_labels, region_factor), dev, nb)
+            keep.append(rf)
+            _set_region(io, world, region_labels, rf)
+            n_reg = region_labels.n
+        if seed_mode:
             seed_fraction = put("seed_fraction", seed_fraction)
             R = 1
             if seed_label is not None:   # seeding by label: [R] shared by the samples or [b, R]
@@ -856,16 +917,17 @@ class _BatchStep(torch.autograd.Function):
             # the samples share the Philox stream: the draw's Gumbel noise is evaluated once per agent
             noise_buf = _buffer(world, "noise_b", Np) if BATCH_SHARED_NOISE else None
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride, noise=_ptr(noise_buf), label_stride=n_lab)
+                            scratch_stride=scr_stride, noise=_ptr(noise_buf), label_stride=n_lab, region_stride=n_reg)
             with _on(dev):
                 _lib.check(L.gj_step_forward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_forward_batch")
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
-        ctx.seed_label = seed_label
+        ctx.seed_label, ctx.region_labels = seed_label, region_labels
+        ctx.region_shape = tuple(region_factor.shape) if region_labels is not None else None
         ctx.shape = (nb, Np, sG, K, nr)
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"], T, seed_fraction,
-                              out["inf_o"], tape_v, tape_y0, S_un)
+                              out["inf_o"], tape_v, tape_y0, S_un, rf)
         if T is not None:
             ctx.mark_non_differentiable(T)
         return (out["s_o"], out["inf_o"], out["tinf_o"], out["cur_o"], out["nxt_o"], out["ttn_o"], T, red, red_label)
@@ -876,7 +938,7 @@ class _BatchStep(torch.autograd.Function):
         world = static.world
         dev = world.device
         nb, Np, sG, K, nr = ctx.shape
-        beta, s, inf, tinf, cur, nxt, ttn, T, seed_fraction, inf_o, tape_v, tape_y0, S_un = ctx.saved_tensors
+        beta, s, inf, tinf, cur, nxt, ttn, T, seed_fraction, inf_o, tape_v, tape_y0, S_un, rf = ctx.saved_tensors
         seed, call_index = ctx.noise_key
         p, _ = _fill_params(world, spec, static.symptoms, seed, call_index)
         seed_mode = spec.mode == MODE_SEED
@@ -906,7 +968,16 @@ class _BatchStep(torch.autograd.Function):
             put("g_red_label", g_red_label)
             io.label = ctx.label.codes.data_ptr()
             n_lab = 2 * ctx.label.n
-        need = ctx.needs_input_grad   # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction)
+        need = ctx.needs_input_grad   # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction, label,
+        #                                 seed_label, region_labels, region_factor)
+        g_region, n_reg = None, 0
+        if ctx.region_labels is not None:
+            n_reg = ctx.region_labels.n
+            _set_region(io, world, ctx.region_labels, rf)
+            io.region_work = _buffer(world, "region_work_b", nb * Np).data_ptr()
+            if need[14]:
+                g_region = torch.empty(nb, n_reg, dtype=torch.float32, device=dev)
+                io.g_region_factor = g_region.data_ptr()
 
         def new(name):
             t = torch.empty(nb, Np, dtype=torch.float32, device=dev)
@@ -948,26 +1019,30 @@ class _BatchStep(torch.autograd.Function):
             io.wq = _buffer(world, "wq_b", nb * Np).data_ptr() if p.n_quar > 0 else io.w
             io.R, io.cR = _buffer(world, "R_b", nb * sG).data_ptr(), _buffer(world, "cR_b", nb * sG).data_ptr()
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride, label_stride=n_lab)
+                            scratch_stride=scr_stride, label_stride=n_lab, region_stride=n_reg)
             with _on(dev):
                 _lib.check(L.gj_step_backward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_backward_batch")
             g_beta = g_beta[:, :K]
+            if g_region is not None and ctx.region_shape != (nb, n_reg):
+                g_region = g_region.sum(0)   # one row of factors shared by the samples
         return (None, None, None, g_beta if need[3] else None,
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_frac if (seed_mode and need[10]) else None, None, None)
+                g_frac if (seed_mode and need[10]) else None, None, None, None, g_region)
 
 
 def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=None, q_in=None, n_in=None,
                    seed_fraction=None, noise=None, next_spec=None, label: Optional[Labels] = None,
-                   seed_label: Optional[SeedLabels] = None):
+                   seed_label: Optional[SeedLabels] = None, region: Optional[Region] = None):
     """Run one (fused or partial) step.  ``state``: s, inf, tinf, cur, nxt, ttn (any may be None when
     the phases do not need it).  Returns a dict with s, inf, tinf, cur, nxt, ttn, T, q, n, red and red_label:
     with ``label`` the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched), else None.
     ``seed_label`` (seeding step only): ``seed_fraction`` then holds one fraction per region ([n], or [b, n]
-    batched) and agent a is seeded with ``seed_fraction[seed_label.codes[a]]``."""
+    batched) and agent a is seeded with ``seed_fraction[seed_label.codes[a]]``.
+    ``region`` (:class:`Region`, steps with the networks phase): every agent's pressure is multiplied by its region's
+    factor before the clamp; the factor is differentiable.  The seeding step ignores it."""
     world = static.world
     if world.device.type != "cuda":
         raise _lib.GradJuneLibraryError(
@@ -982,13 +1057,15 @@ def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=N
         if T_in is not None or q_in is not None or n_in is not None or static.exchange is not None:
             raise _lib.GradJuneLibraryError("batched ensembles run the whole fused step on an unpartitioned world")
         outs = _BatchStep.apply(static, spec, noise, beta, state["s"], state["inf"], state["tinf"], state["cur"],
-                                state["nxt"], state["ttn"], seed_fraction, label, seed_label)
+                                state["nxt"], state["ttn"], seed_fraction, label, seed_label,
+                                None if region is None else region.labels, None if region is None else region.factor)
         names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "red", "red_label")
         ret = dict(zip(names, outs))
         ret.update(q=None, n=None, lam=None)
         return ret
     outs = _Step.apply(static, spec, noise, beta, state.get("s"), state.get("inf"), state.get("tinf"),
                        state.get("cur"), state.get("nxt"), state.get("ttn"), T_in, q_in, n_in, seed_fraction, next_spec,
-                       label, seed_label)
+                       label, seed_label, None if region is None else region.labels,
+                       None if region is None else region.factor)
     names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "q", "n", "red", "lam", "red_label")
     return dict(zip(names, outs))

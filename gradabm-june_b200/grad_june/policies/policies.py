@@ -44,21 +44,26 @@ def _camel(name):
 
 
 class Policies(torch.nn.Module):
-    def __init__(self, interaction_policies=None, quarantine_policies=None, close_venue_policies=None):
+    def __init__(self, interaction_policies=None, quarantine_policies=None, close_venue_policies=None,
+                 regional_policies=None):
         super().__init__()
         self.interaction_policies = interaction_policies
         self.quarantine_policies = quarantine_policies
         self.close_venue_policies = close_venue_policies
+        self.regional_policies = regional_policies
+        if regional_policies is not None:
+            regional_policies.by()   # one region attribute per run
 
     @classmethod
     def from_policy_list(cls, policies):
-        from . import CloseVenuePolicies, InteractionPolicies, QuarantinePolicies
+        from . import CloseVenuePolicies, InteractionPolicies, QuarantinePolicies, RegionalPolicies
 
         policies = [] if policies is None else policies
         return cls(
             interaction_policies=InteractionPolicies(cls._get_policies_by_type(policies, "interaction")),
             quarantine_policies=QuarantinePolicies(cls._get_policies_by_type(policies, "quarantine")),
             close_venue_policies=CloseVenuePolicies(cls._get_policies_by_type(policies, "close_venue")),
+            regional_policies=RegionalPolicies(cls._get_policies_by_type(policies, "regional")),
         )
 
     @classmethod

@@ -46,29 +46,30 @@ def label_codes(labels, columns):
     return codes
 
 
-def seed_log_fractions(mapping, labels):
+def seed_log_fractions(mapping, labels, what="seeding", value="log-fraction"):
     """A per-region log-fraction mapping ``{label: value, ..., "default": value}`` (the YAML form) as a list in the
     order of the sorted ``labels``.  Labels the mapping does not list take ``default``; a label in the mapping that no
-    agent carries raises, and so does a missing ``default`` when some label is not listed."""
+    agent carries raises, and so does a missing ``default`` when some label is not listed.  ``what`` / ``value`` name
+    the setting and the quantity in the errors (the regional policies parse their factors with the same rules)."""
     mapping = dict(mapping)
     default = mapping.pop("default", None)
     labels = np.asarray(labels)
     out = [None] * len(labels)
-    for key, value in mapping.items():
+    for key, v in mapping.items():
         if labels.dtype.kind in "iu" and not isinstance(key, (int, np.integer)):
             try:
                 key = int(key)
             except (TypeError, ValueError):
-                raise ValueError(f"seeding: label {key!r} is not carried by any agent") from None
+                raise ValueError(f"{what}: label {key!r} is not carried by any agent") from None
         elif labels.dtype.kind in "US" and not isinstance(key, str):
             key = str(key)
         i = int(np.searchsorted(labels, key))
         if i >= len(labels) or labels[i] != key:
-            raise ValueError(f"seeding: label {key!r} is not carried by any agent")
-        out[i] = float(value)
+            raise ValueError(f"{what}: label {key!r} is not carried by any agent")
+        out[i] = float(v)
     missing = [labels[i] for i, v in enumerate(out) if v is None]
     if missing and default is None:
-        raise ValueError(f"seeding: no log-fraction for label {missing[0]!r} and no 'default'")
+        raise ValueError(f"{what}: no {value} for label {missing[0]!r} and no 'default'")
     return [float(default) if v is None else v for v in out]
 
 
@@ -120,6 +121,19 @@ class Runner(torch.nn.Module):
             self._seed_fraction_shape(log_fraction_initial_cases)
         elif isinstance(log_fraction_initial_cases, dict):
             raise ValueError("a per-region log_fraction_initial_cases mapping needs infection_seed.by (seed_by)")
+        # regional policies (RegionalSocialDistancing): one transmission factor per value of data["agent"][by], the
+        # sorted distinct values over every rank of a partitioned world
+        rp = getattr(model.policies, "regional_policies", None)
+        self.region_by = rp.by() if rp is not None else None
+        self.region_labels = None
+        if self.region_by is not None:
+            if self.region_by == results_by:
+                self.region_labels = self.result_labels
+            elif self.region_by == seed_by:
+                self.region_labels = self.seed_labels
+            else:
+                labels = agent_labels(data["agent"][self.region_by], self.n_agents)
+                self.region_labels = label_union(np.unique(labels), data.__dict__.get("_gj_partition"))
         # batched ensemble (SURVEY 8e-2): ``runner.batch = b`` makes ``forward()`` step b independent samples of the
         # epidemic at once — the networks' ``log_beta`` then hold b values each, the state tensors are [b, Np] and
         # every result series is [T+1, b].  All samples draw the same noise (common random numbers).
@@ -279,6 +293,34 @@ class Runner(torch.nn.Module):
             hit = self.__dict__["_seed_codes"] = (values, dev, ops.make_seed_labels(codes, len(self.seed_labels), dev))
         return hit[2]
 
+    def _region_codes(self):
+        """ops.SeedLabels of the regional policies' ``by`` on the device (built once per label array and device; shares
+        the device codes of ``results_by`` / ``seed_by`` when they name the same attribute), or None."""
+        if self.region_by is None:
+            return None
+        if self.region_by == self.seed_by:
+            return self._seed_label_codes()
+        values = self.data["agent"][self.region_by]
+        dev = self.data["agent"].susceptibility.device
+        hit = self.__dict__.get("_region_codes_hit")
+        if hit is None or hit[0] is not values or hit[1] != dev:
+            if self.region_by == self.results_by:
+                codes = self._labels().codes
+            else:
+                codes = label_codes(agent_labels(values, self.n_agents), self.region_labels)
+            hit = self.__dict__["_region_codes_hit"] = (values, dev,
+                                                        ops.make_seed_labels(codes, len(self.region_labels), dev))
+        return hit[2]
+
+    def _region(self, timer):
+        """ops.Region of the step at ``timer``: the product of the factors of the regional policies active then, or None
+        when none is."""
+        rp = getattr(self.model.policies, "regional_policies", None)
+        if self.region_by is None or not rp.active(timer):
+            return None
+        dev = self.data["agent"].susceptibility.device
+        return ops.Region(self._region_codes(), rp.factor(timer, self.region_labels, dev, self.batch))
+
     def _labels(self):
         """ops.Labels of ``results_by`` on the device (built once per label array and device, like
         ``_ethnicity_codes``), or None."""
@@ -324,7 +366,8 @@ class Runner(torch.nn.Module):
             if timer.date < timer.final_date:      # the schedule is known: tell the step what the next one will be
                 ahead = copy.copy(timer)
                 next(ahead)
-            out = model.step(data, timer, age_bins=self._age_bins_host, want_probs=False, next_timer=ahead, label=label)
+            out = model.step(data, timer, age_bins=self._age_bins_host, want_probs=False, next_timer=ahead, label=label,
+                             region=self._region(timer))
             data = out[0]
             reds.append(out[1])
             if label is not None:

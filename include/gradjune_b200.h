@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GJ_ABI_VERSION 12
+#define GJ_ABI_VERSION 13
 
 #define GJ_MAX_TYPES 8      /* edge types (household, company, school, university, care_home, leisure, ...) */
 #define GJ_MAX_NETS 16      /* infection networks active in one step */
@@ -310,6 +310,17 @@ typedef struct gj_fwd_io {
   const int32_t* seed_label;  /* [N] */
   int32_t n_seed_labels;      /* 1 .. 2^30 */
   int32_t _pad_seed;
+  /* regional transmission factor (GJ_MODE_STEP with the networks phase; NULL = none): region[a] is agent a's region in
+   * [0, n_regions), and agent a's summed pressure is multiplied by region_factor[region[a]] before the clamp:
+   * lam' = lam * m, q = clamp(exp(-clamp(lam', 1e-6, 100) * dt), 0, 1).  The factor is the receiving agent's: it
+   * applies to every network.  tape_v keeps the pre-factor value, so the backward is given the same region and
+   * region_factor; lam (the diagnostic output) is lam'.  A factor of 1 leaves lam' bit-equal to lam.  Factors must be
+   * >= 0 and codes must lie in [0, n_regions): neither is checked on the device.  region_factor may be NULL only when
+   * region is.  A call with a region factor does not produce the look-ahead of gj_step_forward_next. */
+  const int32_t* region;      /* [N] */
+  int32_t n_regions;          /* 1 .. 2^30 */
+  int32_t _pad_region;
+  const float* region_factor; /* [n_regions] (batched: [n_samples][region_stride]) */
 } gj_fwd_io;
 
 typedef struct gj_bwd_io {
@@ -370,6 +381,20 @@ typedef struct gj_bwd_io {
   const int32_t* seed_order;    /* [N] */
   const int32_t* seed_offsets;  /* [n_seed_labels + 1] */
   float* seed_work;             /* [N] workspace */
+  /* regional transmission factor: the forward's region / n_regions / region_factor (NULL = none).  The per-agent pass
+   * passes d/dlam' * m down the usual chain (w, g_s) and writes d/dlam' * lam (the pre-factor pressure) to region_work;
+   * with g_region_factor non-NULL a reduction then writes g_region_factor[r] = sum of region_work over the agents of
+   * region r, the same deterministic fp64 reduction as seeding by label: region_order lists the agents stably sorted by
+   * region, region_offsets[r] is where region r starts in it ([n_regions + 1], region_offsets[n_regions] = N).  The
+   * result is bit-reproducible and independent of the launch grid. */
+  const int32_t* region;          /* [N] */
+  int32_t n_regions;
+  int32_t _pad_region;
+  const float* region_factor;     /* [n_regions] (batched: [n_samples][region_stride]) */
+  const int32_t* region_order;    /* [N] */
+  const int32_t* region_offsets;  /* [n_regions + 1] */
+  float* region_work;             /* [N] workspace (batched: [n_samples][agent_stride]) */
+  float* g_region_factor;         /* [n_regions] (batched: [n_samples][region_stride]), or NULL */
 } gj_bwd_io;
 
 /* ---- library ---------------------------------------------------------------------------- */
@@ -446,6 +471,9 @@ typedef struct gj_batch {
   float* noise;
   /* stride of red_label / g_red_label / label_acc (elements, >= 2 * n_labels when a label table is given) */
   int64_t label_stride;
+  /* stride of region_factor / g_region_factor (elements, >= n_regions when a region factor is given): every sample has
+   * its own row of factors and of their gradient */
+  int64_t region_stride;
 } gj_batch;
 int gj_step_forward_batch(const gj_world_desc* w, const gj_step_params* p, const gj_fwd_io* io, const gj_batch* batch,
                           void* stream);
