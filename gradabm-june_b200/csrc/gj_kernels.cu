@@ -44,13 +44,13 @@ static int bad(const char* what) {
 enum KernelId {
   K_TRANSMISSION = 0, K_GROUP_SMALL_F, K_GROUP_CHUNK_F, K_GROUP_FIX_F, K_AGENT_FWD,
   K_AGENT_BWD, K_GROUP_SMALL_B, K_GROUP_CHUNK_B, K_GROUP_FIX_B, K_DBETA, K_AGENT_BWD_GATHER, K_CELL, K_OTHER, K_SEED,
-  K_EXCHANGE, K_SEED_GRAD, K_REGION_GRAD, K_COUNT
+  K_EXCHANGE, K_SEED_GRAD, K_REGION_GRAD, K_VENUE_GRAD, K_COUNT
 };
 static const char* kKernelNames[K_COUNT] = {
   "transmission", "group_small<fwd>", "group_chunk<fwd>", "group_fix<fwd>", "agent_forward",
   "agent_backward", "group_small<bwd>", "group_chunk<bwd>", "group_fix<bwd>", "dbeta",
   "backward_gather", "cell_groups+gather", "other", "seeding", "boundary_exchange", "seed_label_grad",
-  "region_factor_grad"};
+  "region_factor_grad", "venue_factor_grad"};
 constexpr int kMaxProfiled = 16384;
 struct Profiler {
   bool on = false;
@@ -270,13 +270,22 @@ __device__ __forceinline__ void group_store(const gj_world_desc& w, const gj_ste
   }
 }
 
-template <bool kBwd>
-__global__ void __launch_bounds__(kBlock) k_group_small(gj_world_desc w, gj_step_params p, Channels ch,
-                                                        const float* __restrict__ beta,
-                                                        const float* __restrict__ lprob,
-                                                        const float* __restrict__ in0,
-                                                        const float* __restrict__ in1, float* __restrict__ out_a,
-                                                        float* __restrict__ out_b) {
+// per-channel beta of group g; kVenue: times the venue factor of the group's region
+template <bool kVenue>
+__device__ __forceinline__ void group_betas(const Channels& ch, int type, int nch, const float* __restrict__ beta,
+                                            const Venue& v, uint32_t g, float (&beta_c)[GJ_MAX_CHANNELS]) {
+#pragma unroll
+  for (int c = 0; c < GJ_MAX_CHANNELS; ++c)
+    beta_c[c] = (c < nch) ? (kVenue ? beta[ch.net[type][c]] * venue_factor(v, ch.net[type][c], g)
+                                    : beta[ch.net[type][c]])
+                          : 0.0f;
+}
+
+template <bool kBwd, bool kVenue>
+__device__ __forceinline__ void group_small_body(const gj_world_desc& w, const gj_step_params& p, const Channels& ch,
+                                                 const float* __restrict__ beta, const float* __restrict__ lprob,
+                                                 const float* __restrict__ in0, const float* __restrict__ in1,
+                                                 float* __restrict__ out_a, float* __restrict__ out_b, const Venue& v) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= w.n_small) return;
   const uint32_t g = w.small_groups[i];
@@ -284,8 +293,7 @@ __global__ void __launch_bounds__(kBlock) k_group_small(gj_world_desc w, gj_step
   const int nch = ch.nch[type];
   if (nch == 0) return;
   float beta_c[GJ_MAX_CHANNELS];
-#pragma unroll
-  for (int c = 0; c < GJ_MAX_CHANNELS; ++c) beta_c[c] = (c < nch) ? beta[ch.net[type][c]] : 0.0f;
+  group_betas<kVenue>(ch, type, nch, beta, v, g, beta_c);
   const float pcg = w.pc[g];
   GroupAcc acc;
 #pragma unroll
@@ -295,16 +303,33 @@ __global__ void __launch_bounds__(kBlock) k_group_small(gj_world_desc w, gj_step
     group_member<kBwd>(p, ch, type, nch, beta_c, pcg, w.gm_agent[j], in0, in1, w.cls, lprob, acc);
   group_store<kBwd>(w, p, ch, type, nch, beta_c, pcg, g, acc, out_a, out_b);
 }
-
-// one warp per chunk (<= GJ_CHUNK members): lanes stride over the member list, then a fixed shuffle tree
 template <bool kBwd>
-__global__ void __launch_bounds__(kBlock) k_group_chunk(gj_world_desc w, gj_step_params p, Channels ch,
+__global__ void __launch_bounds__(kBlock) k_group_small(gj_world_desc w, gj_step_params p, Channels ch,
                                                         const float* __restrict__ beta,
                                                         const float* __restrict__ lprob,
                                                         const float* __restrict__ in0,
                                                         const float* __restrict__ in1, float* __restrict__ out_a,
-                                                        float* __restrict__ out_b, float* __restrict__ part_a,
-                                                        float* __restrict__ part_b) {
+                                                        float* __restrict__ out_b) {
+  group_small_body<kBwd, false>(w, p, ch, beta, lprob, in0, in1, out_a, out_b, Venue{nullptr, nullptr, 0});
+}
+template <bool kBwd>
+__global__ void __launch_bounds__(kBlock) k_group_small_venue(gj_world_desc w, gj_step_params p, Channels ch,
+                                                              const float* __restrict__ beta,
+                                                              const float* __restrict__ lprob,
+                                                              const float* __restrict__ in0,
+                                                              const float* __restrict__ in1, float* __restrict__ out_a,
+                                                              float* __restrict__ out_b, Venue v) {
+  group_small_body<kBwd, true>(w, p, ch, beta, lprob, in0, in1, out_a, out_b, v);
+}
+
+// one warp per chunk (<= GJ_CHUNK members): lanes stride over the member list, then a fixed shuffle tree
+template <bool kBwd, bool kVenue>
+__device__ __forceinline__ void group_chunk_body(const gj_world_desc& w, const gj_step_params& p, const Channels& ch,
+                                                 const float* __restrict__ beta, const float* __restrict__ lprob,
+                                                 const float* __restrict__ in0, const float* __restrict__ in1,
+                                                 float* __restrict__ out_a, float* __restrict__ out_b,
+                                                 float* __restrict__ part_a, float* __restrict__ part_b,
+                                                 const Venue& v) {
   const int lane = threadIdx.x & 31;
   const int64_t ci = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (ci >= w.n_chunks) return;
@@ -313,8 +338,7 @@ __global__ void __launch_bounds__(kBlock) k_group_chunk(gj_world_desc w, gj_step
   const int nch = ch.nch[type];
   if (nch == 0) return;
   float beta_c[GJ_MAX_CHANNELS];
-#pragma unroll
-  for (int c = 0; c < GJ_MAX_CHANNELS; ++c) beta_c[c] = (c < nch) ? beta[ch.net[type][c]] : 0.0f;
+  group_betas<kVenue>(ch, type, nch, beta, v, g, beta_c);
   const float pcg = w.pc[g];
   GroupAcc acc;
 #pragma unroll
@@ -343,14 +367,34 @@ __global__ void __launch_bounds__(kBlock) k_group_chunk(gj_world_desc w, gj_step
     }
   }
 }
+template <bool kBwd>
+__global__ void __launch_bounds__(kBlock) k_group_chunk(gj_world_desc w, gj_step_params p, Channels ch,
+                                                        const float* __restrict__ beta,
+                                                        const float* __restrict__ lprob,
+                                                        const float* __restrict__ in0,
+                                                        const float* __restrict__ in1, float* __restrict__ out_a,
+                                                        float* __restrict__ out_b, float* __restrict__ part_a,
+                                                        float* __restrict__ part_b) {
+  group_chunk_body<kBwd, false>(w, p, ch, beta, lprob, in0, in1, out_a, out_b, part_a, part_b,
+                                Venue{nullptr, nullptr, 0});
+}
+template <bool kBwd>
+__global__ void __launch_bounds__(kBlock) k_group_chunk_venue(gj_world_desc w, gj_step_params p, Channels ch,
+                                                              const float* __restrict__ beta,
+                                                              const float* __restrict__ lprob,
+                                                              const float* __restrict__ in0,
+                                                              const float* __restrict__ in1, float* __restrict__ out_a,
+                                                              float* __restrict__ out_b, float* __restrict__ part_a,
+                                                              float* __restrict__ part_b, Venue v) {
+  group_chunk_body<kBwd, true>(w, p, ch, beta, lprob, in0, in1, out_a, out_b, part_a, part_b, v);
+}
 
 // groups spanning several chunks: add the chunk partials in chunk order
-template <bool kBwd>
-__global__ void __launch_bounds__(kBlock) k_group_fix(gj_world_desc w, gj_step_params p, Channels ch,
-                                                      const float* __restrict__ beta,
-                                                      const float* __restrict__ part_a,
-                                                      const float* __restrict__ part_b, float* __restrict__ out_a,
-                                                      float* __restrict__ out_b) {
+template <bool kBwd, bool kVenue>
+__device__ __forceinline__ void group_fix_body(const gj_world_desc& w, const gj_step_params& p, const Channels& ch,
+                                               const float* __restrict__ beta, const float* __restrict__ part_a,
+                                               const float* __restrict__ part_b, float* __restrict__ out_a,
+                                               float* __restrict__ out_b, const Venue& v) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= w.n_big) return;
   const uint32_t g = w.big_groups[i];
@@ -358,8 +402,7 @@ __global__ void __launch_bounds__(kBlock) k_group_fix(gj_world_desc w, gj_step_p
   const int nch = ch.nch[type];
   if (nch == 0) return;
   float beta_c[GJ_MAX_CHANNELS];
-#pragma unroll
-  for (int c = 0; c < GJ_MAX_CHANNELS; ++c) beta_c[c] = (c < nch) ? beta[ch.net[type][c]] : 0.0f;
+  group_betas<kVenue>(ch, type, nch, beta, v, g, beta_c);
   GroupAcc acc;
 #pragma unroll
   for (int c = 0; c < GJ_MAX_CHANNELS; ++c) acc.a[c] = acc.b[c] = 0.0f;
@@ -373,6 +416,22 @@ __global__ void __launch_bounds__(kBlock) k_group_fix(gj_world_desc w, gj_step_p
     }
   }
   group_store<kBwd>(w, p, ch, type, nch, beta_c, w.pc[g], g, acc, out_a, out_b);
+}
+template <bool kBwd>
+__global__ void __launch_bounds__(kBlock) k_group_fix(gj_world_desc w, gj_step_params p, Channels ch,
+                                                      const float* __restrict__ beta,
+                                                      const float* __restrict__ part_a,
+                                                      const float* __restrict__ part_b, float* __restrict__ out_a,
+                                                      float* __restrict__ out_b) {
+  group_fix_body<kBwd, false>(w, p, ch, beta, part_a, part_b, out_a, out_b, Venue{nullptr, nullptr, 0});
+}
+template <bool kBwd>
+__global__ void __launch_bounds__(kBlock) k_group_fix_venue(gj_world_desc w, gj_step_params p, Channels ch,
+                                                            const float* __restrict__ beta,
+                                                            const float* __restrict__ part_a,
+                                                            const float* __restrict__ part_b, float* __restrict__ out_a,
+                                                            float* __restrict__ out_b, Venue v) {
+  group_fix_body<kBwd, true>(w, p, ch, beta, part_a, part_b, out_a, out_b, v);
 }
 
 // ================================================================================================
@@ -590,11 +649,15 @@ struct DbetaPlan {
   int64_t n_range_parts;      // partials written by the backward gather (tiles, or CTAs of the persistent grid)
 };
 
-__global__ void __launch_bounds__(kBlock) k_dbeta(gj_world_desc w, gj_step_params p, Plan pl, DbetaPlan dp,
-                                                  const float* __restrict__ S_un, const float* __restrict__ R,
-                                                  const double* __restrict__ dbeta_tile, double* __restrict__ partials,
-                                                  unsigned int* __restrict__ tickets, float* __restrict__ g_beta,
-                                                  Batch bt) {
+// kVenue: dL/dbeta_k = sum_g ((own * pc_g) * f) * S~_g * R_g, and (work != NULL) the per-group terms of
+// dL/df = beta_k * own * pc_g * S~_g * R_g go to work, laid out like S_un / R
+template <bool kVenue>
+__device__ __forceinline__ void dbeta_body(const gj_world_desc& w, const gj_step_params& p, const Plan& pl,
+                                           const DbetaPlan& dp, const float* __restrict__ S_un,
+                                           const float* __restrict__ R, const double* __restrict__ dbeta_tile,
+                                           double* __restrict__ partials, unsigned int* __restrict__ tickets,
+                                           float* __restrict__ g_beta, const Batch& bt, const float* __restrict__ beta,
+                                           Venue v, float* __restrict__ work) {
   pdl_launch();
   pdl_wait();
   if (bt.nb > 1) {   // batched ensemble: sample blockIdx.z
@@ -605,6 +668,11 @@ __global__ void __launch_bounds__(kBlock) k_dbeta(gj_world_desc w, gj_step_param
     partials = scr_shift(partials, bt, s);
     tickets = scr_shift(tickets, bt, s);
     g_beta += (int64_t)s * bt.sBeta;
+    if (kVenue) {
+      beta += (int64_t)s * bt.sBeta;
+      v.factor += (int64_t)s * bt.sVen;
+      if (work) work += (int64_t)s * bt.sG;
+    }
   }
   const int k = blockIdx.y;
   const gj_net net = p.nets[k];
@@ -618,12 +686,40 @@ __global__ void __launch_bounds__(kBlock) k_dbeta(gj_world_desc w, gj_step_param
     const int64_t g0 = w.type_group_off[net.type];
     const int64_t G = w.type_group_off[net.type + 1] - g0;
     const int64_t so = dp.soff[k];
+    const float bk = kVenue ? beta[k] : 0.0f;
+    // network k's own work row (nets[k].s_off): generic networks sharing an edge type share `so` on the throughput
+    // path, but each has its own beta_k and its own row of d/df
+    const int64_t wo = net.s_off;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < G; i += stride) {
       const float own = w.dbeta_w ? w.dbeta_w[g0 + i] : 1.0f;  // partitioned worlds: every group counted by one rank
-      acc[0] += (double)((own * w.pc[g0 + i]) * S_un[so + i]) * (double)R[so + i];
+      if (kVenue) {
+        const float opc = own * w.pc[g0 + i];
+        const float Sg = S_un[so + i], Rg = R[so + i];
+        acc[0] += (double)((opc * venue_factor(v, k, (uint32_t)(g0 + i))) * Sg) * (double)Rg;
+        if (work) work[wo + i] = (float)((double)((bk * opc) * Sg) * (double)Rg);
+      } else {
+        acc[0] += (double)((own * w.pc[g0 + i]) * S_un[so + i]) * (double)R[so + i];
+      }
     }
   }
   block_reduce_finish<1>(acc, 1, partials + (int64_t)k * kRedBlocks, tickets + 1 + k, g_beta + k);
+}
+__global__ void __launch_bounds__(kBlock) k_dbeta(gj_world_desc w, gj_step_params p, Plan pl, DbetaPlan dp,
+                                                  const float* __restrict__ S_un, const float* __restrict__ R,
+                                                  const double* __restrict__ dbeta_tile, double* __restrict__ partials,
+                                                  unsigned int* __restrict__ tickets, float* __restrict__ g_beta,
+                                                  Batch bt) {
+  dbeta_body<false>(w, p, pl, dp, S_un, R, dbeta_tile, partials, tickets, g_beta, bt, nullptr,
+                    Venue{nullptr, nullptr, 0}, nullptr);
+}
+__global__ void __launch_bounds__(kBlock) k_dbeta_venue(gj_world_desc w, gj_step_params p, Plan pl, DbetaPlan dp,
+                                                        const float* __restrict__ S_un, const float* __restrict__ R,
+                                                        const double* __restrict__ dbeta_tile,
+                                                        double* __restrict__ partials,
+                                                        unsigned int* __restrict__ tickets, float* __restrict__ g_beta,
+                                                        Batch bt, const float* __restrict__ beta, Venue v,
+                                                        float* __restrict__ work) {
+  dbeta_body<true>(w, p, pl, dp, S_un, R, dbeta_tile, partials, tickets, g_beta, bt, beta, v, work);
 }
 
 __global__ void k_philox_fill(uint64_t seed, uint32_t call, int64_t first, int64_t n, float* __restrict__ E,
@@ -680,7 +776,8 @@ static int build_channels(const gj_world_desc* w, const gj_step_params* p, Chann
   return 0;
 }
 
-static const Batch kNoBatch = {1, 0u, 0, 0, 0, 0, nullptr, 0};
+static const Batch kNoBatch = {1, 0u, 0, 0, 0, 0, nullptr, 0, 0, 0};
+static const Venue kNoVenue = {nullptr, nullptr, 0};
 // grid of a persistent kernel in a batched launch: the resident wave is split between the samples (block = run * nb +
 // sample), at least one CTA and at most one per tile for each
 static inline int batch_grid(const gj_world_desc* w, int64_t resident, const Batch& bt) {
@@ -786,23 +883,36 @@ static int check_world(const gj_world_desc* w) {
 template <bool kBwd>
 static int launch_group_pass(const gj_world_desc* w, const gj_step_params* p, const Channels& ch, const float* beta,
                              const float* lprob, const float* in0, const float* in1, float* out_a, float* out_b,
-                             const Scratch& sc, cudaStream_t st) {
+                             const Scratch& sc, cudaStream_t st, const Venue& v = kNoVenue) {
+  const bool venue = v.region != nullptr;
   if (w->n_small > 0) {
     ProfScope ps(kBwd ? K_GROUP_SMALL_B : K_GROUP_SMALL_F, st);
-    k_group_small<kBwd><<<blocks_for(w->n_small, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, lprob, in0, in1, out_a,
-                                                                         out_b);
+    if (venue)
+      k_group_small_venue<kBwd><<<blocks_for(w->n_small, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, lprob, in0, in1,
+                                                                                 out_a, out_b, v);
+    else
+      k_group_small<kBwd><<<blocks_for(w->n_small, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, lprob, in0, in1, out_a,
+                                                                           out_b);
     GJ_CHECK_LAUNCH("k_group_small");
   }
   if (w->n_chunks > 0) {
     ProfScope ps(kBwd ? K_GROUP_CHUNK_B : K_GROUP_CHUNK_F, st);
-    k_group_chunk<kBwd><<<blocks_for(w->n_chunks * 32, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, lprob, in0, in1,
-                                                                              out_a, out_b, sc.part_a, sc.part_b);
+    if (venue)
+      k_group_chunk_venue<kBwd><<<blocks_for(w->n_chunks * 32, kBlock), kBlock, 0, st>>>(
+          *w, *p, ch, beta, lprob, in0, in1, out_a, out_b, sc.part_a, sc.part_b, v);
+    else
+      k_group_chunk<kBwd><<<blocks_for(w->n_chunks * 32, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, lprob, in0, in1,
+                                                                                out_a, out_b, sc.part_a, sc.part_b);
     GJ_CHECK_LAUNCH("k_group_chunk");
   }
   if (w->n_big > 0) {
     ProfScope ps(kBwd ? K_GROUP_FIX_B : K_GROUP_FIX_F, st);
-    k_group_fix<kBwd><<<blocks_for(w->n_big, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, sc.part_a, sc.part_b, out_a,
-                                                                     out_b);
+    if (venue)
+      k_group_fix_venue<kBwd><<<blocks_for(w->n_big, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, sc.part_a, sc.part_b,
+                                                                             out_a, out_b, v);
+    else
+      k_group_fix<kBwd><<<blocks_for(w->n_big, kBlock), kBlock, 0, st>>>(*w, *p, ch, beta, sc.part_a, sc.part_b, out_a,
+                                                                       out_b);
     GJ_CHECK_LAUNCH("k_group_fix");
   }
   return 0;
@@ -811,7 +921,7 @@ static int launch_group_pass(const gj_world_desc* w, const gj_step_params* p, co
 // cell tier, part 1: tile partials -> per-group sums (plain + beta*pc-scaled)
 static int launch_cell_groups(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, const float* beta,
                               float* out_scaled, float* out_plain, const Scratch& sc, cudaStream_t st,
-                              const Batch& bt = kNoBatch) {
+                              const Batch& bt = kNoBatch, const Venue& v = kNoVenue) {
   if (pl.n_t2 == 0) return 0;
   int64_t maxG = 1;
   for (int j = 0; j < pl.n_t2; ++j) {
@@ -820,8 +930,12 @@ static int launch_cell_groups(const gj_world_desc* w, const gj_step_params* p, c
     if (G > maxG) maxG = G;
   }
   ProfScope ps(K_CELL, st);
-  launch_pdl(k_cell_groups, dim3(blocks_for(maxG, kBlock), pl.n_t2, bt.nb), dim3(kBlock), 0, st, *w, *p, pl, beta,
-             (const float*)sc.tile_part, out_scaled, out_plain, bt);
+  if (v.region)
+    launch_pdl(k_cell_groups_venue, dim3(blocks_for(maxG, kBlock), pl.n_t2, bt.nb), dim3(kBlock), 0, st, *w, *p, pl,
+               beta, (const float*)sc.tile_part, out_scaled, out_plain, bt, v);
+  else
+    launch_pdl(k_cell_groups, dim3(blocks_for(maxG, kBlock), pl.n_t2, bt.nb), dim3(kBlock), 0, st, *w, *p, pl, beta,
+               (const float*)sc.tile_part, out_scaled, out_plain, bt);
   GJ_CHECK_LAUNCH("k_cell_groups");
   return 0;
 }
@@ -894,16 +1008,16 @@ static bool lean_plan(const gj_world_desc* w, const gj_step_params* p, const Pla
 // n_giant_chunks chunks / n_giant_big multi-chunk groups of the lists), then the accumulators become fp32 sums
 static int launch_lean_group_pass(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, const float* beta,
                                   const float* in, float* out_scaled, float* out_plain, const Scratch& sc, bool bwd,
-                                  cudaStream_t st, const Batch& bt);
+                                  cudaStream_t st, const Batch& bt, const Venue& v);
 static int launch_lean_forward_sums(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, const float* beta,
                                     const float* in, float* out_scaled, float* out_plain, const Scratch& sc,
-                                    cudaStream_t st, const Batch& bt) {
+                                    cudaStream_t st, const Batch& bt, const Venue& v) {
   if (w->n_giant_chunks > 0) {
     gj_world_desc wg = *w;
     wg.n_small = 0;
     wg.n_chunks = w->n_giant_chunks;
     wg.n_big = w->n_giant_big;
-    if (int e = launch_lean_group_pass(&wg, p, pl, beta, in, out_scaled, out_plain, sc, false, st, bt)) return e;
+    if (int e = launch_lean_group_pass(&wg, p, pl, beta, in, out_scaled, out_plain, sc, false, st, bt, v)) return e;
   }
   {
     ProfScope ps(K_GROUP_SMALL_F, st);
@@ -917,8 +1031,12 @@ static int launch_lean_forward_sums(const gj_world_desc* w, const gj_step_params
         ++gr.n;
       }
     if (gr.n == 0) return 0;
-    launch_pdl(k_lean_scatter_finalize, dim3(blocks_for(gr.start[gr.n], kBlock) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl,
-               gr, beta, in, sct, out_scaled, out_plain, bt);
+    if (v.region)
+      launch_pdl(k_lean_scatter_finalize_venue, dim3(blocks_for(gr.start[gr.n], kBlock) * bt.nb), dim3(kBlock), 0, st,
+                 *w, *p, pl, gr, beta, in, sct, out_scaled, out_plain, bt, v);
+    else
+      launch_pdl(k_lean_scatter_finalize, dim3(blocks_for(gr.start[gr.n], kBlock) * bt.nb), dim3(kBlock), 0, st, *w, *p,
+                 pl, gr, beta, in, sct, out_scaled, out_plain, bt);
     GJ_CHECK_LAUNCH("k_lean_scatter_finalize");
   }
   return 0;
@@ -926,19 +1044,27 @@ static int launch_lean_forward_sums(const gj_world_desc* w, const gj_step_params
 
 static int launch_lean_group_pass(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, const float* beta,
                                   const float* in, float* out_scaled, float* out_plain, const Scratch& sc, bool bwd,
-                                  cudaStream_t st, const Batch& bt) {
+                                  cudaStream_t st, const Batch& bt, const Venue& v) {
   if (w->n_small > 0 || w->n_chunks > 0) {
     ProfScope ps(bwd ? K_GROUP_CHUNK_B : K_GROUP_CHUNK_F, st);
     const int chunk_blocks = w->n_chunks > 0 ? blocks_for(w->n_chunks * 32, kBlock) : 0;
     const int small_blocks = w->n_small > 0 ? blocks_for(w->n_small, kBlock) : 0;
-    launch_pdl(k_lean_group_sums, dim3((chunk_blocks + small_blocks) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl, beta, in,
-               out_scaled, out_plain, sc.part_a, chunk_blocks, bt);
+    if (v.region)
+      launch_pdl(k_lean_group_sums_venue, dim3((chunk_blocks + small_blocks) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl,
+                 beta, in, out_scaled, out_plain, sc.part_a, chunk_blocks, bt, v);
+    else
+      launch_pdl(k_lean_group_sums, dim3((chunk_blocks + small_blocks) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl, beta,
+                 in, out_scaled, out_plain, sc.part_a, chunk_blocks, bt);
     GJ_CHECK_LAUNCH("k_lean_group_sums");
   }
   if (w->n_big > 0) {
     ProfScope ps(bwd ? K_GROUP_FIX_B : K_GROUP_FIX_F, st);
-    launch_pdl(k_lean_group_fix, dim3(blocks_for(w->n_big * 32, kBlock) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl, beta,
-               (const float*)sc.part_a, out_scaled, out_plain, bt);
+    if (v.region)
+      launch_pdl(k_lean_group_fix_venue, dim3(blocks_for(w->n_big * 32, kBlock) * bt.nb), dim3(kBlock), 0, st, *w, *p,
+                 pl, beta, (const float*)sc.part_a, out_scaled, out_plain, bt, v);
+    else
+      launch_pdl(k_lean_group_fix, dim3(blocks_for(w->n_big * 32, kBlock) * bt.nb), dim3(kBlock), 0, st, *w, *p, pl,
+                 beta, (const float*)sc.part_a, out_scaled, out_plain, bt);
     GJ_CHECK_LAUNCH("k_lean_group_fix");
   }
   return 0;
@@ -983,11 +1109,12 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
 #undef GJ_K1C
       GJ_CHECK_LAUNCH("k_lean_transmission");
     }
+    const Venue v{io->venue_region, io->venue_factor, io->n_venue_regions};
     if (lp.has_generic)
       if (int e = launch_lean_forward_sums(w, p, pl, io->beta, quar ? io->Tq : io->T, io->S_scaled + lp.gen_base,
-                                           io->S_unscaled + lp.gen_base, sc, st, bt))
+                                           io->S_unscaled + lp.gen_base, sc, st, bt, v))
         return e;
-    if (int e = launch_cell_groups(w, p, pl, io->beta, io->S_scaled, io->S_unscaled, sc, st, bt)) return e;
+    if (int e = launch_cell_groups(w, p, pl, io->beta, io->S_scaled, io->S_unscaled, sc, st, bt, v)) return e;
   }
   if (p->stage == GJ_STAGE_SUMS) return 0;
   if (int e = launch_cell_gather(w, p, pl, io->S_scaled, sc, st, bt)) return e;
@@ -1114,6 +1241,64 @@ static int lean_forward(const gj_world_desc* w, const gj_step_params* p, const P
   return 0;
 }
 
+// seeding by label, backward: the per-agent pass writes d/dseed_fraction to seed_work, then the per-label reduction.
+// The reduction's chunk partials live in the scratch's reduction partials (free once the agent pass is done); the chunk
+// is the smallest power of two >= kSeedChunk whose partials fit there, so it depends on the world only.
+// Venue regions hold few groups each (a leisure venue is often a region of its own): a warp walks its chunk's labels
+// one after the other, so the groups' reduction uses short chunks to spread them over many warps.
+constexpr int64_t kSeedChunk = 2048;
+constexpr int64_t kVenueChunk = 32;
+static int64_t seed_chunk(const gj_world_desc* w, int64_t N, int64_t min_chunk = kSeedChunk) {
+  const int64_t n_tiles = w->n_tiles > 0 ? w->n_tiles : 1;
+  const int64_t slots = (n_tiles > kRedBlocks ? n_tiles : kRedBlocks) * kMaxRed;   // doubles in Scratch::red_part
+  int64_t chunk = min_chunk;
+  while (2 * ((N + chunk - 1) / chunk) > slots) chunk *= 2;
+  return chunk;
+}
+// out[l] = sum of work over the N items (agents, or the groups of one edge type) of label l (order / offsets: the
+// items stably sorted by label), in fp64 over fixed chunks combined in chunk order: bit-reproducible and independent
+// of the launch grid
+static int label_sums(const gj_world_desc* w, int64_t N, const int32_t* order, const int32_t* offsets, int n_labels,
+                      const float* work, const Scratch& sc, float* out, cudaStream_t st,
+                      int64_t min_chunk = kSeedChunk) {
+  const int64_t chunk = seed_chunk(w, N, min_chunk);
+  const int64_t n_chunks = (N + chunk - 1) / chunk;
+  k_seed_label_grad<<<blocks_for(n_chunks * 32, kBlock), kBlock, 0, st>>>(N, chunk, order, offsets, n_labels, work,
+                                                                         sc.red_part, out);
+  GJ_CHECK_LAUNCH("k_seed_label_grad");
+  k_seed_label_fix<<<blocks_for((int64_t)n_labels * 32, kBlock), kBlock, 0, st>>>(chunk, offsets, n_labels, sc.red_part,
+                                                                                  out);
+  GJ_CHECK_LAUNCH("k_seed_label_fix");
+  return 0;
+}
+
+// regional venue factor, backward: k_dbeta_venue wrote network k's per-group terms of dL/df to its own row of
+// venue_work (at nets[k].s_off); the per-label reduction sums them over the groups of the network's edge type, region by region, per network
+// and sample.  A RANGE-tier network has no group terms: its row is 0.
+static int venue_backward(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, const gj_bwd_io* io,
+                          const Scratch& sc, const Batch& bt, cudaStream_t st) {
+  if (!io->venue_region || !io->g_venue_factor) return 0;
+  ProfScope ps(K_VENUE_GRAD, st);
+  const int n = io->n_venue_regions;
+  for (int s = 0; s < bt.nb; ++s) {
+    for (int k = 0; k < p->n_nets; ++k) {
+      float* out = io->g_venue_factor + (int64_t)s * bt.sVen + (int64_t)k * n;
+      const int t = p->nets[k].type;
+      if (pl.tier[k] == GJ_TIER_RANGE) {
+        const cudaError_t e = cudaMemsetAsync(out, 0, sizeof(float) * (size_t)n, st);
+        if (e != cudaSuccess) return fail("cudaMemsetAsync (g_venue_factor)", e);
+        continue;
+      }
+      const int64_t g0 = w->type_group_off[t];
+      if (int e = label_sums(w, w->type_group_off[t + 1] - g0, io->venue_order + g0,
+                             io->venue_offsets + (int64_t)t * (n + 1), n,
+                             io->venue_work + (int64_t)s * bt.sG + p->nets[k].s_off, sc, out, st, kVenueChunk))
+        return e;
+    }
+  }
+  return 0;
+}
+
 static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const Plan& pl, LeanPlan lp,
                          const gj_bwd_io* io, const Scratch& sc, cudaStream_t st, const Batch& bt = kNoBatch) {
   const bool quar = p->n_quar > 0;
@@ -1192,11 +1377,12 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
 #undef GJ_LEAN_BWD_R
       GJ_CHECK_LAUNCH("k_lean_backward");
     }
+    const Venue v{io->venue_region, io->venue_factor, io->n_venue_regions};
     if (lp.has_generic)
       if (int e = launch_lean_group_pass(w, p, pl, io->beta, quar ? io->wq : io->w, io->cR + lp.gen_base,
-                                         io->R + lp.gen_base, sc, true, st, bt))
+                                         io->R + lp.gen_base, sc, true, st, bt, v))
         return e;
-    if (int e = launch_cell_groups(w, p, pl, io->beta, io->cR, io->R, sc, st, bt)) return e;
+    if (int e = launch_cell_groups(w, p, pl, io->beta, io->cR, io->R, sc, st, bt, v)) return e;
   }
   if (p->stage == GJ_STAGE_SUMS) return 0;
   if (int e = launch_cell_gather(w, p, pl, io->cR, sc, st, bt)) return e;
@@ -1234,9 +1420,16 @@ static int lean_backward(const gj_world_desc* w, const gj_step_params* p, const 
     }
     dp.n_range_parts = gather_grid;
     dim3 grid2(kRedBlocks / 8, p->n_nets, bt.nb);
-    launch_pdl(k_dbeta, grid2, dim3(kBlock), 0, st, *w, *p, pl, dp, io->S_unscaled, (const float*)io->R,
-               (const double*)sc.dbeta_tile, sc.dbeta_part, sc.tickets, io->g_beta, bt);
+    if (io->venue_region)
+      launch_pdl(k_dbeta_venue, grid2, dim3(kBlock), 0, st, *w, *p, pl, dp, io->S_unscaled, (const float*)io->R,
+                 (const double*)sc.dbeta_tile, sc.dbeta_part, sc.tickets, io->g_beta, bt, io->beta,
+                 Venue{io->venue_region, io->venue_factor, io->n_venue_regions},
+                 io->g_venue_factor ? io->venue_work : nullptr);
+    else
+      launch_pdl(k_dbeta, grid2, dim3(kBlock), 0, st, *w, *p, pl, dp, io->S_unscaled, (const float*)io->R,
+                 (const double*)sc.dbeta_tile, sc.dbeta_part, sc.tickets, io->g_beta, bt);
     GJ_CHECK_LAUNCH("k_dbeta");
+    if (int e = venue_backward(w, p, pl, io, sc, bt, st)) return e;
   }
   return 0;
 }
@@ -1648,7 +1841,9 @@ static int make_batch(const gj_world_desc* w, const gj_step_params* p, const gj_
   bt->noise = b->noise;
   bt->sLab = b->label_stride;
   bt->sReg = b->region_stride;
+  bt->sVen = b->venue_stride;
   if (b->region_stride < 0) return bad("batch: region_stride must be >= 0");
+  if (b->venue_stride < 0) return bad("batch: venue_stride must be >= 0");
   if (b->noise && !aligned16(b->noise)) return bad("batch: noise must be 16-byte aligned");
   return 0;
 }
@@ -1667,6 +1862,14 @@ static int check_region(const int32_t* region, int n_regions, const float* facto
   if (n_regions < 1 || n_regions > (1 << 30)) return bad("n_regions must lie in [1, 2^30]");
   if (!factor) return bad("region given without region_factor");
   if (bt.nb > 1 && bt.sReg < (int64_t)n_regions) return bad("batch: region_stride must be >= n_regions");
+  return 0;
+}
+// regional venue factor: the checks of the header (codes and factors are not checked)
+static int check_venue(const gj_step_params* p, const int32_t* region, int n, const float* factor, const Batch& bt) {
+  if (!region) return 0;
+  if (n < 1 || n > (1 << 30)) return bad("n_venue_regions must lie in [1, 2^30]");
+  if (!factor) return bad("venue_region given without venue_factor");
+  if (bt.nb > 1 && bt.sVen < (int64_t)p->n_nets * n) return bad("batch: venue_stride must be >= n_nets * n_venue_regions");
   return 0;
 }
 static int finish_labels(const gj_fwd_io* io, cudaStream_t st, const Batch& bt) {
@@ -1692,6 +1895,7 @@ static int step_forward_impl(const gj_world_desc* w, const gj_step_params* p, co
     if (int e = make_batch(w, p, batch, &bt)) return e;
   if (int e = check_labels(io, bt)) return e;
   if (int e = check_region(io->region, io->n_regions, io->region_factor, bt)) return e;
+  if (int e = check_venue(p, io->venue_region, io->n_venue_regions, io->venue_factor, bt)) return e;
   const int rc = step_forward_run(w, p, next, io, stream, batch);
   if (rc < 0 || p->stage == GJ_STAGE_SUMS) return rc;
   if (int e = finish_labels(io, (cudaStream_t)stream, bt)) return e;
@@ -1831,11 +2035,12 @@ static int step_forward_run(const gj_world_desc* w, const gj_step_params* p, con
     }
     const float* T = io->T_in ? io->T_in : io->T;
     const float* Tq = (p->n_quar > 0) ? io->Tq : T;
+    const Venue v{io->venue_region, io->venue_factor, io->n_venue_regions};
     if (pl.n_generic > 0)
       if (int e = launch_group_pass<false>(w, &pp, ch, io->beta, io->leisure_prob, T, Tq, io->S_scaled, io->S_unscaled,
-                                           sc, st))
+                                           sc, st, v))
         return e;
-    if (int e = launch_cell_groups(w, &pp, pl, io->beta, io->S_scaled, io->S_unscaled, sc, st)) return e;
+    if (int e = launch_cell_groups(w, &pp, pl, io->beta, io->S_scaled, io->S_unscaled, sc, st, kNoBatch, v)) return e;
   }
   if (pp.stage == GJ_STAGE_SUMS) return 0;
   if (int e = launch_cell_gather(w, &pp, pl, io->S_scaled, sc, st)) return e;
@@ -1870,33 +2075,6 @@ int gj_step_forward_batch(const gj_world_desc* w, const gj_step_params* p, const
   return rc > 0 ? 0 : rc;
 }
 
-// seeding by label, backward: the per-agent pass writes d/dseed_fraction to seed_work, then the per-label reduction.
-// The reduction's chunk partials live in the scratch's reduction partials (free once the agent pass is done); the chunk
-// is the smallest power of two >= kSeedChunk whose partials fit there, so it depends on the world only.
-constexpr int64_t kSeedChunk = 2048;
-static int64_t seed_chunk(const gj_world_desc* w) {
-  const int64_t n_tiles = w->n_tiles > 0 ? w->n_tiles : 1;
-  const int64_t slots = (n_tiles > kRedBlocks ? n_tiles : kRedBlocks) * kMaxRed;   // doubles in Scratch::red_part
-  int64_t chunk = kSeedChunk;
-  while (2 * ((w->n_agents + chunk - 1) / chunk) > slots) chunk *= 2;
-  return chunk;
-}
-// out[l] = sum of work over the agents of label l (order / offsets: the agents stably sorted by label), in fp64 over
-// fixed chunks combined in chunk order: bit-reproducible and independent of the launch grid
-static int label_sums(const gj_world_desc* w, const int32_t* order, const int32_t* offsets, int n_labels,
-                      const float* work, const Scratch& sc, float* out, cudaStream_t st) {
-  const int64_t N = w->n_agents;
-  const int64_t chunk = seed_chunk(w);
-  const int64_t n_chunks = (N + chunk - 1) / chunk;
-  k_seed_label_grad<<<blocks_for(n_chunks * 32, kBlock), kBlock, 0, st>>>(N, chunk, order, offsets, n_labels, work,
-                                                                         sc.red_part, out);
-  GJ_CHECK_LAUNCH("k_seed_label_grad");
-  k_seed_label_fix<<<blocks_for((int64_t)n_labels * 32, kBlock), kBlock, 0, st>>>(chunk, offsets, n_labels, sc.red_part,
-                                                                                  out);
-  GJ_CHECK_LAUNCH("k_seed_label_fix");
-  return 0;
-}
-
 static int seed_backward(const gj_world_desc* w, const gj_step_params& pp, const gj_bwd_io* io, const Scratch& sc,
                          cudaStream_t st) {
   if (io->n_seed_labels < 1 || io->n_seed_labels > (1 << 30)) return bad("n_seed_labels must lie in [1, 2^30]");
@@ -1911,7 +2089,8 @@ static int seed_backward(const gj_world_desc* w, const gj_step_params& pp, const
   }
   if (!io->g_seed_fraction) return 0;
   ProfScope ps(K_SEED_GRAD, st);
-  return label_sums(w, io->seed_order, io->seed_offsets, io->n_seed_labels, io->seed_work, sc, io->g_seed_fraction, st);
+  return label_sums(w, w->n_agents, io->seed_order, io->seed_offsets, io->n_seed_labels, io->seed_work, sc,
+                    io->g_seed_fraction, st);
 }
 
 // regional transmission factor, backward: the agent kernels wrote d/dlam' * lam to region_work; the same per-label
@@ -1922,8 +2101,8 @@ static int region_backward(const gj_world_desc* w, const gj_bwd_io* io, const Sc
   if (!io->region || !io->g_region_factor) return 0;
   ProfScope ps(K_REGION_GRAD, st);
   for (int s = 0; s < bt.nb; ++s)
-    if (int e = label_sums(w, io->region_order, io->region_offsets, io->n_regions, io->region_work + (int64_t)s * bt.sN,
-                           sc, io->g_region_factor + (int64_t)s * bt.sReg, st))
+    if (int e = label_sums(w, w->n_agents, io->region_order, io->region_offsets, io->n_regions,
+                           io->region_work + (int64_t)s * bt.sN, sc, io->g_region_factor + (int64_t)s * bt.sReg, st))
       return e;
   return 0;
 }
@@ -1963,6 +2142,9 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
   if (io->region && !io->region_work) return bad("region given without region_work");
   if (io->region && io->g_region_factor && (!io->region_order || !io->region_offsets))
     return bad("g_region_factor given without region_order / region_offsets");
+  if (int e = check_venue(p, io->venue_region, io->n_venue_regions, io->venue_factor, bt)) return e;
+  if (io->venue_region && io->g_venue_factor && (!io->venue_order || !io->venue_offsets || !io->venue_work || !io->g_beta))
+    return bad("g_venue_factor given without venue_order / venue_offsets / venue_work / g_beta");
   const bool region_last = io->region && pp.stage != GJ_STAGE_SUMS;   // the per-region reduction ends the call
   if (!io->g_T && (!io->tinf || !io->inf || !io->maxinf || !io->k0 || !io->g_inf || !io->g_tinf))
     return bad("state arrays are NULL");
@@ -1991,10 +2173,12 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
       else k_tile_backward<false><<<grid, kBlock, 0, st>>>(*w, pp, pl, *io, sc.tile_part);
       GJ_CHECK_LAUNCH("k_tile_backward");
     }
+    const Venue v{io->venue_region, io->venue_factor, io->n_venue_regions};
     if (pl.n_generic > 0)
-      if (int e = launch_group_pass<true>(w, &pp, ch, io->beta, io->leisure_prob, io->w, io->wq, io->cR, io->R, sc, st))
+      if (int e = launch_group_pass<true>(w, &pp, ch, io->beta, io->leisure_prob, io->w, io->wq, io->cR, io->R, sc, st,
+                                          v))
         return e;
-    if (int e = launch_cell_groups(w, &pp, pl, io->beta, io->cR, io->R, sc, st)) return e;
+    if (int e = launch_cell_groups(w, &pp, pl, io->beta, io->cR, io->R, sc, st, kNoBatch, v)) return e;
   }
   if (pp.stage == GJ_STAGE_SUMS) return 0;
   if (int e = launch_cell_gather(w, &pp, pl, io->cR, sc, st)) return e;
@@ -2009,9 +2193,16 @@ static int step_backward_impl(const gj_world_desc* w, const gj_step_params* p, c
     for (int k = 0; k < GJ_MAX_NETS; ++k) dp.soff[k] = k < pp.n_nets ? pp.nets[k].s_off : 0;
     dp.n_range_parts = w->n_tiles;
     dim3 grid2(kRedBlocks / 8, pp.n_nets);
-    k_dbeta<<<grid2, kBlock, 0, st>>>(*w, pp, pl, dp, io->S_unscaled, io->R, sc.dbeta_tile, sc.dbeta_part, sc.tickets,
-                                      io->g_beta, kNoBatch);
+    if (io->venue_region)
+      k_dbeta_venue<<<grid2, kBlock, 0, st>>>(*w, pp, pl, dp, io->S_unscaled, io->R, sc.dbeta_tile, sc.dbeta_part,
+                                              sc.tickets, io->g_beta, kNoBatch, io->beta,
+                                              Venue{io->venue_region, io->venue_factor, io->n_venue_regions},
+                                              io->g_venue_factor ? io->venue_work : nullptr);
+    else
+      k_dbeta<<<grid2, kBlock, 0, st>>>(*w, pp, pl, dp, io->S_unscaled, io->R, sc.dbeta_tile, sc.dbeta_part,
+                                        sc.tickets, io->g_beta, kNoBatch);
     GJ_CHECK_LAUNCH("k_dbeta");
+    if (int e = venue_backward(w, &pp, pl, io, sc, kNoBatch, st)) return e;
   }
   return region_last ? region_backward(w, io, sc, bt, st) : 0;
 }

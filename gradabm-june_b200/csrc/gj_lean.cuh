@@ -505,14 +505,57 @@ __device__ __forceinline__ float lean_group_beta(const LeanGroupShared& sh, uint
   for (int i = 1; i < GJ_MAX_TYPES; ++i) t += (g >= sh.toff[i]) ? 1 : 0;
   return sh.bsum[t];
 }
+// regional venue factor: the generic networks of each type (ascending k, the order of lean_beta_sums) and their betas
+struct LeanVenueShared {
+  int nk[GJ_MAX_TYPES];
+  int k[GJ_MAX_TYPES][GJ_MAX_CHANNELS];
+  float beta[GJ_MAX_NETS];
+};
+__device__ __forceinline__ void lean_venue_nets(LeanVenueShared& vs, const gj_step_params& p, const Plan& pl,
+                                                const float* __restrict__ beta) {
+  if (threadIdx.x < GJ_MAX_TYPES) {
+    int n = 0;
+    for (int k = 0; k < p.n_nets; ++k)
+      if (pl.tier[k] == GJ_TIER_GENERIC && p.nets[k].type == (int)threadIdx.x && n < GJ_MAX_CHANNELS)
+        vs.k[threadIdx.x][n++] = k;
+    vs.nk[threadIdx.x] = n;
+  }
+  if (threadIdx.x < GJ_MAX_NETS) vs.beta[threadIdx.x] = (int)threadIdx.x < p.n_nets ? beta[threadIdx.x] : 0.0f;
+  // the caller's lean_beta_sums synchronises
+}
+// the value that replaces the type's beta sum for group g: sum_k beta_k * f_k[region(g)] (NaN = no active network);
+// a factor of 1 gives the beta sum bit for bit
+__device__ __forceinline__ float lean_venue_beta(const LeanGroupShared& sh, const LeanVenueShared& vs, const Venue& v,
+                                                 uint32_t g) {
+  int t = 0;
+#pragma unroll
+  for (int i = 1; i < GJ_MAX_TYPES; ++i) t += (g >= sh.toff[i]) ? 1 : 0;
+  float b = sh.bsum[t];
+  if (b == b) {
+    const int64_t r = __ldg(v.region + g);
+    b = 0.0f;
+    for (int i = 0; i < vs.nk[t]; ++i) {
+      const int k = vs.k[t][i];
+      b += vs.beta[k] * __ldg(v.factor + (int64_t)k * v.n + r);
+    }
+  }
+  return b;
+}
+template <bool kVenue>
+__device__ __forceinline__ float lean_beta_of(const LeanGroupShared& sh, const LeanVenueShared* vs, const Venue& v,
+                                              uint32_t g) {
+  return kVenue ? lean_venue_beta(sh, *vs, v, g) : lean_group_beta(sh, g);
+}
 
 // one group of <= GJ_SMALL_GROUP members per thread
+template <bool kVenue = false>
 __device__ __forceinline__ void lean_group_small_body(const gj_world_desc& w, const LeanGroupShared& gs, int64_t i,
                                                       const float* __restrict__ in, float* __restrict__ out_scaled,
-                                                      float* __restrict__ out_plain) {
+                                                      float* __restrict__ out_plain,
+                                                      const LeanVenueShared* vs = nullptr, const Venue& v = Venue{}) {
   if (i >= w.n_small) return;
   const uint32_t g = w.small_groups[i];
-  const float b = lean_group_beta(gs, g);
+  const float b = lean_beta_of<kVenue>(gs, vs, v, g);
   float S = 0.0f;
   if (b == b) {
     const uint32_t j0 = w.gm_ptr[g], j1 = w.gm_ptr[g + 1];
@@ -532,13 +575,15 @@ __device__ __forceinline__ void lean_group_small_body(const gj_world_desc& w, co
 }
 
 // one chunk of <= GJ_CHUNK members per warp
+template <bool kVenue = false>
 __device__ __forceinline__ void lean_group_chunk_body(const gj_world_desc& w, const LeanGroupShared& gs, int64_t ci,
                                                       const float* __restrict__ in, float* __restrict__ out_scaled,
-                                                      float* __restrict__ out_plain, float* __restrict__ part) {
+                                                      float* __restrict__ out_plain, float* __restrict__ part,
+                                                      const LeanVenueShared* vs = nullptr, const Venue& v = Venue{}) {
   const int lane = threadIdx.x & 31;
   if (ci >= w.n_chunks) return;
   const uint32_t g = w.chunk_group[ci];
-  const float b = lean_group_beta(gs, g);
+  const float b = lean_beta_of<kVenue>(gs, vs, v, g);
   float S = 0.0f;
   if (b == b) {
     const uint32_t j0 = w.chunk_begin[ci], j1 = w.chunk_end[ci];
@@ -594,15 +639,47 @@ __global__ void __launch_bounds__(kBlock) k_lean_group_sums(gj_world_desc w, gj_
     lean_group_small_body(w, gs, (int64_t)(bx - chunk_blocks) * blockDim.x + threadIdx.x, in, out_scaled,
                           out_plain);
 }
+// k_lean_group_sums with the regional venue factor
+__global__ void __launch_bounds__(kBlock) k_lean_group_sums_venue(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                  const float* __restrict__ beta,
+                                                                  const float* __restrict__ in,
+                                                                  float* __restrict__ out_scaled,
+                                                                  float* __restrict__ out_plain,
+                                                                  float* __restrict__ part, int chunk_blocks, Batch bt,
+                                                                  Venue v) {
+  __shared__ LeanGroupShared gs;
+  __shared__ LeanVenueShared vs;
+  pdl_launch();
+  pdl_wait();
+  uint32_t bx = blockIdx.x;
+  if (bt.nb > 1) {
+    const int s = (int)(bx % (uint32_t)bt.nb);
+    bx /= (uint32_t)bt.nb;
+    beta += (int64_t)s * bt.sBeta;
+    in += (int64_t)s * bt.sN;
+    out_scaled += (int64_t)s * bt.sG;
+    out_plain += (int64_t)s * bt.sG;
+    part = scr_shift(part, bt, s);
+    v.factor += (int64_t)s * bt.sVen;
+  }
+  lean_venue_nets(vs, p, pl, beta);
+  lean_beta_sums(gs, w, p, pl, beta);
+  if ((int)bx < chunk_blocks)
+    lean_group_chunk_body<true>(w, gs, ((int64_t)bx * blockDim.x + threadIdx.x) >> 5, in, out_scaled, out_plain, part,
+                                &vs, v);
+  else
+    lean_group_small_body<true>(w, gs, (int64_t)(bx - chunk_blocks) * blockDim.x + threadIdx.x, in, out_scaled,
+                                out_plain, &vs, v);
+}
 
 // groups spanning several chunks: one WARP per group adds the chunk partials (lanes stride over them, then the fixed
 // shuffle tree): a handful of groups, so the kernel is pure latency — a serial walk per thread measured 8.6 us
-__global__ void __launch_bounds__(kBlock) k_lean_group_fix(gj_world_desc w, gj_step_params p, Plan pl,
-                                                           const float* __restrict__ beta,
-                                                           const float* __restrict__ part,
-                                                           float* __restrict__ out_scaled,
-                                                           float* __restrict__ out_plain, Batch bt) {
-  __shared__ LeanGroupShared gs;
+template <bool kVenue>
+__device__ __forceinline__ void lean_group_fix_body(const gj_world_desc& w, const gj_step_params& p, const Plan& pl,
+                                                    const float* __restrict__ beta, const float* __restrict__ part,
+                                                    float* __restrict__ out_scaled, float* __restrict__ out_plain,
+                                                    const Batch& bt, LeanGroupShared& gs, LeanVenueShared* vs,
+                                                    Venue v) {
   pdl_launch();
   pdl_wait();
   uint32_t bx = blockIdx.x;
@@ -613,19 +690,38 @@ __global__ void __launch_bounds__(kBlock) k_lean_group_fix(gj_world_desc w, gj_s
     out_scaled += (int64_t)s * bt.sG;
     out_plain += (int64_t)s * bt.sG;
     part = scr_shift(part, bt, s);
+    if (kVenue) v.factor += (int64_t)s * bt.sVen;
   }
+  if (kVenue) lean_venue_nets(*vs, p, pl, beta);
   lean_beta_sums(gs, w, p, pl, beta);
   const int lane = threadIdx.x & 31;
   const int64_t i = ((int64_t)bx * blockDim.x + threadIdx.x) >> 5;
   if (i >= w.n_big) return;
   const uint32_t g = w.big_groups[i];
-  const float b = lean_group_beta(gs, g);
+  const float b = lean_beta_of<kVenue>(gs, vs, v, g);
   float S = 0.0f;
   for (uint32_t j = w.big_part_ptr[i] + lane; j < w.big_part_ptr[i + 1]; j += 32) S += part[j];
   S = warp_sum(S);
   if (lane != 0) return;
   out_plain[g] = S;
   out_scaled[g] = (b == b) ? (b * w.pc[g]) * S : 0.0f;
+}
+__global__ void __launch_bounds__(kBlock) k_lean_group_fix(gj_world_desc w, gj_step_params p, Plan pl,
+                                                           const float* __restrict__ beta,
+                                                           const float* __restrict__ part,
+                                                           float* __restrict__ out_scaled,
+                                                           float* __restrict__ out_plain, Batch bt) {
+  __shared__ LeanGroupShared gs;
+  lean_group_fix_body<false>(w, p, pl, beta, part, out_scaled, out_plain, bt, gs, nullptr, Venue{nullptr, nullptr, 0});
+}
+__global__ void __launch_bounds__(kBlock) k_lean_group_fix_venue(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                 const float* __restrict__ beta,
+                                                                 const float* __restrict__ part,
+                                                                 float* __restrict__ out_scaled,
+                                                                 float* __restrict__ out_plain, Batch bt, Venue v) {
+  __shared__ LeanGroupShared gs;
+  __shared__ LeanVenueShared vs;
+  lean_group_fix_body<true>(w, p, pl, beta, part, out_scaled, out_plain, bt, gs, &vs, v);
 }
 
 // the generic-tier types' global group id ranges, concatenated: thread i -> group (host-built, passed by value)
@@ -634,12 +730,13 @@ struct GenericRanges {
   int64_t first[GJ_MAX_TYPES];   // first global group id of the range
   int64_t start[GJ_MAX_TYPES + 1];   // first linear index of the range
 };
-__global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize(gj_world_desc w, gj_step_params p, Plan pl,
-                                                                  GenericRanges gr, const float* __restrict__ beta,
-                                                                  const float* __restrict__ in, Scatter sct,
-                                                                  float* __restrict__ out_scaled,
-                                                                  float* __restrict__ out_plain, Batch bt) {
-  __shared__ LeanGroupShared gs;
+template <bool kVenue>
+__device__ __forceinline__ void lean_scatter_finalize_body(const gj_world_desc& w, const gj_step_params& p,
+                                                           const Plan& pl, const GenericRanges& gr,
+                                                           const float* __restrict__ beta, const float* __restrict__ in,
+                                                           Scatter sct, float* __restrict__ out_scaled,
+                                                           float* __restrict__ out_plain, const Batch& bt,
+                                                           LeanGroupShared& gs, LeanVenueShared* vs, Venue v) {
   pdl_launch();
   pdl_wait();
   uint32_t bx = blockIdx.x;
@@ -652,7 +749,9 @@ __global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize(gj_world_desc 
     out_plain += (int64_t)s * bt.sG;
     sct.acc = scr_shift(sct.acc, bt, s);
     sct.dirty = scr_shift(sct.dirty, bt, s);
+    if (kVenue) v.factor += (int64_t)s * bt.sVen;
   }
+  if (kVenue) lean_venue_nets(*vs, p, pl, beta);
   lean_beta_sums(gs, w, p, pl, beta);
   const int64_t i = (int64_t)bx * blockDim.x + threadIdx.x;
   if (i >= gr.start[gr.n]) return;
@@ -665,7 +764,7 @@ __global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize(gj_world_desc 
   const unsigned long long acc = sct.acc[g];
   const bool dirty = sct.dirty[g] != 0;
   if (acc != 0ull) sct.acc[g] = 0ull;
-  const float b = lean_group_beta(gs, (uint32_t)g);
+  const float b = lean_beta_of<kVenue>(gs, vs, v, (uint32_t)g);
   float S = (float)((double)(long long)acc * (1.0 / (double)(1ull << GJ_SCATTER_FRAC)));
   if (dirty) {
     sct.dirty[g] = 0;
@@ -674,6 +773,26 @@ __global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize(gj_world_desc 
   }
   out_plain[g] = S;
   out_scaled[g] = (b == b) ? (b * w.pc[g]) * S : 0.0f;
+}
+__global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                  GenericRanges gr, const float* __restrict__ beta,
+                                                                  const float* __restrict__ in, Scatter sct,
+                                                                  float* __restrict__ out_scaled,
+                                                                  float* __restrict__ out_plain, Batch bt) {
+  __shared__ LeanGroupShared gs;
+  lean_scatter_finalize_body<false>(w, p, pl, gr, beta, in, sct, out_scaled, out_plain, bt, gs, nullptr,
+                                    Venue{nullptr, nullptr, 0});
+}
+__global__ void __launch_bounds__(kBlock) k_lean_scatter_finalize_venue(gj_world_desc w, gj_step_params p, Plan pl,
+                                                                        GenericRanges gr,
+                                                                        const float* __restrict__ beta,
+                                                                        const float* __restrict__ in, Scatter sct,
+                                                                        float* __restrict__ out_scaled,
+                                                                        float* __restrict__ out_plain, Batch bt,
+                                                                        Venue v) {
+  __shared__ LeanGroupShared gs;
+  __shared__ LeanVenueShared vs;
+  lean_scatter_finalize_body<true>(w, p, pl, gr, beta, in, sct, out_scaled, out_plain, bt, gs, &vs, v);
 }
 
 // per-agent arithmetic of the forward pass, shared by the register-batched kernel below and the bulk-copy pipelined

@@ -45,7 +45,18 @@ struct Batch {
   const float* noise;  // [n_agents] the draw's Gumbel noise difference, evaluated once for all samples; NULL = in-kernel
   int64_t sLab;        // stride of red_label / g_red_label / label_acc (elements)
   int64_t sReg;        // stride of region_factor / g_region_factor (elements, >= n_regions: a row per sample)
+  int64_t sVen;        // stride of venue_factor / g_venue_factor (elements, >= n_nets * n: a table per sample)
 };
+// regional venue factor of a step (gj_fwd_io / gj_bwd_io venue_*): network k's beta is multiplied by
+// factor[k * n + region[g]] wherever group g's beta * pc is formed
+struct Venue {
+  const int32_t* region;   // [n_groups] by global group id
+  const float* factor;     // [n_nets][n]
+  int n;
+};
+__device__ __forceinline__ float venue_factor(const Venue& v, int k, uint32_t g) {
+  return __ldg(v.factor + (int64_t)k * v.n + __ldg(v.region + g));
+}
 struct BatchCta {
   int s;           // sample of this CTA
   uint32_t bx, gx; // its block index among the sample's CTAs, and how many those are
@@ -207,11 +218,12 @@ __global__ void __launch_bounds__(kBlock) k_tile_transmission(gj_world_desc w, g
 // cell tier: tiles -> cells -> groups, and groups -> cells
 // =====================================================================================================
 // one thread per (cell channel, group): sum the tile partials of the group's cells in ascending order
-__global__ void __launch_bounds__(kBlock) k_cell_groups(gj_world_desc w, gj_step_params p, Plan pl,
-                                                        const float* __restrict__ beta,
-                                                        const float* __restrict__ tile_part,
-                                                        float* __restrict__ out_scaled, float* __restrict__ out_plain,
-                                                        Batch bt) {
+// kVenue: the group's beta is multiplied by its region's venue factor first
+template <bool kVenue>
+__device__ __forceinline__ void cell_groups_body(const gj_world_desc& w, const gj_step_params& p, const Plan& pl,
+                                                 const float* __restrict__ beta, const float* __restrict__ tile_part,
+                                                 float* __restrict__ out_scaled, float* __restrict__ out_plain,
+                                                 const Batch& bt, Venue v) {
   pdl_launch();
   pdl_wait();
   if (bt.nb > 1) {   // batched ensemble: sample blockIdx.z
@@ -220,6 +232,7 @@ __global__ void __launch_bounds__(kBlock) k_cell_groups(gj_world_desc w, gj_step
     tile_part = scr_shift(tile_part, bt, s);
     out_scaled += (int64_t)s * bt.sG;
     out_plain += (int64_t)s * bt.sG;
+    if (kVenue) v.factor += (int64_t)s * bt.sVen;
   }
   const int j = blockIdx.y;
   const int k = pl.t2_net[j];
@@ -234,9 +247,24 @@ __global__ void __launch_bounds__(kBlock) k_cell_groups(gj_world_desc w, gj_step
     for (uint32_t tl = w.cell_tile_ptr[t][c]; tl < w.cell_tile_ptr[t][c + 1]; ++tl)
       sum += tile_part[(int64_t)tl * GJ_MAX_CHANNELS + j];
   }
-  const float cg = beta[k] * w.pc[w.type_group_off[t] + g];
+  const int64_t gg = w.type_group_off[t] + g;
+  const float cg = kVenue ? (beta[k] * venue_factor(v, k, (uint32_t)gg)) * w.pc[gg] : beta[k] * w.pc[gg];
   out_plain[(int64_t)net.s_off + g] = sum;
   out_scaled[(int64_t)net.s_off + g] = cg * sum;
+}
+__global__ void __launch_bounds__(kBlock) k_cell_groups(gj_world_desc w, gj_step_params p, Plan pl,
+                                                        const float* __restrict__ beta,
+                                                        const float* __restrict__ tile_part,
+                                                        float* __restrict__ out_scaled, float* __restrict__ out_plain,
+                                                        Batch bt) {
+  cell_groups_body<false>(w, p, pl, beta, tile_part, out_scaled, out_plain, bt, Venue{nullptr, nullptr, 0});
+}
+__global__ void __launch_bounds__(kBlock) k_cell_groups_venue(gj_world_desc w, gj_step_params p, Plan pl,
+                                                              const float* __restrict__ beta,
+                                                              const float* __restrict__ tile_part,
+                                                              float* __restrict__ out_scaled,
+                                                              float* __restrict__ out_plain, Batch bt, Venue v) {
+  cell_groups_body<true>(w, p, pl, beta, tile_part, out_scaled, out_plain, bt, v);
 }
 
 // one thread per (cell channel, cell): sum over the cell's groups (agent edge order)

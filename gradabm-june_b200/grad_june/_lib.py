@@ -18,7 +18,7 @@ GJ_MAX_STAGES = 16
 GJ_MAX_QUAR = 4
 GJ_MAX_AGE_BINS = 8
 GJ_MAX_CHANNELS = 8
-GJ_ABI_VERSION = 13
+GJ_ABI_VERSION = 14
 
 KIND_PLAIN, KIND_HOUSEHOLD, KIND_LEISURE, KIND_CARE_VISIT = 0, 1, 2, 3
 PHASE_NETWORKS, PHASE_SAMPLE, PHASE_INFECT, PHASE_SYMPTOMS, PHASE_ALL = 1, 2, 4, 8, 15
@@ -110,7 +110,10 @@ class FwdIO(C.Structure):
         # seeding by label: region codes and their count
         ("seed_label", C.c_void_p), ("n_seed_labels", C.c_int32), ("_pad_seed", C.c_int32),
         # regional transmission factor: region codes, their count, the factor per region
-        ("region", C.c_void_p), ("n_regions", C.c_int32), ("_pad_region", C.c_int32), ("region_factor", C.c_void_p)]
+        ("region", C.c_void_p), ("n_regions", C.c_int32), ("_pad_region", C.c_int32), ("region_factor", C.c_void_p),
+        # regional venue factor: region of every group, their count, the factor table [n_nets][n]
+        ("venue_region", C.c_void_p), ("n_venue_regions", C.c_int32), ("_pad_venue", C.c_int32),
+        ("venue_factor", C.c_void_p)]
 
 
 class BwdIO(C.Structure):
@@ -119,7 +122,10 @@ class BwdIO(C.Structure):
         ("seed_offsets", C.c_void_p), ("seed_work", C.c_void_p)] + [
         ("region", C.c_void_p), ("n_regions", C.c_int32), ("_pad_region", C.c_int32), ("region_factor", C.c_void_p),
         ("region_order", C.c_void_p), ("region_offsets", C.c_void_p), ("region_work", C.c_void_p),
-        ("g_region_factor", C.c_void_p)]
+        ("g_region_factor", C.c_void_p)] + [
+        ("venue_region", C.c_void_p), ("n_venue_regions", C.c_int32), ("_pad_venue", C.c_int32),
+        ("venue_factor", C.c_void_p), ("venue_order", C.c_void_p), ("venue_offsets", C.c_void_p),
+        ("venue_work", C.c_void_p), ("g_venue_factor", C.c_void_p)]
 
 
 class Batch(C.Structure):
@@ -127,7 +133,7 @@ class Batch(C.Structure):
     _fields_ = [("n_samples", C.c_int32), ("_pad0", C.c_int32), ("agent_stride", C.c_int64),
                 ("group_stride", C.c_int64), ("beta_stride", C.c_int64), ("red_stride", C.c_int64),
                 ("scratch_stride", C.c_int64), ("noise", C.c_void_p), ("label_stride", C.c_int64),
-                ("region_stride", C.c_int64)]
+                ("region_stride", C.c_int64), ("venue_stride", C.c_int64)]
 
 
 class GradJuneLibraryError(RuntimeError):

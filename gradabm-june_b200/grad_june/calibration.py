@@ -90,23 +90,26 @@ class Calibrator:
         cal = Calibrator(runner, loss_fn=lambda r: ((r["cases_per_timestep"] - target) ** 2).mean())
         history = cal.fit(50)              # pandas DataFrame: iteration, loss, log_beta_<network>..., grad_<network>...
                                            # (fit_seed=True: also log_fraction_<label>..., grad_log_fraction_<label>...;
-                                           #  fit_regional=True: log_factor_<policy>_<label>..., grad_log_factor_...)
+                                           #  fit_regional=True: log_factor_<policy>_<label>..., grad_log_factor_...;
+                                           #  fit_venue=True: log_venue_factor_<policy>_<key>_<label>..., grad_...)
         cal.save(history)                  # <save_path>/calibration.csv + the reference's results.csv of the last run
     """
 
     def __init__(self, runner, loss_fn: Callable[[dict], torch.Tensor], networks: Optional[Sequence[str]] = None,
                  lr: float = 0.05, optimizer: str = "adam", seed: int = 0, reseed_every: int = 0, fit_seed: bool = False,
-                 fit_regional: bool = False):
+                 fit_regional: bool = False, fit_venue: bool = False):
         """``fit_seed=True`` also calibrates the initial-case log-fractions (one national value, or one per region of
         ``runner.seed_labels``): they sit after the log-betas in the parameter vector.  ``fit_regional=True`` also
         calibrates the log10 of every regional policy's factors (R per policy, ``runner.region_labels`` order), after
-        those."""
+        those.  ``fit_venue=True`` also calibrates the log10 of every venue policy entry's factors (R per entry,
+        ``runner.venue_labels`` order), after the regional ones."""
         self.runner = runner
         self.graphed = GraphedRunner(runner, loss_fn, networks=networks, seed=seed, fit_seed=fit_seed,
-                                     fit_regional=fit_regional)
+                                     fit_regional=fit_regional, fit_venue=fit_venue)
         self.names = self.graphed.names
         self.seed_names = self.graphed.seed_names
         self.regional_names = self.graphed.regional_names
+        self.venue_names = self.graphed.venue_names
         dev = self.graphed.device
         self.log_beta = self.graphed.log_beta.detach().clone().requires_grad_(True)
         opt = {"adam": torch.optim.Adam, "sgd": torch.optim.SGD}[optimizer.lower()]
@@ -141,6 +144,9 @@ class Calibrator:
             S = K + len(self.seed_names)
             row.update({f"log_factor_{k}": v for k, v in zip(self.regional_names, lb[S:])})
             row.update({f"grad_log_factor_{k}": v for k, v in zip(self.regional_names, grads[S:])})
+            V = S + len(self.regional_names)
+            row.update({f"log_venue_factor_{k}": v for k, v in zip(self.venue_names, lb[V:])})
+            row.update({f"grad_log_venue_factor_{k}": v for k, v in zip(self.venue_names, grads[V:])})
             rows.append(row)
             if callback is not None:
                 callback(row)

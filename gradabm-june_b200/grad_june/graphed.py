@@ -18,6 +18,10 @@ factors, R values per policy (``runner.region_labels`` order) in the order the p
 log-betas and the seeding values; a factor of 0 has no log10 and is rejected.  Regional factors that are not fitted
 are constants of the graph, used through a device copy made at construction; the policies themselves are not changed.
 
+``fit_venue=True`` calibrates the regional venue policies the same way: the log10 of every
+``RegionalVenueDistancing`` entry's factors, R values (``runner.venue_labels`` order) per (policy, entry) in the order
+the policies and their entries were given, after the regional factors.
+
 Noise: the Philox key and call indices are kernel arguments, so every replay draws the SAME noise (common random
 numbers across parameter samples — the usual variance reduction for calibration gradients); ``recapture(seed)``
 re-records the graph with another key.
@@ -41,8 +45,9 @@ from . import ops
 class GraphedRunner:
     def __init__(self, runner, loss_fn: Callable[[dict], torch.Tensor], networks: Optional[Sequence[str]] = None,
                  seed: int = 0, warmup: int = 1, batch: Optional[int] = None, fit_seed: bool = False,
-                 fit_regional: bool = False):
+                 fit_regional: bool = False, fit_venue: bool = False):
         self.runner = runner
+        self.fit_venue = bool(fit_venue)
         self.fit_seed = bool(fit_seed)
         self.fit_regional = bool(fit_regional)
         self.loss_fn = loss_fn
@@ -86,6 +91,27 @@ class GraphedRunner:
         # iteration swaps the values in and restores the originals afterwards.
         self._fixed_factors = [pol.beta_factors.detach().to(device=self.device, dtype=torch.float32)
                                if torch.is_tensor(pol.beta_factors) else None for pol in self.regional]
+        self.n_regional = len(init) - self.n_beta - self.n_seed
+        vp = getattr(runner.model.policies, "venue_policies", None)
+        self.venue = list(vp.policies) if (vp is not None and runner.venue_by is not None) else []
+        self.venue_names = []
+        if self.fit_venue:   # log10 of each venue policy entry's factors, R per (policy, entry), after the regional ones
+            if not self.venue:
+                raise ValueError("fit_venue=True needs at least one regional venue policy")
+            labels = runner.venue_labels
+            for i, pol in enumerate(self.venue):
+                for key in pol.beta_factors:
+                    f = pol.factors(key, labels, "cpu").detach().reshape(-1, len(labels))[0]
+                    if not bool((f > 0).all()):
+                        zero = labels[int(torch.nonzero(f <= 0)[0])]
+                        raise ValueError(f"fit_venue=True fits log10 of the factors: venue policy {i} ({key}) has "
+                                         f"factor {float(f[f <= 0][0])} for region {zero!r}; start the fit from a "
+                                         "factor > 0")
+                    init += [float(v) for v in torch.log10(f.double())]
+                    self.venue_names += [f"{i}_{key}_{v}" for v in labels]
+        # venue entries that are not fitted: tensors through a device copy, like the regional factors
+        self._fixed_venue = [{k: v.detach().to(device=self.device, dtype=torch.float32)
+                              for k, v in pol.beta_factors.items() if torch.is_tensor(v)} for pol in self.venue]
         self.log_beta = torch.tensor(init, dtype=torch.float32).to(self.device)
         if self.batch:
             self.log_beta = self.log_beta.repeat(self.batch, 1)          # [b, K]
@@ -129,12 +155,26 @@ class GraphedRunner:
                 continue
             pol._parameters.pop("beta_factors", None)   # an nn.Parameter is unregistered first, like log_beta
             pol.beta_factors = value
+        venue_originals = [pol.beta_factors for pol in self.venue]
+        R = len(self.runner.venue_labels) if self.venue else 0
+        off = self.n_beta + self.n_seed + self.n_regional
+        for i, pol in enumerate(self.venue):
+            swapped = dict(pol.beta_factors)
+            for key in pol.beta_factors:
+                if self.fit_venue:
+                    swapped[key] = 10.0 ** (self.log_beta[:, off:off + R] if self.batch else self.log_beta[off:off + R])
+                    off += R
+                elif key in self._fixed_venue[i]:
+                    swapped[key] = self._fixed_venue[i][key]
+            pol.beta_factors = swapped
         try:
             with ops.philox_seed(self.seed):
                 results, is_infected = self.runner()
         finally:
             for pol, value in zip(self.regional, originals):
                 pol._parameters.pop("beta_factors", None)
+                pol.beta_factors = value
+            for pol, value in zip(self.venue, venue_originals):
                 pol.beta_factors = value
         loss = self.loss_fn(results)
         if self.batch and tuple(loss.shape) != (self.batch,):
@@ -181,7 +221,8 @@ class GraphedRunner:
     @torch.no_grad()
     def __call__(self, log_beta: Optional[torch.Tensor] = None):
         """Replay with ``log_beta`` ([K], or [b, K] for a batched window; [K + R] / [b, K + R] with ``fit_seed``, the
-        log-fractions after the log-betas; then, with ``fit_regional``, R log10-factors per regional policy; any device;
+        log-fractions after the log-betas; then, with ``fit_regional``, R log10-factors per regional policy, and with
+        ``fit_venue`` R log10-factors per venue policy entry; any device;
         None = keep).  Returns (loss, d loss / d log_beta, results): static device
         tensors that the next replay overwrites."""
         if log_beta is not None:

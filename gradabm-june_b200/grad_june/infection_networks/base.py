@@ -84,7 +84,7 @@ class InfectionNetwork(torch.nn.Module):
                 return True
         return False
 
-    def _custom_pressure(self, data, timer, policies):
+    def _custom_pressure(self, data, timer, policies, venue=None):
         """base.py:61-84 with the hooks' own tensors: C_g = sum of T'_a * beta_eff * pc_g over the members, P_a = C_g(a)
         * s'_a, through the stand-alone NETWORKS phase with no built-in mask (differentiable with respect to T', s'
         and beta_eff)."""
@@ -100,14 +100,15 @@ class InfectionNetwork(torch.nn.Module):
 
         static = ops.StepStatic(world=world, exchange=exchange_for(data, world))
         beta = self.beta_eff(policies, timer).reshape(1).to(device=dev, dtype=torch.float32)
-        out = ops.infection_step(static, spec, beta, {"s": ops._f32(sm, dev)}, T_in=ops._f32(Tm, dev))
+        out = ops.infection_step(static, spec, beta, {"s": ops._f32(sm, dev)}, T_in=ops._f32(Tm, dev), venue=venue)
         return out["lam"]
 
-    def forward(self, data, timer, policies):
-        """Pressure this network alone exerts on every agent (the reference's per-network output)."""
+    def forward(self, data, timer, policies, venue=None):
+        """Pressure this network alone exerts on every agent (the reference's per-network output).  ``venue``
+        (:class:`grad_june.ops.Venue` of one row): the regional venue factor of this network's groups."""
         if self.is_custom():
-            return self._custom_pressure(data, timer, policies)
-        out = _run_networks([self], data, timer, policies, self.device, want_lam=True)
+            return self._custom_pressure(data, timer, policies, venue)
+        out = _run_networks([self], data, timer, policies, self.device, want_lam=True, venue=venue)
         return out["lam"]
 
 
@@ -178,7 +179,7 @@ def beta_vector(networks, policies, timer, device):
                         for net in networks])
 
 
-def _run_networks(networks, data, timer, policies, device, want_lam=False, region=None):
+def _run_networks(networks, data, timer, policies, device, want_lam=False, region=None, venue=None):
     agent = data["agent"]
     ops.require_cuda(agent.susceptibility, "data['agent'].susceptibility")
     dev = agent.susceptibility.device
@@ -196,7 +197,7 @@ def _run_networks(networks, data, timer, policies, device, want_lam=False, regio
 
     static = ops.StepStatic(world=world, leisure_prob=table, exchange=exchange_for(data, world))
     return ops.infection_step(static, spec, beta_vector(networks, policies, timer, dev), state,
-                              T_in=agent.transmission, region=region)
+                              T_in=agent.transmission, region=region, venue=venue)
 
 
 class InfectionNetworks(torch.nn.Module):
@@ -235,19 +236,21 @@ class InfectionNetworks(torch.nn.Module):
     def has_custom(self, nets=None):
         return any(net.is_custom() for net in (self.networks.values() if nets is None else nets))
 
-    def forward(self, data, timer, policies, region=None):
+    def forward(self, data, timer, policies, region=None, venue=None):
         """not_infected_probs of the step.  ``region`` (:class:`grad_june.ops.Region`): every agent's summed pressure is
-        multiplied by its region's factor before the clamp (the regional policies active at this step)."""
+        multiplied by its region's factor before the clamp (the regional policies active at this step).  ``venue``
+        (:class:`grad_june.ops.Venue`): the regional venue factors of the step's networks, row k for the k-th."""
         policies.apply(timer=timer, data=data)
         nets = self.active_networks(timer, policies)
         if not self.has_custom(nets):
-            return _run_networks(nets, data, timer, policies, self.device, region=region)["q"]
+            return _run_networks(nets, data, timer, policies, self.device, region=region, venue=venue)["q"]
         # a user-defined network among them: network by network in the activity order, then the reference's clamp /
         # exp chain (base.py:133-140) in torch
         agent = data["agent"]
         lam = torch.zeros_like(agent.susceptibility)
-        for net in nets:
-            lam = lam + net(data=data, timer=timer, policies=policies)
+        for k, net in enumerate(nets):
+            kw = {} if venue is None else {"venue": venue.row(k)}
+            lam = lam + net(data=data, timer=timer, policies=policies, **kw)
         if region is not None:
             lam = lam * region.factor.to(lam.device)[region.labels.codes.long()]
         lam = torch.clamp(lam, min=1e-6, max=100)

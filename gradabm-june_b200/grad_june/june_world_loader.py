@@ -105,6 +105,9 @@ def world_from_june_arrays(f: Mapping, k_leisure: int = 3, load_leisure: bool = 
         data["agent", "attends_leisure", "leisure"].edge_index = torch.from_numpy(np.vstack((person, group)))
         data["leisure"].id = torch.from_numpy(sa_ids.astype(np.int64))
         data["leisure"].people = torch.from_numpy(people)
+        # a leisure group IS a super-area (its region for regional venue policies; a majority over the k-nearest
+        # attendees could name a neighbour instead)
+        data["leisure"].super_area = torch.from_numpy(sa_ids.astype(np.int64))
     data = ToUndirected()(data)
     # agent attributes (agent_data_loader.py:20-33)
     agent = data["agent"]

@@ -91,7 +91,7 @@ class GradJune(torch.nn.Module):
         return spec, nets
 
     def step(self, data, timer, age_bins=None, mode=ops.MODE_STEP, seed_fraction=None, noise=None, want_probs=True,
-             next_timer=None, label=None, seed_label=None, region=None):
+             next_timer=None, label=None, seed_label=None, region=None, venue=None):
         """Fused step; returns (data, reductions) where reductions = [cases, deaths, cases by age bin...]
         (None unless ``age_bins`` is given).  With ``label`` (:class:`grad_june.ops.Labels`) it returns
         (data, reductions, label_table): the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched),
@@ -103,21 +103,30 @@ class GradJune(torch.nn.Module):
         step and the agents' region codes (``Runner`` builds it); every agent's force of infection is multiplied by its
         region's factor before the clamp.  A step with an active regional policy and no ``region`` raises; the
         seeding step has no networks and ignores it.
+        ``venue`` (:class:`grad_june.ops.Venue`): the regional venue factor table of the step's networks (step order)
+        and the groups' region codes (``Runner`` builds it); network k's beta at group g is multiplied by its factor of
+        g's region.  A step where an active venue policy has an entry for one of its networks and no ``venue`` raises.
         ``next_timer``: the timer as it will be at the FOLLOWING call (the driver knows the schedule): the
         kernels then run that step's transmission pass inside this one (used only if the next call matches)."""
         agent = data["agent"]
         if mode != ops.MODE_STEP:
-            region = None
+            region = venue = None
         else:
             rp = self.policies.regional_policies
             if region is None and rp is not None and rp.active(timer):
                 raise ValueError(f"a regional policy is active on {timer.date}: GradJune.step needs its region factors "
                                  "(region=ops.Region(...), built by Runner)")
+            vp = getattr(self.policies, "venue_policies", None)
+            if venue is None and vp is not None and vp.active(timer):
+                names = [net.name for net in self.infection_networks.active_networks(timer, self.policies)]
+                if any(pol.entry(n) is not None for pol in vp.active(timer) for n in names):
+                    raise ValueError(f"a regional venue policy is active on {timer.date}: GradJune.step needs its "
+                                     "factor table (venue=ops.Venue(...), built by Runner)")
         ops.require_cuda(agent.susceptibility, "data['agent'].susceptibility")
         dev = agent.susceptibility.device
         if mode == ops.MODE_STEP and self.infection_networks.has_custom(
                 self.infection_networks.active_networks(timer, self.policies)):
-            return self._step_modular(data, timer, age_bins, label, region)
+            return self._step_modular(data, timer, age_bins, label, region, venue)
         static, rows = self._static(data, dev)
         policies = self.policies
         spec, nets = self._spec(timer, rows, age_bins, mode, want_probs)
@@ -129,7 +138,8 @@ class GradJune(torch.nn.Module):
                  "cur": sym["current_stage"], "nxt": sym["next_stage"], "ttn": sym["time_to_next_stage"]}
         beta = beta_vector(nets, policies, timer, dev) if nets else None
         out = ops.infection_step(static, spec, beta, state, seed_fraction=seed_fraction, noise=noise,
-                                 next_spec=next_spec, label=label, seed_label=seed_label, region=region)
+                                 next_spec=next_spec, label=label, seed_label=seed_label, region=region,
+                                 venue=venue)
         if out["T"] is not None:
             agent.transmission = out["T"]
         agent.susceptibility = out["s"]
@@ -146,13 +156,13 @@ class GradJune(torch.nn.Module):
             return data, out["red"], out["red_label"]
         return data, out["red"]
 
-    def _step_modular(self, data, timer, age_bins, label=None, region=None):
+    def _step_modular(self, data, timer, age_bins, label=None, region=None, venue=None):
         """The reference's own sequencing (model.py:112-144), module by module, for steps with a user-defined network
         subclass (its masking hooks return arbitrary tensors, which the fused kernels cannot evaluate in registers):
         every module is still a CUDA kernel of the library (stand-alone phases), only the fusion is lost."""
         agent = data["agent"]
         agent.transmission = self.transmission_updater(data=data, timer=timer)
-        q = self.infection_networks(data=data, timer=timer, policies=self.policies, region=region)
+        q = self.infection_networks(data=data, timer=timer, policies=self.policies, region=region, venue=venue)
         n = self.is_infected_sampler(q)
         self.infect_people(data, timer, n)
         self.symptoms_updater(data=data, timer=timer, new_infected=n)

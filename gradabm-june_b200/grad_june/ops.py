@@ -268,6 +268,73 @@ def _region_factor(region: Region, dev, nb: int = 0):
     return f.contiguous()
 
 
+@dataclass(frozen=True)
+class VenueLabels:
+    """Region codes of the GROUPS (venues) of a world: ``codes[g]`` in ``[0, n)`` is the region of global group g (the
+    group's location).  For the backward's deterministic per-region reduction, ``order`` holds every edge type's groups
+    (indices within the type) stably sorted by region at the type's positions ``[type_group_off[t],
+    type_group_off[t + 1])``, and ``offsets[t * (n + 1) + r]`` is where region r starts in that part.  Build it with
+    :func:`make_venue_labels`."""
+    codes: torch.Tensor     # [n_groups] int32
+    n: int
+    order: torch.Tensor     # [n_groups] int32
+    offsets: torch.Tensor   # [n_types * (n + 1)] int32
+
+
+def make_venue_labels(codes, n: int, type_group_off: Sequence[int], device=None) -> VenueLabels:
+    """Validated :class:`VenueLabels` from the per-group codes (global group ids, types concatenated as in
+    ``type_group_off``): :func:`make_seed_labels` over the groups of each type."""
+    lab = make_labels(codes, n, device)
+    if lab.codes.numel() != type_group_off[-1]:
+        raise ValueError(f"venue region codes must hold one entry per group ({type_group_off[-1]}), "
+                         f"got {lab.codes.numel()}")
+    orders, offsets = [], []
+    for t in range(len(type_group_off) - 1):
+        sl = make_seed_labels(lab.codes[type_group_off[t]:type_group_off[t + 1]], lab.n)
+        orders.append(sl.order)
+        offsets.append(sl.offsets)
+    order = torch.cat(orders) if orders else torch.zeros(0, dtype=torch.int32, device=lab.codes.device)
+    return VenueLabels(lab.codes, lab.n, order.contiguous(), torch.cat(offsets).contiguous())
+
+
+@dataclass(frozen=True)
+class Venue:
+    """Regional venue factor of one step: network k's beta is multiplied by ``factor[k, labels.codes[g]]`` wherever
+    group g's ``beta * pc`` is formed (the group passes, the cell tier and d/dbeta), so a factor of 0 closes network k's
+    venues in that region.  Row k belongs to the step's k-th network (``StepSpec.nets``); ``factor`` is [K, n]
+    ([K, n] or [b, K, n] batched), differentiable."""
+    labels: VenueLabels
+    factor: torch.Tensor
+
+    def row(self, k: int) -> "Venue":
+        """The venue factor of the step's k-th network alone (a one-network call of the same step)."""
+        return Venue(self.labels, self.factor[..., k:k + 1, :])
+
+
+def _venue_factor(labels: VenueLabels, factor, K: int, dev, nb: int = 0):
+    """The factor table as a contiguous fp32 tensor on ``dev``: [K, n], or [nb, K, n] for a batch of ``nb``."""
+    f = _f32(factor, dev)
+    n = labels.n
+    if nb:
+        if tuple(f.shape) not in ((K, n), (nb, K, n)):
+            raise ValueError(f"a venue factor table must hold {K} x {n} values (network x region) or {nb} x {K} x {n}, "
+                             f"got {tuple(f.shape)}")
+        return f.expand(nb, K, n).contiguous()
+    if tuple(f.shape) != (K, n):
+        raise ValueError(f"a venue factor table must hold {K} x {n} values (network x region), got {tuple(f.shape)}")
+    return f.contiguous()
+
+
+def _set_venue(io, world: DeviceWorld, labels: VenueLabels, factor):
+    """Point the io struct at the group region codes and the factor table (and, on the backward's struct, at the
+    reduction's order and offsets)."""
+    if labels.codes.numel() != world.n_groups or labels.codes.device != world.device:
+        raise ValueError(f"venue region codes must hold one entry per group ({world.n_groups}) on {world.device}")
+    io.venue_region, io.n_venue_regions, io.venue_factor = labels.codes.data_ptr(), labels.n, factor.data_ptr()
+    if hasattr(io, "venue_order"):
+        io.venue_order, io.venue_offsets = labels.order.data_ptr(), labels.offsets.data_ptr()
+
+
 def _label_acc(world: DeviceWorld, n: int):
     """The integer accumulator of the label table ([n] uint32, zero; every call leaves it zero)."""
     t = world.__dict__.get("_label_acc")
@@ -521,7 +588,8 @@ class _Step(torch.autograd.Function):
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in,
                 seed_fraction, next_spec=None, label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None,
-                region_labels: Optional[SeedLabels] = None, region_factor=None):
+                region_labels: Optional[SeedLabels] = None, region_factor=None,
+                venue_labels: Optional[VenueLabels] = None, venue_factor=None):
         world = static.world
         dev = world.device
         N = world.n_agents
@@ -551,6 +619,13 @@ class _Step(torch.autograd.Function):
             _set_region(io, world, region_labels, region_factor)
         else:
             region_factor = None
+        venue_labels = venue_labels if nets_on else None
+        if venue_labels is not None:
+            venue_factor = _venue_factor(venue_labels, venue_factor, p.n_nets, dev)
+            keep.append(venue_factor)
+            _set_venue(io, world, venue_labels, venue_factor)
+        else:
+            venue_factor = None
         put("leisure_prob", static.leisure_prob)
         if static.symptoms is not None:
             put("stage_prob", static.symptoms.stage_prob)
@@ -649,11 +724,12 @@ class _Step(torch.autograd.Function):
                 cur=out.get("cur_o"))
 
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
-        ctx.seed_label, ctx.region_labels = seed_label, region_labels
+        ctx.seed_label, ctx.region_labels, ctx.venue_labels = seed_label, region_labels, venue_labels
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"],
                               T_in if T_in is not None else T, q_in, n_in,
-                              seed_fraction, out.get("inf_o"), tape_v, tape_y0, S_un, E, u, z, q, n, region_factor)
+                              seed_fraction, out.get("inf_o"), tape_v, tape_y0, S_un, E, u, z, q, n, region_factor,
+                              venue_factor)
         ctx.fused_T = fused_T
         outs = (out.get("s_o"), out.get("inf_o"), out.get("tinf_o"), out.get("cur_o"), out.get("nxt_o"),
                 out.get("ttn_o"), T, q, n, red, lam, red_label)
@@ -671,7 +747,7 @@ class _Step(torch.autograd.Function):
         world = static.world
         dev, N = world.device, world.n_agents
         (beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, seed_fraction, inf_o, tape_v, tape_y0, S_un, E, u, z,
-         q_saved, n_saved, region_factor) = ctx.saved_tensors
+         q_saved, n_saved, region_factor, venue_factor) = ctx.saved_tensors
         seed, call_index = ctx.noise_key
         p, s_total = _fill_params(world, spec, static.symptoms, seed, call_index)
         phases, seed_mode = spec.phases, spec.mode == MODE_SEED
@@ -716,7 +792,8 @@ class _Step(torch.autograd.Function):
             io.label = ctx.label.codes.data_ptr()
 
         need = ctx.needs_input_grad  # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, T_in, q_in, n_in, frac,
-        #                                next_spec, label, seed_label, region_labels, region_factor)
+        #                                next_spec, label, seed_label, region_labels, region_factor, venue_labels,
+        #                                venue_factor)
         g_region = None
         if ctx.region_labels is not None:   # the per-agent terms always; their per-region sums when wanted
             _set_region(io, world, ctx.region_labels, region_factor)
@@ -757,6 +834,13 @@ class _Step(torch.autograd.Function):
             io.wq = _buffer(world, "wq", N).data_ptr() if p.n_quar > 0 else io.w
             R_buf, cR_buf = _buffer(world, "R", s_total), _buffer(world, "cR", s_total)
             io.R, io.cR = R_buf.data_ptr(), cR_buf.data_ptr()
+        g_venue = None
+        if ctx.venue_labels is not None:   # the group passes always; the per-region gradient when wanted
+            _set_venue(io, world, ctx.venue_labels, venue_factor)
+            if need[20]:
+                g_venue = torch.empty(p.n_nets, ctx.venue_labels.n, dtype=torch.float32, device=dev)
+                io.g_venue_factor = g_venue.data_ptr()
+                io.venue_work = _buffer(world, "venue_work", s_total).data_ptr()
         io.scratch = _scratch(world).data_ptr()
         desc = world.desc()
         if static.exchange is not None:
@@ -772,7 +856,7 @@ class _Step(torch.autograd.Function):
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
                 g_T_in if need[10] else None, g_q_in, g_n_in, g_frac if need[13] else None, None, None, None, None,
-                g_region)
+                g_region, None, g_venue)
 
 
 # --------------------------------------------------------------------------------------
@@ -820,7 +904,8 @@ class _BatchStep(torch.autograd.Function):
     @staticmethod
     def forward(ctx, static: StepStatic, spec: StepSpec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction,
                 label: Optional[Labels] = None, seed_label: Optional[SeedLabels] = None,
-                region_labels: Optional[SeedLabels] = None, region_factor=None):
+                region_labels: Optional[SeedLabels] = None, region_factor=None,
+                venue_labels: Optional[VenueLabels] = None, venue_factor=None):
         world = static.world
         dev, N = world.device, world.n_agents
         L = _lib.lib()
@@ -881,13 +966,19 @@ class _BatchStep(torch.autograd.Function):
         if not seed_mode:
             seed_label = None
         if seed_mode:
-            region_labels = None
+            region_labels = venue_labels = None
         rf, n_reg = None, 0
         if region_labels is not None:   # [b, R]: every sample its own row of factors
             rf = _region_factor(Region(region_labels, region_factor), dev, nb)
             keep.append(rf)
             _set_region(io, world, region_labels, rf)
             n_reg = region_labels.n
+        vf, n_ven = None, 0
+        if venue_labels is not None:    # [b, K, R]: every sample its own table of factors
+            vf = _venue_factor(venue_labels, venue_factor, p.n_nets, dev, nb)
+            keep.append(vf)
+            _set_venue(io, world, venue_labels, vf)
+            n_ven = p.n_nets * venue_labels.n
         if seed_mode:
             seed_fraction = put("seed_fraction", seed_fraction)
             R = 1
@@ -917,17 +1008,20 @@ class _BatchStep(torch.autograd.Function):
             # the samples share the Philox stream: the draw's Gumbel noise is evaluated once per agent
             noise_buf = _buffer(world, "noise_b", Np) if BATCH_SHARED_NOISE else None
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride, noise=_ptr(noise_buf), label_stride=n_lab, region_stride=n_reg)
+                            scratch_stride=scr_stride, noise=_ptr(noise_buf), label_stride=n_lab, region_stride=n_reg,
+                            venue_stride=n_ven)
             with _on(dev):
                 _lib.check(L.gj_step_forward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_forward_batch")
         ctx.static, ctx.spec, ctx.noise_key, ctx.label = static, spec, (seed, call_index), label
         ctx.seed_label, ctx.region_labels = seed_label, region_labels
         ctx.region_shape = tuple(region_factor.shape) if region_labels is not None else None
+        ctx.venue_labels = venue_labels
+        ctx.venue_shape = tuple(venue_factor.shape) if venue_labels is not None else None
         ctx.shape = (nb, Np, sG, K, nr)
         ctx.set_materialize_grads(False)
         ctx.save_for_backward(beta, st["s"], st["inf"], st["tinf"], st["cur"], st["nxt"], st["ttn"], T, seed_fraction,
-                              out["inf_o"], tape_v, tape_y0, S_un, rf)
+                              out["inf_o"], tape_v, tape_y0, S_un, rf, vf)
         if T is not None:
             ctx.mark_non_differentiable(T)
         return (out["s_o"], out["inf_o"], out["tinf_o"], out["cur_o"], out["nxt_o"], out["ttn_o"], T, red, red_label)
@@ -938,7 +1032,7 @@ class _BatchStep(torch.autograd.Function):
         world = static.world
         dev = world.device
         nb, Np, sG, K, nr = ctx.shape
-        beta, s, inf, tinf, cur, nxt, ttn, T, seed_fraction, inf_o, tape_v, tape_y0, S_un, rf = ctx.saved_tensors
+        beta, s, inf, tinf, cur, nxt, ttn, T, seed_fraction, inf_o, tape_v, tape_y0, S_un, rf, vf = ctx.saved_tensors
         seed, call_index = ctx.noise_key
         p, _ = _fill_params(world, spec, static.symptoms, seed, call_index)
         seed_mode = spec.mode == MODE_SEED
@@ -969,7 +1063,7 @@ class _BatchStep(torch.autograd.Function):
             io.label = ctx.label.codes.data_ptr()
             n_lab = 2 * ctx.label.n
         need = ctx.needs_input_grad   # (static, spec, noise, beta, s, inf, tinf, cur, nxt, ttn, seed_fraction, label,
-        #                                 seed_label, region_labels, region_factor)
+        #                                 seed_label, region_labels, region_factor, venue_labels, venue_factor)
         g_region, n_reg = None, 0
         if ctx.region_labels is not None:
             n_reg = ctx.region_labels.n
@@ -978,6 +1072,14 @@ class _BatchStep(torch.autograd.Function):
             if need[14]:
                 g_region = torch.empty(nb, n_reg, dtype=torch.float32, device=dev)
                 io.g_region_factor = g_region.data_ptr()
+        g_venue, n_ven = None, 0
+        if ctx.venue_labels is not None:
+            n_ven = K * ctx.venue_labels.n
+            _set_venue(io, world, ctx.venue_labels, vf)
+            if need[16]:
+                g_venue = torch.empty(nb, K, ctx.venue_labels.n, dtype=torch.float32, device=dev)
+                io.g_venue_factor = g_venue.data_ptr()
+                io.venue_work = _buffer(world, "venue_work_b", nb * sG).data_ptr()
 
         def new(name):
             t = torch.empty(nb, Np, dtype=torch.float32, device=dev)
@@ -1019,30 +1121,35 @@ class _BatchStep(torch.autograd.Function):
             io.wq = _buffer(world, "wq_b", nb * Np).data_ptr() if p.n_quar > 0 else io.w
             io.R, io.cR = _buffer(world, "R_b", nb * sG).data_ptr(), _buffer(world, "cR_b", nb * sG).data_ptr()
             bt = _lib.Batch(n_samples=nb, agent_stride=Np, group_stride=max(sG, 1), beta_stride=K, red_stride=nr,
-                            scratch_stride=scr_stride, label_stride=n_lab, region_stride=n_reg)
+                            scratch_stride=scr_stride, label_stride=n_lab, region_stride=n_reg, venue_stride=n_ven)
             with _on(dev):
                 _lib.check(L.gj_step_backward_batch(C.byref(desc), C.byref(p), C.byref(io), C.byref(bt), _stream(dev)),
                            "gj_step_backward_batch")
             g_beta = g_beta[:, :K]
             if g_region is not None and ctx.region_shape != (nb, n_reg):
                 g_region = g_region.sum(0)   # one row of factors shared by the samples
+            if g_venue is not None and len(ctx.venue_shape) == 2:
+                g_venue = g_venue.sum(0)     # one table shared by the samples
         return (None, None, None, g_beta if need[3] else None,
                 grads.get("s") if need[4] else None, grads.get("inf") if need[5] else None,
                 grads.get("tinf") if need[6] else None, grads.get("cur") if need[7] else None,
                 grads.get("nxt") if need[8] else None, grads.get("ttn") if need[9] else None,
-                g_frac if (seed_mode and need[10]) else None, None, None, None, g_region)
+                g_frac if (seed_mode and need[10]) else None, None, None, None, g_region, None, g_venue)
 
 
 def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=None, q_in=None, n_in=None,
                    seed_fraction=None, noise=None, next_spec=None, label: Optional[Labels] = None,
-                   seed_label: Optional[SeedLabels] = None, region: Optional[Region] = None):
+                   seed_label: Optional[SeedLabels] = None, region: Optional[Region] = None,
+                   venue: Optional[Venue] = None):
     """Run one (fused or partial) step.  ``state``: s, inf, tinf, cur, nxt, ttn (any may be None when
     the phases do not need it).  Returns a dict with s, inf, tinf, cur, nxt, ttn, T, q, n, red and red_label:
     with ``label`` the post-step cases and deaths per label column, [n, 2] ([b, n, 2] batched), else None.
     ``seed_label`` (seeding step only): ``seed_fraction`` then holds one fraction per region ([n], or [b, n]
     batched) and agent a is seeded with ``seed_fraction[seed_label.codes[a]]``.
     ``region`` (:class:`Region`, steps with the networks phase): every agent's pressure is multiplied by its region's
-    factor before the clamp; the factor is differentiable.  The seeding step ignores it."""
+    factor before the clamp; the factor is differentiable.  The seeding step ignores it.
+    ``venue`` (:class:`Venue`, steps with the networks phase): network k's beta is multiplied by the factor of each
+    group's region, ``venue.factor[k, venue.labels.codes[g]]``, in the group passes; differentiable."""
     world = static.world
     if world.device.type != "cuda":
         raise _lib.GradJuneLibraryError(
@@ -1058,7 +1165,8 @@ def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=N
             raise _lib.GradJuneLibraryError("batched ensembles run the whole fused step on an unpartitioned world")
         outs = _BatchStep.apply(static, spec, noise, beta, state["s"], state["inf"], state["tinf"], state["cur"],
                                 state["nxt"], state["ttn"], seed_fraction, label, seed_label,
-                                None if region is None else region.labels, None if region is None else region.factor)
+                                None if region is None else region.labels, None if region is None else region.factor,
+                                None if venue is None else venue.labels, None if venue is None else venue.factor)
         names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "red", "red_label")
         ret = dict(zip(names, outs))
         ret.update(q=None, n=None, lam=None)
@@ -1066,6 +1174,7 @@ def infection_step(static: StepStatic, spec: StepSpec, beta, state: dict, T_in=N
     outs = _Step.apply(static, spec, noise, beta, state.get("s"), state.get("inf"), state.get("tinf"),
                        state.get("cur"), state.get("nxt"), state.get("ttn"), T_in, q_in, n_in, seed_fraction, next_spec,
                        label, seed_label, None if region is None else region.labels,
-                       None if region is None else region.factor)
+                       None if region is None else region.factor, None if venue is None else venue.labels,
+                       None if venue is None else venue.factor)
     names = ("s", "inf", "tinf", "cur", "nxt", "ttn", "T", "q", "n", "red", "lam", "red_label")
     return dict(zip(names, outs))

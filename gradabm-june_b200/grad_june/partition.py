@@ -120,6 +120,15 @@ def partition_world(data: HeteroData, rank: int, world_size: int, bounds: Option
         local[t].id = torch.arange(mine.numel(), device=dev)
         people = torch.as_tensor(data[t]["people"])
         local[t].people = people.to(dev)[mine]
+        for key, v in data[t].items():   # every other per-group attribute (a region label, ...) of my groups
+            if key in ("id", "people"):
+                continue
+            if torch.is_tensor(v) and v.dim() >= 1 and v.shape[0] == G:
+                local[t][key] = v.to(dev)[mine]
+            elif isinstance(v, np.ndarray) and v.ndim >= 1 and v.shape[0] == G:
+                local[t][key] = v[mine.cpu().numpy()]
+            else:
+                local[t][key] = v
         local["agent", "attends_" + t, t].edge_index = torch.stack((lsrc, ldst))
         is_b = n_ranks[mine] >= 2
         lid = torch.nonzero(is_b).flatten()

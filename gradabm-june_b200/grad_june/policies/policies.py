@@ -45,18 +45,21 @@ def _camel(name):
 
 class Policies(torch.nn.Module):
     def __init__(self, interaction_policies=None, quarantine_policies=None, close_venue_policies=None,
-                 regional_policies=None):
+                 regional_policies=None, venue_policies=None):
         super().__init__()
         self.interaction_policies = interaction_policies
         self.quarantine_policies = quarantine_policies
         self.close_venue_policies = close_venue_policies
         self.regional_policies = regional_policies
+        self.venue_policies = venue_policies
         if regional_policies is not None:
             regional_policies.by()   # one region attribute per run
+        if venue_policies is not None:
+            venue_policies.by()
 
     @classmethod
     def from_policy_list(cls, policies):
-        from . import CloseVenuePolicies, InteractionPolicies, QuarantinePolicies, RegionalPolicies
+        from . import CloseVenuePolicies, InteractionPolicies, QuarantinePolicies, RegionalPolicies, VenuePolicies
 
         policies = [] if policies is None else policies
         return cls(
@@ -64,6 +67,7 @@ class Policies(torch.nn.Module):
             quarantine_policies=QuarantinePolicies(cls._get_policies_by_type(policies, "quarantine")),
             close_venue_policies=CloseVenuePolicies(cls._get_policies_by_type(policies, "close_venue")),
             regional_policies=RegionalPolicies(cls._get_policies_by_type(policies, "regional")),
+            venue_policies=VenuePolicies(cls._get_policies_by_type(policies, "venue")),
         )
 
     @classmethod

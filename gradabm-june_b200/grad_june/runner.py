@@ -21,7 +21,7 @@ from .paths import ensure_default_config
 from .timer import Timer
 from .transmission import PROFILE_KEYS, TransmissionSampler
 from .utils import read_path
-from .world import load_world, original_order, renumber_world
+from .world import group_labels, load_world, original_order, renumber_world, tier_candidates
 
 _STATE_KEYS = ("susceptibility", "is_infected", "infection_time", "transmission")
 _SYMPTOM_KEYS = ("current_stage", "next_stage", "time_to_next_stage")
@@ -134,6 +134,18 @@ class Runner(torch.nn.Module):
             else:
                 labels = agent_labels(data["agent"][self.region_by], self.n_agents)
                 self.region_labels = label_union(np.unique(labels), data.__dict__.get("_gj_partition"))
+        # regional venue policies (RegionalVenueDistancing): one factor per network and value of the groups' ``by``
+        # (``venue_labels``: the sorted distinct group labels of the covered edge types, over every rank)
+        vp = getattr(model.policies, "venue_policies", None)
+        self.venue_by = vp.by() if vp is not None else None
+        self.venue_labels = None
+        if self.venue_by is not None:
+            self._venue_group_labels = self._check_venue_policies(vp, data)
+            found = [np.unique(v) for v in self._venue_group_labels.values()]
+            self.venue_labels = label_union(np.unique(np.concatenate(found)) if found else np.zeros(0, np.int64),
+                                            data.__dict__.get("_gj_partition"))
+            if len(self.venue_labels) == 0:
+                raise ValueError("regional venue policies: the networks they name have no groups")
         # batched ensemble (SURVEY 8e-2): ``runner.batch = b`` makes ``forward()`` step b independent samples of the
         # epidemic at once — the networks' ``log_beta`` then hold b values each, the state tensors are [b, Np] and
         # every result series is [T+1, b].  All samples draw the same noise (common random numbers).
@@ -321,6 +333,61 @@ class Runner(torch.nn.Module):
         dev = self.data["agent"].susceptibility.device
         return ops.Region(self._region_codes(), rp.factor(timer, self.region_labels, dev, self.batch))
 
+    def _check_venue_policies(self, vp, data):
+        """Check the venue policies against the model and the world; returns {edge type: group labels} of the edge
+        types their entries cover.  A network the model does not have raises, and so does an entry covering a network
+        whose edge type runs on the RANGE tier (it has no group pass; households are covered with
+        RegionalSocialDistancing)."""
+        nets = self.model.infection_networks.networks
+        for policy in vp.policies:
+            for name in policy.beta_factors:
+                if name != "all" and name not in nets:
+                    raise ValueError(f"regional_venue_distancing: the model has no network {name!r} "
+                                     f"(it has {sorted(nets)})")
+        types = data.venue_types()
+        range_type, _ = tier_candidates(len(data["agent"].id), types, {t: data["attends_" + t].edge_index for t in types},
+                                        {t: len(data[t]["id"]) for t in types})
+        out = {}
+        for name in vp.covered(list(nets)):
+            t = nets[name].edge_type()
+            if t == range_type:
+                raise ValueError(f"regional_venue_distancing covers network {name!r}, whose edge type {t!r} runs on the "
+                                 "RANGE tier (per-agent re-sums, no group pass): give it no entry (an 'all' entry covers "
+                                 "it too) and use regional_social_distancing for it")
+            if t not in out:
+                out[t] = group_labels(data, t, self.venue_by)
+        return out
+
+    def _venue_codes(self):
+        """ops.VenueLabels of the venue policies' ``by`` on the device: every group's code in ``venue_labels`` (0 for
+        the groups of edge types no policy covers), built once per device."""
+        dev = self.data["agent"].susceptibility.device
+        hit = self.__dict__.get("_venue_codes_hit")
+        if hit is None or hit[0] != dev:
+            types = self.data.venue_types()
+            off = [0]
+            codes = []
+            for t in types:
+                G = len(self.data[t]["id"])
+                off.append(off[-1] + G)
+                v = self._venue_group_labels.get(t)
+                codes.append(np.zeros(G, np.int64) if v is None else label_codes(np.asarray(v), self.venue_labels))
+            codes = torch.as_tensor(np.concatenate(codes) if codes else np.zeros(0, np.int64))
+            hit = self.__dict__["_venue_codes_hit"] = (dev, ops.make_venue_labels(codes, len(self.venue_labels), off,
+                                                                                  dev))
+        return hit[1]
+
+    def _venue(self, timer):
+        """ops.Venue of the step at ``timer``: the factor table of its networks (step order), or None when no active
+        venue policy has an entry for any of them."""
+        if self.venue_by is None:
+            return None
+        vp = self.model.policies.venue_policies
+        names = [net.name for net in self.model.infection_networks.active_networks(timer, self.model.policies)]
+        dev = self.data["agent"].susceptibility.device
+        table = vp.table(timer, names, self.venue_labels, dev, self.batch)
+        return None if table is None else ops.Venue(self._venue_codes(), table)
+
     def _labels(self):
         """ops.Labels of ``results_by`` on the device (built once per label array and device, like
         ``_ethnicity_codes``), or None."""
@@ -367,7 +434,7 @@ class Runner(torch.nn.Module):
                 ahead = copy.copy(timer)
                 next(ahead)
             out = model.step(data, timer, age_bins=self._age_bins_host, want_probs=False, next_timer=ahead, label=label,
-                             region=self._region(timer))
+                             region=self._region(timer), venue=self._venue(timer))
             data = out[0]
             reds.append(out[1])
             if label is not None:

@@ -222,6 +222,42 @@ def world_from_arrays(arrays: Dict[str, np.ndarray], types: List[str], device="c
     return data.to(device)
 
 
+def group_labels(data: HeteroData, edge_type: str, by: str) -> np.ndarray:
+    """The region of every group of ``edge_type`` (numpy array, one entry per group in id order): the group attribute
+    ``data[edge_type][by]`` when the world carries it, else derived from the members: the value of
+    ``data["agent"][by]`` that most of the group's members carry, ties going to the smallest value (a group without
+    members takes the smallest value of the world).  The derivation needs every member of a group, so it runs on a
+    complete world: a partitioned world whose groups carry no ``by`` raises."""
+    store = data[edge_type]
+    G = len(store["id"])
+    if by in store:
+        v = store[by]
+        a = v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)
+        if a.ndim != 1 or a.shape[0] != G:
+            raise ValueError(f"data[{edge_type!r}].{by} must hold one value per group ({G}), got shape {a.shape}")
+        return a
+    if "_gj_partition" in data.__dict__ or "_gj_block" in data.__dict__:
+        raise ValueError(f"the groups of {edge_type!r} carry no {by!r}: a rank of a partitioned world cannot see all of a "
+                         f"group's members; set data[{edge_type!r}].{by} on the complete world before partitioning")
+    v = data["agent"][by]
+    agent = v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)
+    ei = data["attends_" + edge_type].edge_index.detach().cpu().numpy()
+    n = len(data["agent"].id)
+    if agent.ndim != 1 or agent.shape[0] not in (1, n):
+        raise ValueError(f"data['agent'].{by} must hold one value per agent ({n}), got shape {agent.shape}")
+    values, codes = np.unique(np.broadcast_to(agent, (n,)), return_inverse=True)
+    L = len(values)
+    pair, count = np.unique(ei[1].astype(np.int64) * L + codes[ei[0]], return_counts=True)
+    grp, code = pair // L, pair % L
+    # per group: the largest count, then the smallest code (lexsort: last key first)
+    idx = np.lexsort((code, -count, grp))
+    first = np.ones(idx.shape[0], dtype=bool)
+    first[1:] = grp[idx][1:] != grp[idx][:-1]
+    out = np.zeros(G, dtype=np.int64)
+    out[grp[idx][first]] = code[idx][first]
+    return values[out]
+
+
 # --------------------------------------------------------------------------------------
 # CSR layout
 # --------------------------------------------------------------------------------------

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define GJ_ABI_VERSION 13
+#define GJ_ABI_VERSION 14
 
 #define GJ_MAX_TYPES 8      /* edge types (household, company, school, university, care_home, leisure, ...) */
 #define GJ_MAX_NETS 16      /* infection networks active in one step */
@@ -321,6 +321,17 @@ typedef struct gj_fwd_io {
   int32_t n_regions;          /* 1 .. 2^30 */
   int32_t _pad_region;
   const float* region_factor; /* [n_regions] (batched: [n_samples][region_stride]) */
+  /* regional venue factor (GJ_MODE_STEP with the networks phase; NULL = none): venue_region[g] is the region in
+   * [0, n_venue_regions) of global group g (the group's location, not its visitors'), and network k's per-group value
+   * uses beta_k * venue_factor[k * n_venue_regions + venue_region[g]] instead of beta_k wherever it is formed:
+   * ((beta_k * f) * pc_g) * S_g.  Row k belongs to nets[k]; a row of ones leaves every output bit-equal to the call
+   * without the factor, and a factor of 0 closes network k's venues in that region.  The factor applies to the
+   * GENERIC and CELL tiers; a RANGE-tier network (households) ignores its row.  Factors must be >= 0 and codes must lie
+   * in [0, n_venue_regions): neither is checked on the device.  venue_factor may be NULL only when venue_region is. */
+  const int32_t* venue_region;  /* [n_groups] by global group id */
+  int32_t n_venue_regions;      /* 1 .. 2^30 */
+  int32_t _pad_venue;
+  const float* venue_factor;    /* [n_nets][n_venue_regions] (batched: [n_samples][venue_stride]) */
 } gj_fwd_io;
 
 typedef struct gj_bwd_io {
@@ -395,6 +406,23 @@ typedef struct gj_bwd_io {
   const int32_t* region_offsets;  /* [n_regions + 1] */
   float* region_work;             /* [N] workspace (batched: [n_samples][agent_stride]) */
   float* g_region_factor;         /* [n_regions] (batched: [n_samples][region_stride]), or NULL */
+  /* regional venue factor: the forward's venue_region / n_venue_regions / venue_factor (NULL = none).  The group passes
+   * of the backward apply the same factor, and d/dbeta_k = sum_g ((own_g * pc_g) * f) * S_g * R_g.  With g_venue_factor
+   * non-NULL, the d/dbeta pass also writes beta_k * own_g * pc_g * S_g * R_g per group to network k's own row of
+   * venue_work (at nets[k].s_off, one entry per group of its edge type; a buffer sized like R holds every row), and a
+   * reduction writes g_venue_factor[k * n_venue_regions + r] = the sum of that row over the
+   * groups of network k's edge type in region r (0 for a RANGE-tier network), with the deterministic fp64 reduction of
+   * seeding by label.  venue_order holds, for every edge type t, its groups' indices WITHIN the type, stably sorted by
+   * region, at positions [type_group_off[t], type_group_off[t + 1]); venue_offsets[t * (n_venue_regions + 1) + r] is
+   * where region r starts within type t's part (relative to type_group_off[t]; [n_types][n_venue_regions + 1]). */
+  const int32_t* venue_region;    /* [n_groups] */
+  int32_t n_venue_regions;
+  int32_t _pad_venue;
+  const float* venue_factor;      /* [n_nets][n_venue_regions] (batched: [n_samples][venue_stride]) */
+  const int32_t* venue_order;     /* [n_groups] */
+  const int32_t* venue_offsets;   /* [n_types][n_venue_regions + 1] */
+  float* venue_work;              /* sized like R (batched: [n_samples][group_stride]) */
+  float* g_venue_factor;          /* [n_nets][n_venue_regions] (batched: [n_samples][venue_stride]), or NULL */
 } gj_bwd_io;
 
 /* ---- library ---------------------------------------------------------------------------- */
@@ -474,6 +502,9 @@ typedef struct gj_batch {
   /* stride of region_factor / g_region_factor (elements, >= n_regions when a region factor is given): every sample has
    * its own row of factors and of their gradient */
   int64_t region_stride;
+  /* stride of venue_factor / g_venue_factor (elements, >= n_nets * n_venue_regions when a venue factor is given):
+   * every sample has its own table of factors and of their gradient */
+  int64_t venue_stride;
 } gj_batch;
 int gj_step_forward_batch(const gj_world_desc* w, const gj_step_params* p, const gj_fwd_io* io, const gj_batch* batch,
                           void* stream);
